@@ -12,12 +12,14 @@ thresholded-FC graphs per batch. At N>1 every rank trains on its own 1024-graph 
 global batch 1024*N: `value`) with BatchNorm statistics, DGI negatives and gradients synchronised; the same line
 carries a `strong` block (BASELINE configs[2]: ONE global batch of 1024 graphs sharded 1024/N per GPU) and
 `dp_parity_err` (an N-rank step against rank 0 recomputing the same global batch single-process, before timing).
-The timed region is K x `config.inner_repeats` steps (>= ~1 s of device time); ms_per_step is per step.
-Prints ONE JSON line (rank 0).
+The timed region is exactly K steps (default 400, >= ~1 s of device time on one B200); ms_per_step is per step.
+Prints ONE JSON line (rank 0). `--dump-outputs DIR` also writes what the last timed step produced as DIR/<name>.npy;
+the inputs are seeded, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
 import os
+import re
 import subprocess
 import sys
 import tempfile
@@ -26,6 +28,7 @@ import time
 import numpy as np
 import torch
 
+sys.dont_write_bytecode = True          # the tree may be read-only: the benchmark writes nothing into it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -37,12 +40,20 @@ METRIC = "gin_train_graphs_per_sec_400roi"
 UNIT = "graphs/s"
 N_ROIS, HIDDEN, LAYERS, MLP_LAYERS, BETA, LR = 400, 64, 5, 2, 0.05, 0.005
 EDGES_PER_GRAPH = 47600
+# untimed steps before the timed region, whatever --warmup says: driver.Trainer runs the first two steps of a batch
+# shape eagerly and captures the whole-step CUDA graph in the third; three replays follow before the clock starts
+MIN_WARMUP = 6
+# default timed steps: 400 training steps of ~2.8 ms (saliency calls of ~3.4 ms) keep the timed window above ~1 s, long
+# enough for the clock sampler and the card's power management to settle
+DEFAULT_STEPS, DEFAULT_STEPS_REFERENCE = 400, 10
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default %d: >= ~1 s of device time on one B200; %d for --impl reference, whose "
+                         "steps run on the host cores)" % (DEFAULT_STEPS, DEFAULT_STEPS_REFERENCE))
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--batch", type=int, default=None, help="graphs per GPU per step (default 1024; 128 for --config c4)")
@@ -62,15 +73,22 @@ def parse():
     ap.add_argument("--saliency", action="store_true",
                     help="measure gradient-saliency extraction (graphcnn.py:254-299) throughput instead of training")
     ap.add_argument("--saliency-batch", type=int, default=1024, help="graphs per batched saliency call")
-    ap.add_argument("--min-seconds", type=float, default=1.0,
-                    help="lower bound on the device time of the timed region: the K steps are repeated `inner_repeats` "
-                         "times (declared in config) so that clocks / throttling are sampled over >= this long")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one produced as DIR/<name>.npy (float32/float64): "
+                         "training - the loss, the gradients and the BatchNorm running statistics of a last step that "
+                         "starts from the initial parameters; --saliency - a fixed sample of the batch's saliency maps")
     ap.add_argument("--no-strong", action="store_true", help="N>1: skip the strong-scaling block (global batch fixed)")
     ap.add_argument("--no-dp-parity", action="store_true", help="N>1: skip the data-parallel parity step before timing")
     ap.add_argument("--no-breakdown", action="store_true",
                     help="skip the eager per-kernel timing pass (no `roofline` / `kernel_breakdown`): for ncu launch lists "
                          "of the captured step")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = DEFAULT_STEPS_REFERENCE if args.impl == "reference" else DEFAULT_STEPS
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this repository's CUDA path (--impl b200)")
     global N_ROIS, HIDDEN, EDGES_PER_GRAPH
     if args.config == "c4":
         N_ROIS, HIDDEN = 1000, 128
@@ -288,6 +306,50 @@ class ClockSampler(object):
 
 
 # ------------------------------------------------------------------------------------------
+# --dump-outputs
+# ------------------------------------------------------------------------------------------
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+# An MLP's Linear bias feeds a train-mode BatchNorm: its true gradient is exactly zero, and what a step computes for it
+# is rounding noise of the fp32 atomics (~1e-7 of the largest gradient), different in every run
+ZERO_GRAD_BIAS = re.compile(r"^mlps\.\d+\.(linear|linears\.\d+)\.bias$")
+ZERO_GRAD_FLUSH = 1e-4
+
+
+def step_outputs(model, loss):
+    """What a training step computed: the loss it returned, every parameter's gradient and the BatchNorm running
+    statistics it updated. In the ZERO_GRAD_BIAS gradients, entries below ZERO_GRAD_FLUSH x the largest gradient entry
+    are written as 0, so that the run-to-run noise drops out while a build that gets them wrong still shows."""
+    out = {"loss": loss.reshape(1)}
+    for k, v in model.named_buffers():
+        if v.is_floating_point():
+            out[k] = v
+    grads = {k: p.grad.detach() for k, p in model.named_parameters() if p.grad is not None}
+    gmax = max(float(g.abs().max()) for g in grads.values())
+    for k, g in grads.items():
+        if ZERO_GRAD_BIAS.match(k):
+            g = torch.where(g.abs() < ZERO_GRAD_FLUSH * gmax, torch.zeros_like(g), g)
+        out[k + ".grad"] = g
+    return out
+
+
+def write_outputs(out_dir, arrays):
+    """One DIR/<name>.npy per array: float64 stays float64, everything else is written as float32."""
+    host = {}
+    for k, v in arrays.items():
+        a = v.detach().cpu().numpy() if torch.is_tensor(v) else np.asarray(v)
+        host[k] = a if a.dtype == np.float64 else a.astype(np.float32)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
+# ------------------------------------------------------------------------------------------
 # the B200 arm
 # ------------------------------------------------------------------------------------------
 
@@ -387,43 +449,53 @@ def run_b200(args):
             return trainer.step([pool[i] for i in sel], labels_np[sel])
         return step
 
-    def timed(step, n_graphs, steps, what):
-        """W warm-up steps, then `steps` x inner steps between two events, max over ranks. Returns (ms per step,
-        inner, clocks, libgnm kernels launched in the region)."""
-        for _ in range(max(args.warmup, 3)):
+    def timed(step, n_graphs, steps, what, before_last=None):
+        """W warm-up steps, then `steps` steps between two events, max over ranks; `before_last()` runs ahead of the
+        last step, outside the timed window. Returns (ms per step, clocks, libgnm kernels launched in the region, what
+        the last step returned)."""
+        for _ in range(max(args.warmup, MIN_WARMUP)):
             step()
-        barrier()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(3):
-            step()
-        e1.record()
-        torch.cuda.synchronize()
-        est = torch.tensor([e0.elapsed_time(e1) / 3.0], dtype=torch.float64, device=dev)
-        if world > 1:
-            torch.distributed.all_reduce(est, op=torch.distributed.ReduceOp.MAX)
-        inner = max(1, int(np.ceil(args.min_seconds * 1e3 / (float(est.item()) * steps))))
         barrier()
         sampler = ClockSampler(local_rank) if rank == 0 else None
         k0 = ops.kernels_launched()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         e0.record()
-        for _ in range(steps * inner):
-            step()
+        for i in range(steps):
+            if before_last is not None and i == steps - 1:
+                p0.record()
+                before_last()
+                p1.record()
+            last = step()
         e1.record()
         barrier()
-        ms = e0.elapsed_time(e1)
+        ms = e0.elapsed_time(e1) - (p0.elapsed_time(p1) if before_last is not None else 0.0)
         launched = ops.kernels_launched() - k0
         clk = sampler.stop() if sampler else None
         check_status(what)
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
         if world > 1:
             torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
-        return float(t.item()) / (steps * inner), inner, clk, launched
+        return float(t.item()) / steps, clk, launched, last
+
+    # --dump-outputs: the last timed step starts from the model's initial parameters and buffers. Adam turns the last-bit
+    # differences between two runs (the fp32 atomics that merge the kernels' dW partials) into lr-sized steps of
+    # near-zero gradient components, so after a dozen steps two runs of one build differ by 1e-2 and more; from the
+    # initial state, what the last step computes is a reproducible function of the seeded inputs.
+    initial = {k: v.detach().clone() for k, v in model.state_dict().items()} if args.dump_outputs else None
+
+    def restore_initial():
+        with torch.no_grad():
+            for k, v in model.state_dict().items():
+                v.copy_(initial[k])
 
     step_resident = make_step(B)
-    ms_per_step, inner, clocks, launches = timed(step_resident, B, args.steps, "the timed steps")
+    ms_per_step, clocks, launches, last_loss = timed(step_resident, B, args.steps, "the timed steps",
+                                                     restore_initial if args.dump_outputs else None)
+    if args.dump_outputs and rank == 0:
+        # before anything below trains the model further
+        write_outputs(args.dump_outputs, step_outputs(model, last_loss))
     elapsed_ms = ms_per_step * args.steps
     value = B * world / (ms_per_step / 1e3)
 
@@ -431,9 +503,9 @@ def run_b200(args):
     strong = None
     if world > 1 and not args.no_strong and B % world == 0:
         bs_local = B // world
-        ms_s, inner_s, clk_s, _ = timed(make_step(bs_local), bs_local, args.steps, "the strong-scaling steps")
+        ms_s, clk_s, _, _ = timed(make_step(bs_local), bs_local, args.steps, "the strong-scaling steps")
         strong = {"global_batch": B, "graphs_per_gpu": bs_local, "value": B / (ms_s / 1e3), "unit": UNIT,
-                  "ms_per_step": ms_s, "inner_repeats": inner_s, "clocks": clk_s,
+                  "ms_per_step": ms_s, "clocks": clk_s,
                   "what": "same step, the global batch held at %d graphs (main.py:26-41 at one global batch): each rank "
                           "trains on %d graphs, BatchNorm over the global M = %d rows" % (B, bs_local, B * N_ROIS)}
 
@@ -523,7 +595,7 @@ def run_b200(args):
             model.cache_graphs = True
             return B * world * steps / float(tt.item()), int(h2d)
         v_cold, h2d_cold = timed_e2e(True, max(2, min(args.steps, 5)), 1)
-        v_warm, h2d_warm = timed_e2e(False, args.steps * inner, 2)
+        v_warm, h2d_warm = timed_e2e(False, args.steps, 2)
         e2e = {"value": v_warm, "unit": UNIT, "h2d_bytes_per_step": h2d_warm, "d2h_bytes_per_step": 4,
                "what": "the literal main.py:25-43 loop body: model(batch_graph) on host S2VGraph lists, labels and DGI "
                        "targets built on the host and copied in every step, loss.cpu() every step. Steady state of "
@@ -545,7 +617,7 @@ def run_b200(args):
                 step_e2e_trainer()
             barrier()
             h0 = trainer.h2d_bytes
-            n_tr = args.steps * inner
+            n_tr = args.steps
             t0 = time.perf_counter()
             for _ in range(n_tr):
                 step_e2e_trainer()
@@ -566,14 +638,14 @@ def run_b200(args):
 
     if rank == 0:
         line = {"metric": METRIC if N_ROIS == 400 else "gin_train_graphs_per_sec_%droi" % N_ROIS, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps,
-                "warmup": max(args.warmup, 3), "ms_per_step": elapsed_ms / args.steps, "higher_is_better": True,
+                "warmup": max(args.warmup, MIN_WARMUP), "ms_per_step": elapsed_ms / args.steps, "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
-                "config": dict(workload_config(args, world), cuda_graphs=bool(model.use_cuda_graphs), inner_repeats=inner,
-                               steps_timed=args.steps * inner,
+                "config": dict(workload_config(args, world), cuda_graphs=bool(model.use_cuda_graphs),
+                               steps_timed=args.steps,
                                driver=("driver.Trainer: whole step (assembly, forward, heads, loss, backward, gradient "
                                        "averaging, Adam) as one CUDA graph" if args.driver == "fused" else
                                        "main.py loop body over the drop-in model (encoder forward / backward as CUDA graphs)")),
-                "clocks": clocks, "gpu_launches": launches, "gpu_launches_per_step": launches / float(args.steps * inner),
+                "clocks": clocks, "gpu_launches": launches, "gpu_launches_per_step": launches / float(args.steps),
                 "e2e": e2e, "roofline": roof, "cpu_baseline": cpu_baseline, "strong": strong, "dp_parity_err": dp_parity,
                 "kernel_breakdown": breakdown}
         print(json.dumps(line))
@@ -592,7 +664,6 @@ def dp_parity_check(args, comm, dev, per_rank=16):
     state and permutation. 16 graphs per rank = 6400 rows: the tcgen05 kernel family of the timed run. Returns the
     largest per-tensor scaled error (each tensor on its own max-abs; MLP Linear biases - true gradient zero in front
     of a train-mode BatchNorm - on the largest gradient's scale)."""
-    import re
     from graph_neural_mapping_b200 import dist as gdist, synth
     from graph_neural_mapping_b200.models import GIN_InfoMaxReg
     world, rank = comm.world, comm.rank
@@ -647,12 +718,11 @@ def dp_parity_check(args, comm, dev, per_rank=16):
             return float((a.double() - b.double()).abs().max() / max(float(b.double().abs().max()), floor, 1e-30))
         errs = {"c_logit": err(torch.cat(cs, 0), c_s), "d_logit": err(d_all, d_s), "loss": err(torch.stack(ls).mean(), loss_s)}
         gmax = max(float(p.grad.abs().max()) for p in single.parameters() if p.grad is not None)
-        zero_bias = re.compile(r"^mlps\.\d+\.(linear|linears\.\d+)\.bias$")
         worst = ("", 0.0)
         for (k, p), (_, q) in zip(model.named_parameters(), single.named_parameters()):
             if q.grad is None:
                 continue
-            e = err(p.grad, q.grad, 1e-2 * gmax if zero_bias.match(k) else 0.0)
+            e = err(p.grad, q.grad, 1e-2 * gmax if ZERO_GRAD_BIAS.match(k) else 0.0)
             if e > worst[1]:
                 worst = (k, e)
         for (k, b1), (_, b2) in zip(model.named_buffers(), single.named_buffers()):
@@ -705,22 +775,16 @@ def run_saliency(args):
         state["i"] += 1
         return s
 
-    for _ in range(max(args.warmup, 3)):
+    for _ in range(max(args.warmup, MIN_WARMUP)):
         sal = step()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for _ in range(3):
-        step()
-    e1.record()
-    torch.cuda.synchronize()
-    inner = max(1, int(np.ceil(args.min_seconds * 1e3 / (e0.elapsed_time(e1) / 3.0 * args.steps))))
     if comm.world > 1:
         torch.distributed.barrier()
     sampler = ClockSampler(local_rank) if comm.rank == 0 else None
     k0 = ops.kernels_launched()
     e0.record()
-    for _ in range(args.steps * inner):
+    for _ in range(args.steps):
         sal = step()
     e1.record()
     torch.cuda.synchronize()
@@ -731,13 +795,18 @@ def run_saliency(args):
     t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     if comm.world > 1:
         torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
-    ms = float(t.item()) / (args.steps * inner)
+    ms = float(t.item()) / args.steps
+    if args.dump_outputs and comm.rank == 0:
+        # the whole [b * N, N] map is 4 * b * N^2 bytes (655 MB at b = 1024, N = 400): keep a seeded sample of its graphs
+        maps = sal.reshape(b, N_ROIS, N_ROIS)
+        pick = np.sort(np.random.default_rng(0).choice(b, size=min(b, (32 << 20) // (4 * N_ROIS * N_ROIS)), replace=False))
+        write_outputs(args.dump_outputs, {"saliency": maps[torch.from_numpy(pick).to(dev)], "saliency_graphs": pick})
     # e2e: maps land in pinned host memory (the sink touches every batch once, like a file writer would)
     seen = {"bytes": 0}
 
     def sink(first, arr):
         seen["bytes"] += arr.nbytes
-    n_e2e = min(len(pool), max(4 * b, (args.steps * inner * b) // 4 // b * b))
+    n_e2e = min(len(pool), max(4 * b, args.steps // 4 * b))
     driver.stream_saliency(model, pool[:2 * b], 1, sink, batch=b)          # warm the pinned buffers
     torch.cuda.synchronize()
     seen["bytes"] = 0
@@ -758,17 +827,17 @@ def run_saliency(args):
     if comm.rank == 0:
         print(json.dumps({
             "metric": "gin_saliency_graphs_per_sec_%droi" % N_ROIS, "value": b * comm.world / (ms / 1e3), "unit": UNIT,
-            "n_gpus": comm.world, "steps": args.steps, "warmup": max(args.warmup, 3), "ms_per_step": ms,
+            "n_gpus": comm.world, "steps": args.steps, "warmup": max(args.warmup, MIN_WARMUP), "ms_per_step": ms,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": "gradient saliency (graphcnn.py:254-299), %d graphs per GPU of BASELINE configs[4] (100k "
                                    "graphs over 8 GPUs), %d graphs per batched call, N=%d, 5-layer hidden %d"
                                    % (len(pool), b, N_ROIS, HIDDEN),
-                       "graphs_per_gpu": len(pool), "graphs_per_call": b, "inner_repeats": inner,
-                       "steps_timed": args.steps * inner, "bytes_written_per_step": int(out_bytes),
+                       "graphs_per_gpu": len(pool), "graphs_per_call": b,
+                       "steps_timed": args.steps, "bytes_written_per_step": int(out_bytes),
                        "generate_and_ingest_s": t_gen, "parallelism": "shard%d (no collective)" % comm.world,
                        "l2_policy": "inputs_larger_than_l2 (each call writes %d MB and cycles through %d batches)"
                                     % (int(out_bytes / 1e6), len(batches))},
-            "clocks": clocks, "gpu_launches": launches, "gpu_launches_per_step": launches / float(args.steps * inner),
+            "clocks": clocks, "gpu_launches": launches, "gpu_launches_per_step": launches / float(args.steps),
             "e2e": {"value": n_e2e * comm.world / float(dt.item()), "unit": UNIT, "h2d_bytes_per_step": 41 * b,
                     "d2h_bytes_per_step": int(seen["bytes"] / max(1, n_e2e // b)),
                     "what": "driver.stream_saliency over %d graphs: every batch's [b, N, N] map copied to pinned host "

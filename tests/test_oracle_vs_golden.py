@@ -103,8 +103,19 @@ def test_eval_and_saliency_match_reference(name):
         assert_close(s[n0:], g.z["saliency/g1_c1"], TOL_GRAD, "batched saliency g1")
 
 
+@pytest.fixture
+def golden_threads():
+    """The intra-op thread count tests/golden/make_golden.py ran the reference with. ATen splits its CPU reductions by
+    thread count, so only with the same count does the port repeat the reference's summation order, whatever the host's
+    core count."""
+    saved = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(saved)
+
+
 @pytest.mark.parametrize("name", [n for n in golden_names() if "max" not in n])
-def test_aten_port_matches_reference(name):
+def test_aten_port_matches_reference(name, golden_threads):
     """oracle/aten_port.py (the CPU baseline that bench.py times) against the reference's outputs."""
     from oracle import aten_port
     g = Golden(name)

@@ -3,7 +3,12 @@ repo-root `models/` shim - the drop-in claim of SURVEY 8(b): `from models.graphc
 the libgnm-backed classes and `train()` / `test()` / `get_saliency_map()` / `get_latent_space()` (main.py:19-96) run
 unchanged. The same functions run on the reference's own classes on the CPU give the expected values.
 
-oracle/_ref is git-ignored and built where /root/reference exists (build() does it); the tests skip without it."""
+Why these tests skip in a plain checkout: both sides of the comparison execute the reference's own sources (main.py and
+its models/), which this repository does not contain. `python oracle/make_ref.py` stages them, byte for byte, into the
+git-ignored oracle/_ref from a checkout of the original project named by GNM_REFERENCE_ROOT; build() does the same when
+that checkout is present. The expected values cannot be stored instead: they are main.py's outputs on the reference's
+classes, so writing them needs those same sources. What the reference's classes compute on these graphs (train step,
+eval logits, latent, saliency) is stored in tests/golden/ and checked there against this repository's models."""
 import argparse
 import warnings
 

@@ -193,6 +193,113 @@ dgi_score_bwd_vec_kernel(const float* __restrict__ h_all, int64_t layer_stride, 
     }
 }
 
+// Training-step scorer (driver.Trainer). The BCE-with-logits gradient of a score is local - ds = grad_scale *
+// (sigmoid(s) - y), y = 1 for the positives and 0 for the negatives (main.py:32-37) - so the pass that forms the scores
+// also forms what the backward needs from n_f: d_score[r] of the positives, du_g, s2_g, d_bias, and the loss. One read
+// of the L slices instead of two (dgi_score_fwd + dgi_score_bwd) and no BCE launch. Rows go to threads as in
+// dgi_score_fwd_kernel<16> / dgi_score_bwd_vec_kernel and the arithmetic is theirs and bce_logits_kernel's, in the same
+// order: the scores and d_score are bit-identical to that three-launch sequence; du and s2 agree to fp32 rounding (the
+// negatives' gradient, formed once per graph here, can round differently), the loss differs in summation order.
+template <int NL>
+__global__ void __launch_bounds__(256)
+dgi_score_train_kernel(const float* __restrict__ h_all, int64_t layer_stride, int64_t ldh, int n_rows,
+                       const float* __restrict__ u, const float* __restrict__ neg_table,
+                       const int32_t* __restrict__ neg_idx, const int32_t* __restrict__ node_off,
+                       const float* __restrict__ bias, float grad_scale, double loss_scale, float* __restrict__ out,
+                       float* __restrict__ d_score, float* __restrict__ du, float* __restrict__ s2,
+                       double* __restrict__ d_bias, double* __restrict__ loss_acc) {
+    constexpr int F = 64, NH = NL * F;
+    __shared__ __align__(16) float us[NH];
+    __shared__ __align__(16) float part[8][NH];
+    __shared__ float red[2][8];
+    __shared__ double lred[8];
+    __shared__ float s_neg;
+    const int g = blockIdx.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int half = lane >> 4, c4 = lane & 15;
+    for (int i = threadIdx.x; i < NH; i += blockDim.x) us[i] = u[(int64_t)g * NH + i];
+    __syncthreads();
+    const float b = bias ? __ldg(bias) : 0.f;
+    const float* nr = neg_table + (int64_t)neg_idx[g] * NH;
+    if (warp == 0) {
+        float a = 0.f;
+        for (int i = lane; i < NH; i += 32) a = fmaf(nr[i], us[i], a);
+        a = warp_sum(a);
+        if (lane == 0) s_neg = a + b;
+    }
+    __syncthreads();
+    const float sn = s_neg;
+    const float y_neg = 0.f, y_pos = 1.f;
+    const float d_neg = (1.f / (1.f + expf(-sn)) - y_neg) * grad_scale;     // every negative row of the graph
+    const int r0 = node_off[g], r1 = node_off[g + 1];
+    float4 acc[NL];
+#pragma unroll
+    for (int l = 0; l < NL; ++l) acc[l] = make_float4(0.f, 0.f, 0.f, 0.f);
+    float sum1 = 0.f, sum2 = 0.f;
+    double loss = 0.0;
+    for (int rb = r0 + warp * 2; rb < r1; rb += 16) {
+        const int r = rb + half;
+        const bool row = r < r1;
+        float4 hv[NL];
+        float a = 0.f;
+        if (row) {
+            const float* hr = h_all + (int64_t)r * ldh + c4 * 4;
+#pragma unroll
+            for (int l = 0; l < NL; ++l) hv[l] = ld_stream_f4(hr + l * layer_stride);
+#pragma unroll
+            for (int l = 0; l < NL; ++l) {
+                const float4 uv = *reinterpret_cast<const float4*>(us + l * F + c4 * 4);
+                a = fmaf(hv[l].x, uv.x, a); a = fmaf(hv[l].y, uv.y, a); a = fmaf(hv[l].z, uv.z, a); a = fmaf(hv[l].w, uv.w, a);
+            }
+        }
+        a = group_sum<16>(a);
+        if (row) {
+            const float v = a + b;
+            const float d1 = (1.f / (1.f + expf(-v)) - y_pos) * grad_scale;
+#pragma unroll
+            for (int l = 0; l < NL; ++l) {
+                acc[l].x = fmaf(d1, hv[l].x, acc[l].x); acc[l].y = fmaf(d1, hv[l].y, acc[l].y);
+                acc[l].z = fmaf(d1, hv[l].z, acc[l].z); acc[l].w = fmaf(d1, hv[l].w, acc[l].w);
+            }
+            if (c4 == 0) {
+                out[r] = v;
+                out[n_rows + r] = sn;
+                d_score[r] = d1;
+                sum1 += d1;
+                sum2 += d_neg;
+                loss += (double)(fmaxf(v, 0.f) - v * y_pos + log1pf(expf(-fabsf(v))));
+            }
+        }
+    }
+#pragma unroll
+    for (int l = 0; l < NL; ++l) {
+        acc[l].x += __shfl_xor_sync(GNM_FULL_MASK, acc[l].x, 16); acc[l].y += __shfl_xor_sync(GNM_FULL_MASK, acc[l].y, 16);
+        acc[l].z += __shfl_xor_sync(GNM_FULL_MASK, acc[l].z, 16); acc[l].w += __shfl_xor_sync(GNM_FULL_MASK, acc[l].w, 16);
+        if (half == 0) *reinterpret_cast<float4*>(&part[warp][l * F + c4 * 4]) = acc[l];
+    }
+    sum1 = warp_sum(sum1);
+    sum2 = warp_sum(sum2);
+    loss = warp_sum_d(loss);
+    if (lane == 0) { red[0][warp] = sum1; red[1][warp] = sum2; lred[warp] = loss; }
+    __syncthreads();
+    float t1 = 0.f, t2 = 0.f;
+    for (int w = 0; w < 8; ++w) { t1 += red[0][w]; t2 += red[1][w]; }
+    for (int i = threadIdx.x; i < NH; i += blockDim.x) {
+        float a = 0.f;
+#pragma unroll
+        for (int w = 0; w < 8; ++w) a += part[w][i];
+        du[(int64_t)g * NH + i] = fmaf(t2, nr[i], a);
+    }
+    if (threadIdx.x == 0) {
+        s2[g] = t2;
+        atomicAdd(d_bias, (double)t1 + (double)t2);
+        // the graph's negative rows all carry the score sn: their loss terms are one value times the row count
+        double lt = (double)(r1 - r0) * (double)(fmaxf(sn, 0.f) - sn * y_neg + log1pf(expf(-fabsf(sn))));
+        for (int w = 0; w < 8; ++w) lt += lred[w];
+        atomicAdd(loss_acc, lt * loss_scale);
+    }
+}
+
 __global__ void __launch_bounds__(256)
 rowdot_score_kernel(const float* __restrict__ h, int64_t ldh, int n_rows, int n_feat, const float* __restrict__ u,
                     int64_t ldu, int rows_per_graph, const float* __restrict__ bias, const float* __restrict__ s_bias,
@@ -287,6 +394,33 @@ extern "C" int gnm_dgi_score_bwd(const float* h_all, int64_t layer_stride, int n
     dgi_score_bwd_kernel<<<n_graphs, 256, smem, gnm_cast_stream(stream)>>>(h_all, layer_stride, n_layers, n_feat, ldh,
                                                                            n_rows, d_out, neg_table, neg_idx, node_off,
                                                                            du, s2, d_bias);
+    GNM_RETURN_IF_LAUNCH_FAILED();
+    return GNM_OK;
+}
+
+extern "C" int gnm_dgi_score_train(const float* h_all, int64_t layer_stride, int n_layers, int n_feat, int64_t ldh,
+                                   int n_rows, const float* u, const float* neg_table, const int32_t* neg_idx,
+                                   const int32_t* node_off, int n_graphs, const float* bias, float grad_scale,
+                                   double loss_scale, float* out, float* d_score, float* du, float* s2, double* d_bias,
+                                   double* loss_acc, gnm_stream_t stream) {
+    if (n_layers < 0 || n_feat < 0 || n_rows < 0 || n_graphs < 0) return GNM_ERR_BAD_ARG;
+    if (n_graphs == 0 || n_rows == 0) return GNM_OK;
+    if (!h_all || !u || !neg_table || !neg_idx || !node_off || !out || !d_score || !du || !s2 || !d_bias || !loss_acc)
+        return GNM_ERR_BAD_ARG;
+    if (n_feat != 64 || n_layers < 1 || n_layers > 5) return GNM_ERR_TOO_LARGE;
+    if ((ldh & 3) != 0 || (layer_stride & 3) != 0 || !gnm_aligned16(h_all)) return GNM_ERR_ALIGN;
+#define GNM_DGI_TRAIN(NL) \
+    do { gnm_count_launch(GNM_K_OTHER); \
+    dgi_score_train_kernel<NL><<<n_graphs, 256, 0, gnm_cast_stream(stream)>>>(h_all, layer_stride, ldh, n_rows, u, neg_table, \
+        neg_idx, node_off, bias, grad_scale, loss_scale, out, d_score, du, s2, d_bias, loss_acc); } while (0)
+    switch (n_layers) {
+        case 1: GNM_DGI_TRAIN(1); break;
+        case 2: GNM_DGI_TRAIN(2); break;
+        case 3: GNM_DGI_TRAIN(3); break;
+        case 4: GNM_DGI_TRAIN(4); break;
+        default: GNM_DGI_TRAIN(5); break;
+    }
+#undef GNM_DGI_TRAIN
     GNM_RETURN_IF_LAUNCH_FAILED();
     return GNM_OK;
 }

@@ -84,7 +84,8 @@ class _WholeStepPlan(object):
     def body_fused(self):
         """One training step without torch autograd / torch.optim / torch loss kernels: encoder + DGI forward
         (engine.run_forward), prediction heads + dropout + CrossEntropy forward and backward (gnm_heads_ce),
-        BCEWithLogits forward and backward (gnm_bce_logits), the hand-derived backward (engine.run_backward),
+        BCEWithLogits forward and backward (in the scoring pass of run_forward, or gnm_bce_logits where that kernel does
+        not take the shape), the hand-derived backward (engine.run_backward),
         gradient averaging and Adam (gnm_adam_step). Same arithmetic as main.py:31-41."""
         tr = self.trainer
         model = tr.model
@@ -94,8 +95,11 @@ class _WholeStepPlan(object):
         bs.set_pooling(model.graph_pooling_type, dev)
         enc_params = _engine.flat_params(model)
         params = [p.detach() for p in enc_params]
-        g_f, d_logit, sv = _engine.run_forward(model, bs, self.neg_idx, True, True, None, params, tr.comm)
         b, m = bs.n_graphs, bs.n_rows
+        self.loss_terms.zero_()                     # [CE mean, beta * BCE mean], float64
+        w_bce = tr.beta / (2.0 * m)                 # main.py:32-37: BCEWithLogits mean over 2m scores, times beta
+        g_f, d_logit, sv = _engine.run_forward(model, bs, self.neg_idx, True, True, None, params, tr.comm,
+                                               bce=(w_bce, w_bce, self.loss_terms[1:2]))
         heads = list(model.linears_prediction)
         n_layers, n_cls, n_feat = len(heads), heads[0].weight.shape[0], heads[0].weight.shape[1]
         hw = [h.weight.detach() for h in heads]
@@ -107,14 +111,15 @@ class _WholeStepPlan(object):
             # F.dropout's keep mask (graphcnn.py:230), one draw for all layers from torch's (CUDA-graph aware) generator
             keep = 1.0 - float(model.final_dropout)
             mask = torch.empty(n_layers, b, n_cls, dtype=torch.float32, device=dev).bernoulli_(keep).mul_(1.0 / keep)
-        self.loss_terms.zero_()                     # [CE mean, beta * BCE mean], float64
         c_logit = torch.empty(b, n_cls, dtype=torch.float32, device=dev)
         d_gf = torch.empty_like(g_f)
         _ops.heads_ce(g_f, hw, hb, mask, self.labels, 1.0 / b, c_logit, self.loss_terms[0:1], d_gf, d_hw, d_hb,
                       self.heads_ws, self.heads_counter)
-        dd = torch.empty(2 * m, 1, dtype=torch.float32, device=dev)
-        w_bce = tr.beta / (2.0 * m)
-        _ops.bce_logits(d_logit.view(-1), m, w_bce, w_bce, self.loss_terms[1:2], dd.view(-1))       # main.py:32-37
+        dd = None
+        if sv.scored is None:
+            # the scoring kernel did not take this shape: BCE forward and backward on the scores here
+            dd = torch.empty(2 * m, 1, dtype=torch.float32, device=dev)
+            _ops.bce_logits(d_logit.view(-1), m, w_bce, w_bce, self.loss_terms[1:2], dd.view(-1))
         _, enc_grads = _engine.run_backward(model, sv, params, d_gf, dd, False, tr.comm)
         tensors, grads = [], []
         for p, g in zip(enc_params, enc_grads):

@@ -561,8 +561,12 @@ def first_argmax_from_padded(h, padded, cmin_values):
     return idx.gather(1, pos).to(torch.int32)
 
 
-def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, max_padded=None):
-    """graphcnn.py:194-251 (and :254-294 when with_dgi is False). Returns (g_f, d_logit, saved)."""
+def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, max_padded=None, bce=None):
+    """graphcnn.py:194-251 (and :254-294 when with_dgi is False). Returns (g_f, d_logit, saved).
+    bce = (grad_scale, loss_scale, loss_acc): the caller's loss on d_logit is BCEWithLogits against main.py:32's targets
+    with these scales (driver.Trainer). The scoring pass then also adds the loss to loss_acc and forms the scorer's
+    backward (saved.scored = (d_score, du, s2, d_bias)) when its kernel takes the shape; saved.scored is None otherwise
+    and the caller applies the loss to d_logit itself."""
     dev = params[0].device
     L, F = model.num_layers, model.hidden_dim
     M, B = bs.n_rows, bs.n_graphs
@@ -576,6 +580,7 @@ def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, m
     sv.training = training
     sv.with_dgi = with_dgi
     sv.x_dense = x_dense
+    sv.scored = None
     h_all = torch.empty(L, M, F, dtype=torch.float32, device=dev)
     g_f = torch.empty(B, L * F, dtype=torch.float32, device=dev)
     sv.h_all = h_all
@@ -673,7 +678,20 @@ def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, m
             neg_table = _ops.gather_nf_rows(h_all, b_neg)
             my_neg = neg_idx
         d_logit = torch.empty(2 * M, 1, dtype=torch.float32, device=dev)
-        _ops.dgi_score_fwd(h_all, u_mat, neg_table, my_neg, bs.node_off, B, disc_b, d_logit)
+        scored = False
+        if bce is not None:
+            # the BCE gradient of a score is local: one pass over n_f forms the scores, the loss and the scorer's
+            # backward (dgi_score_bwd would read the same L slices again)
+            d_score = torch.empty(M, dtype=torch.float32, device=dev)
+            du = torch.empty(B, lf, dtype=torch.float32, device=dev)
+            s2 = torch.empty(B, dtype=torch.float32, device=dev)
+            d_bias = zp.f64(1)[0]
+            scored = _ops.dgi_score_train(h_all, u_mat, neg_table, my_neg, bs.node_off, B, disc_b, bce[0], bce[1],
+                                          d_logit, d_score, du, s2, d_bias, bce[2])
+            if scored:
+                sv.scored = (d_score, du, s2, d_bias)
+        if not scored:
+            _ops.dgi_score_fwd(h_all, u_mat, neg_table, my_neg, bs.node_off, B, disc_b, d_logit)
         sv.c, sv.u_mat, sv.neg_table, sv.my_neg, sv.neg_idx = c, u_mat, neg_table, my_neg, neg_idx
     return g_f, d_logit, sv
 
@@ -729,13 +747,18 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
     d_pooled = dg_f
     d_score = u_mat = d_neg = None
     n_neg = 0
-    if sv.with_dgi and dd_logit is not None:
-        dd = dd_logit.contiguous().view(-1)
-        du = torch.empty(B, L * F, dtype=torch.float32, device=dev)
-        s2 = torch.empty(B, dtype=torch.float32, device=dev)
-        d_bias, c_, o_ = zp.f64(1)
-        from_f64.append((2, c_, o_, 1, False))
-        _ops.dgi_score_bwd(sv.h_all, dd, sv.neg_table, sv.my_neg, bs.node_off, B, du, s2, d_bias)
+    if sv.with_dgi and (dd_logit is not None or sv.scored is not None):
+        if sv.scored is not None:
+            d_score, du, s2, d_bias = sv.scored            # formed by run_forward's scoring pass
+            grads[2] = d_bias.to(torch.float32).view(tuple(params[2].shape))
+        else:
+            dd = dd_logit.contiguous().view(-1)
+            d_score = dd[:M]
+            du = torch.empty(B, L * F, dtype=torch.float32, device=dev)
+            s2 = torch.empty(B, dtype=torch.float32, device=dev)
+            d_bias, c_, o_ = zp.f64(1)
+            from_f64.append((2, c_, o_, 1, False))
+            _ops.dgi_score_bwd(sv.h_all, dd, sv.neg_table, sv.my_neg, bs.node_off, B, du, s2, d_bias)
         # [B, L*F]-sized glue of u = c W^T, c = sigmoid(g_f): dW[i,j] = sum_b du[b,i] c[b,j];
         # d g_f = dg_f (heads) + (du W) c (1 - c); gradient reaching the shuffled rows n_f[perm[g]]
         lf = L * F
@@ -764,7 +787,6 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
                 comm.reduce_sum(d_neg, 0)
                 if comm.rank != 0:
                     d_neg, n_neg = None, 0
-        d_score = dd[:M]
         u_mat = sv.u_mat
     if d_pooled is None:
         d_pooled = torch.zeros(B, L * F, dtype=torch.float32, device=dev)

@@ -11,7 +11,7 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.path.join(CSRC, "libgnm.so")
-ABI_VERSION = 22
+ABI_VERSION = 23
 
 _c_i32 = ctypes.c_int
 _c_i64 = ctypes.c_int64
@@ -72,6 +72,8 @@ SIGNATURES = {
     "gnm_gather_nf_rows": [_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i32, _p, _p],
     "gnm_dgi_score_fwd": [_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i32, _p, _p, _p, _p, _c_i32, _p, _p, _p],
     "gnm_dgi_score_bwd": [_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i32, _p, _p, _p, _p, _c_i32, _p, _p, _p, _p],
+    "gnm_dgi_score_train": [_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i32, _p, _p, _p, _p, _c_i32, _p, _c_f32, _c_f64, _p, _p,
+                            _p, _p, _p, _p, _p],
     "gnm_heads_ce_workspace": [_c_i32, _c_i32, _c_i32, _c_i32],
     "gnm_heads_ce": [_p, _c_i64, _c_i32, _c_i32, _c_i32, _c_i32, _p, _p, _p, _p, _c_f32, _p, _p, _p, _c_i64, _p, _p, _p,
                      _c_i64, _p, _p],

@@ -675,6 +675,24 @@ def dgi_score_bwd(h_all, d_out, neg_table, neg_idx, node_off, n_graphs, du, s2, 
                   "gnm_dgi_score_bwd")
 
 
+def dgi_score_train(h_all, u, neg_table, neg_idx, node_off, n_graphs, bias, grad_scale, loss_scale, out, d_score, du, s2,
+                    d_bias, loss_acc):
+    """dgi_score_fwd + bce_logits + dgi_score_bwd in one pass (include/gnm.h: gnm_dgi_score_train). Returns False, with
+    nothing launched, when the shape does not fit the kernel - make the three calls then."""
+    hp, ls, nl, nf, ldh = _hall(h_all)
+    rc = _lib().gnm_dgi_score_train(hp, ls, nl, nf, ldh, int(h_all.shape[1]), _ptr(u.contiguous(), torch.float32),
+                                    _ptr(neg_table, torch.float32), _ptr(neg_idx, torch.int32), _ptr(node_off, torch.int32),
+                                    n_graphs, _ptr(bias, torch.float32), float(grad_scale), float(loss_scale),
+                                    _ptr(out, torch.float32), _ptr(d_score, torch.float32), _ptr(du, torch.float32),
+                                    _ptr(s2, torch.float32), _ptr(d_bias, torch.float64), _ptr(loss_acc, torch.float64),
+                                    _stream(out))
+    if rc in (-2, -3):                      # GNM_ERR_TOO_LARGE / GNM_ERR_ALIGN: not the kernel's shape
+        LAUNCHES[0] -= 1
+        return False
+    _libmod.check(rc, "gnm_dgi_score_train")
+    return True
+
+
 def rowdot_score(h, u, rows_per_graph, bias, s_bias, out):
     hp, ldh = _mat(h)
     up, ldu = _mat(u)

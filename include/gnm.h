@@ -33,7 +33,7 @@ extern "C" {
 #define GNM_ERR_TOO_LARGE (-2)
 #define GNM_ERR_ALIGN (-3)
 
-#define GNM_ABI_VERSION 22
+#define GNM_ABI_VERSION 23
 
 typedef void* gnm_stream_t;
 
@@ -346,6 +346,20 @@ int gnm_dgi_score_bwd(const float* h_all, int64_t layer_stride, int n_layers, in
                       const float* d_out, const float* neg_table, const int32_t* neg_idx,
                       const int32_t* node_off, int n_graphs, float* du, float* s2, double* d_bias,
                       gnm_stream_t stream);
+
+/* gnm_dgi_score_fwd, BCEWithLogits against the targets of main.py:32 (positives 1, negatives 0) and gnm_dgi_score_bwd
+ * in ONE pass over n_f, for a training step whose loss is the BCE mean (the gradient of a score is local):
+ *   out[r], out[M + r] as gnm_dgi_score_fwd;
+ *   d_score[r] = grad_scale * (sigmoid(out[r]) - 1)              (d_logits[:M] of gnm_bce_logits)
+ *   du, s2, *d_bias += as gnm_dgi_score_bwd with d_out = [d_score, grad_scale * sigmoid(out[M:])];
+ *   *loss_acc += loss_scale * sum_{i < 2M} bce(out[i], y_i).
+ * Arguments as in those calls (d_bias, loss_acc: DEVICE double[1], accumulated). out and d_score are bit-identical to the
+ * three calls, du and s2 equal to fp32 rounding. n_feat == 64 and n_layers <= 5 only (GNM_ERR_TOO_LARGE otherwise),
+ * 16-byte aligned rows (GNM_ERR_ALIGN); nothing is launched then - make the three calls instead. */
+int gnm_dgi_score_train(const float* h_all, int64_t layer_stride, int n_layers, int n_feat, int64_t ldh, int n_rows,
+                        const float* u, const float* neg_table, const int32_t* neg_idx, const int32_t* node_off,
+                        int n_graphs, const float* bias, float grad_scale, double loss_scale, float* out, float* d_score,
+                        float* du, float* s2, double* d_bias, double* loss_acc, gnm_stream_t stream);
 
 /* Standalone Discriminator.forward on materialised tensors (discriminator.py:19-38):
  * out[r] = <h[r], u[r / rows_per_graph]> + *bias (+ s_bias[r] if non-NULL). */

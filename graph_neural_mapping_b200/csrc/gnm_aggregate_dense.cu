@@ -306,12 +306,15 @@ int gnm_launch_aggregate_tc(const int64_t* bitmap_addr, const int32_t* node_off,
                             int n_max, const float* src, int64_t ld_src, const int32_t* src_map, float* dst,
                             int64_t ld_dst, int n_feat, int mode, const float* eps, const float* bias,
                             const float* aff_coef, const float* aff_z, int64_t ld_aff_z, const GnmReluBnBwdFuse* fuse,
-                            int b_shared, double* out_stats, const gnm_bn_tail* tail, cudaStream_t stream);
+                            int b_shared, double* out_stats, const gnm_bn_tail* tail, const float* bn_scale,
+                            const float* bn_shift, float* pooled, int64_t ld_pooled, const float* pool_scale,
+                            cudaStream_t stream);
 
 extern "C" int gnm_aggregate_dense(const int64_t* bitmap_addr, const int32_t* node_off, const int32_t* rowptr,
                                    int n_graphs, int n_max, const float* src, int64_t ld_src, const int32_t* src_map,
                                    float* dst, int64_t ld_dst, int n_feat, int mode, const float* eps,
-                                   const float* bias, int impl, gnm_stream_t stream) {
+                                   const float* bias, int impl, const float* bn_scale, const float* bn_shift,
+                                   float* pooled, int64_t ld_pooled, const float* pool_scale, gnm_stream_t stream) {
     if (n_graphs < 0 || n_max < 0 || n_feat < 0 || mode < 0 || mode > 2) return GNM_ERR_BAD_ARG;
     if (n_graphs == 0 || n_max == 0 || n_feat == 0) return GNM_OK;
     if (!bitmap_addr || !node_off || !src || !dst || (mode != 0 && !rowptr)) return GNM_ERR_BAD_ARG;
@@ -319,10 +322,19 @@ extern "C" int gnm_aggregate_dense(const int64_t* bitmap_addr, const int32_t* no
         (bias && !gnm_aligned16(bias)))
         return GNM_ERR_ALIGN;
     if (impl < 0 || impl > 2) return GNM_ERR_BAD_ARG;
+    if (bn_scale != nullptr || bn_shift != nullptr || pooled != nullptr) {
+        // BatchNorm + ReLU on load (and pooling): the tcgen05 kernel only, nothing launched when it declines
+        if (bn_scale == nullptr || bn_shift == nullptr) return GNM_ERR_BAD_ARG;
+        if (impl == 1) return GNM_ERR_TOO_LARGE;
+        if ((ld_dst % 4) || (pooled != nullptr && ((ld_pooled % 4) || !gnm_aligned16(pooled)))) return GNM_ERR_ALIGN;
+        return gnm_launch_aggregate_tc(bitmap_addr, node_off, rowptr, n_graphs, n_max, src, ld_src, src_map, dst, ld_dst,
+                                       n_feat, mode, eps, bias, nullptr, nullptr, 0, nullptr, 0, nullptr, nullptr, bn_scale,
+                                       bn_shift, pooled, ld_pooled, pool_scale, gnm_cast_stream(stream));
+    }
     if (impl != 1) {
         const int rc = gnm_launch_aggregate_tc(bitmap_addr, node_off, rowptr, n_graphs, n_max, src, ld_src, src_map, dst,
                                                ld_dst, n_feat, mode, eps, bias, nullptr, nullptr, 0, nullptr, 0, nullptr,
-                                               nullptr, gnm_cast_stream(stream));
+                                               nullptr, nullptr, nullptr, nullptr, 0, nullptr, gnm_cast_stream(stream));
         if (rc == GNM_OK || impl == 2 || (rc != GNM_ERR_TOO_LARGE && rc != GNM_ERR_ALIGN)) return rc;
     }
     AggDenseParams p;
@@ -359,7 +371,8 @@ extern "C" int gnm_aggregate_dense_affine(const int64_t* bitmap_addr, const int3
     if (!bitmap_addr || !node_off || !dy || !z || !coef || !dst || (mode != 0 && !rowptr)) return GNM_ERR_BAD_ARG;
     if ((n_feat % 4) || (ld_dy % 4) || (ld_dst % 4) || !gnm_aligned16(dy) || !gnm_aligned16(dst)) return GNM_ERR_ALIGN;
     return gnm_launch_aggregate_tc(bitmap_addr, node_off, rowptr, n_graphs, n_max, dy, ld_dy, nullptr, dst, ld_dst, n_feat,
-                                   mode, nullptr, nullptr, coef, z, ld_z, nullptr, 0, nullptr, nullptr, gnm_cast_stream(stream));
+                                   mode, nullptr, nullptr, coef, z, ld_z, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr,
+                                   0, nullptr, gnm_cast_stream(stream));
 }
 
 /* Layer 0 on one-hot inputs when every graph of the batch carries the SAME injective tag sequence (util.py:106-116: one
@@ -381,8 +394,8 @@ extern "C" int gnm_aggregate_dense_table(const int64_t* bitmap_addr, const int32
         (bias && !gnm_aligned16(bias)))
         return GNM_ERR_ALIGN;
     return gnm_launch_aggregate_tc(bitmap_addr, node_off, rowptr, n_graphs, n_max, table, ld_table, tags, dst, ld_dst,
-                                   n_feat, mode, eps, bias, nullptr, nullptr, 0, nullptr, 1, out_stats, tail,
-                                   gnm_cast_stream(stream));
+                                   n_feat, mode, eps, bias, nullptr, nullptr, 0, nullptr, 1, out_stats, tail, nullptr,
+                                   nullptr, nullptr, 0, nullptr, gnm_cast_stream(stream));
 }
 
 /* Backward aggregation fused with its consumer: dy = relu'(bn(z)) * (Agg(src) [+ (1+eps) src] + d_pooled[g]*pool_scale[g]
@@ -408,5 +421,6 @@ extern "C" int gnm_aggregate_dense_relu_bn_bwd(const int64_t* bitmap_addr, const
     f.ld_dpooled = ld_dpooled; f.pool_scale = pool_scale; f.d_score = d_score; f.u = u; f.ldu = ldu; f.d_neg = d_neg;
     f.ld_dneg = ld_dneg; f.n_neg = n_neg; f.stats = stats;
     return gnm_launch_aggregate_tc(bitmap_addr, node_off, rowptr, n_graphs, n_max, src, ld_src, nullptr, dy, lddy, n_feat,
-                                   mode, eps, nullptr, nullptr, nullptr, 0, &f, 0, nullptr, tail, gnm_cast_stream(stream));
+                                   mode, eps, nullptr, nullptr, nullptr, 0, &f, 0, nullptr, tail, nullptr, nullptr, nullptr, 0,
+                                   nullptr, gnm_cast_stream(stream));
 }

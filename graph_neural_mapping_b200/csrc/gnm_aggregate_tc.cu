@@ -24,7 +24,9 @@
 //     of an item are written chunk by chunk together with the A stages of its first row tile; item parameters and the
 //     next item's first loads are requested one item / one row tile ahead.
 //   * optional fusions on the same kernel: a per-column affine of two streams applied to the B rows on load
-//     (gnm_aggregate_dense_affine) and a consumer of the output rows in the copy-out (gnm_aggregate_dense_relu_bn_bwd).
+//     (gnm_aggregate_dense_affine), BatchNorm + ReLU of the layer below applied to the B rows on load together with
+//     that layer's graph pooling (gnm_aggregate_dense with bn_scale), and a consumer of the output rows in the copy-out
+//     (gnm_aggregate_dense_relu_bn_bwd).
 //   * every wait is bounded: on a timeout the kernel raises an abort flag and drains instead of hanging.
 #include <cuda_bf16.h>
 
@@ -83,14 +85,20 @@ struct AggTcParams {
     // [k_lo, k_lo + k_pass) of every graph; accumulate != 0 adds the result to what dst already holds
     int k_lo, k_pass, accumulate;
     BnTailDev tail;              // BatchNorm tail on out_stats (forward) or r_stats (fused backward); kind 0: none
+    // TCV_BN: the source rows are the pre-BatchNorm output z of the layer below; h = relu(z*bn_scale + bn_shift) is
+    // formed when a chunk is converted into the B planes, and pooled (nullable) receives the graph's column sums of h
+    // (times pool_scale[g], nullable) - the readout of the layer below, from the rows the producers load anyway
+    const float* bn_scale; const float* bn_shift;
+    float* pooled; int64_t ld_pooled; const float* pool_scale;
     long long* dbg;              // nullable: per-CTA wait/busy cycle counters (profiling aid)
 };
 
 // VAR: which optional paths this instantiation carries (the others are compiled out: the three roles run different code
 // at the same time, and the all-in-one kernel - 81 KB of SASS - lost 20 % to instruction fetch and dead branches):
 //   TCV_FUSE relu / BatchNorm-backward consumer in the copy-out, TCV_AFF affine of two streams on the B rows,
-//   TCV_MAP row map / bias / shared table / output statistics (layer 0), TCV_EPS (1 + eps) self term, TCV_AVG degree weights.
-enum { TCV_FUSE = 1, TCV_AFF = 2, TCV_MAP = 4, TCV_EPS = 8, TCV_AVG = 16, TCV_ALL = 31, TCV_KSPLIT = 32 };
+//   TCV_MAP row map / bias / shared table / output statistics (layer 0), TCV_EPS (1 + eps) self term, TCV_AVG degree weights,
+//   TCV_BN BatchNorm + ReLU of the source on load and graph pooling of the activated rows (sum pooling, one slab, alone).
+enum { TCV_FUSE = 1, TCV_AFF = 2, TCV_MAP = 4, TCV_EPS = 8, TCV_AVG = 16, TCV_ALL = 31, TCV_KSPLIT = 32, TCV_BN = 64 };
 
 // bulk prefetch of [ptr, ptr + bytes) into L2 (no destination, no completion tracking); 16-byte granularity
 __device__ __forceinline__ void l2_prefetch(const void* ptr, int64_t bytes) {
@@ -102,10 +110,11 @@ __device__ __forceinline__ void l2_prefetch(const void* ptr, int64_t bytes) {
 template <bool DBG, int VAR>
 __global__ void __launch_bounds__(TC_THREADS, 1) aggregate_tc_kernel(const AggTcParams p) {
     constexpr bool kFuse = (VAR & TCV_FUSE) != 0, kAff = (VAR & TCV_AFF) != 0, kMap = (VAR & TCV_MAP) != 0,
-                   kEps = (VAR & TCV_EPS) != 0, kAvg = (VAR & TCV_AVG) != 0, kSplit = (VAR & TCV_KSPLIT) != 0;
+                   kEps = (VAR & TCV_EPS) != 0, kAvg = (VAR & TCV_AVG) != 0, kSplit = (VAR & TCV_KSPLIT) != 0,
+                   kBn = (VAR & TCV_BN) != 0;
     const int k_lo = kSplit ? p.k_lo : 0;
     extern __shared__ __align__(1024) unsigned char tc_smem[];
-    __shared__ __align__(8) uint64_t bars[2 * TC_STAGES + 6];
+    __shared__ __align__(8) uint64_t bars[2 * TC_STAGES + 10];
     __shared__ uint32_t s_tmem;
     __shared__ int s_abort;
     uint64_t* a_full = bars;
@@ -114,6 +123,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) aggregate_tc_kernel(const AggTc
     uint64_t* acc_empty = acc_full + 2;
     uint64_t* b_full = acc_empty + 2;
     uint64_t* b_free = b_full + 1;
+    uint64_t* pool_full = b_free + 1;     // [2] TCV_BN pooling: the producers' partial column sums of an item are in place
+    uint64_t* pool_empty = pool_full + 2; // [2] ... and have been read (partials double-buffered by item parity)
     const int b_ncore_stride = p.kcores_max * 128 + 16;            // SBO of B (padded: conflict-free plane fill)
     unsigned char* sm_b = tc_smem;                                  // 24 n-cores x b_ncore_stride
     float* sm_stg = reinterpret_cast<float*>(tc_smem + (size_t)24 * b_ncore_stride);   // TC_EPI_WARPS staging tiles
@@ -128,6 +139,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) aggregate_tc_kernel(const AggTc
     // affine variant only: landing area of the second stream's rows (cp.async, eight 16-byte slots per producer thread)
     float4* sm_aff = reinterpret_cast<float4*>(tc_smem + (size_t)24 * b_ncore_stride + TC_EPI_WARPS * TC_STG + 4096 +
                                                ((kFuse && p.rz != nullptr) ? TC_EPI_WARPS * TC_STG : 0));
+    // pooling variant only: [2 item parities][8 producer warps][64 columns] partial column sums of the activated rows
+    float* sm_pool = reinterpret_cast<float*>(tc_smem + (size_t)24 * b_ncore_stride + TC_EPI_WARPS * TC_STG + 4096);
+    const bool pool_on = kBn && p.pooled != nullptr;
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     pdl_launch_dependents();
@@ -142,6 +156,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) aggregate_tc_kernel(const AggTc
         for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 4); }
         mbar_init(b_full, TC_PROD_WARPS);
         mbar_init(b_free, 1);
+        for (int i = 0; i < 2; ++i) { mbar_init(&pool_full[i], TC_PROD_WARPS); mbar_init(&pool_empty[i], 2); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == TC_MMA_WARP) {
@@ -161,7 +176,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) aggregate_tc_kernel(const AggTc
         // plane accumulators of its 32 rows, stages them in shared memory and copies them out with coalesced 128-bit
         // stores (a row-per-lane store costs 32 L1 wavefronts per instruction); the eps self term and the bias are
         // added during the copy-out, where the source rows are read coalesced as well.
-        uint32_t acc_it = 0;
+        uint32_t acc_it = 0, pool_it = 0;
         long long w_acc = 0, c_drain = 0, c_copy = 0;
         const long long t_role = clock64();
         const float self_c = (kEps && p.eps) ? 1.f + __ldg(p.eps) : 0.f;
@@ -399,6 +414,22 @@ __global__ void __launch_bounds__(TC_THREADS, 1) aggregate_tc_kernel(const AggTc
                 }
                 if (DBG) c_copy += clock64() - t_d1;
             }
+            if (pool_on && warp < 2) {
+                // graph pooling of the layer below: the eight producer warps' partial column sums of this item (complete
+                // once its first row tile was converted), added in a fixed order - one lane per column, no atomics
+                const uint32_t pb = pool_it & 1, pph = (pool_it >> 1) & 1;
+                if (!mbar_wait<32>(&pool_full[pb], pph, abort_flag)) break;
+                const int c = warp * 32 + lane;
+                const float* part = sm_pool + pb * (TC_PROD_WARPS * TC_SLAB) + c;
+                float t = 0.f;
+#pragma unroll
+                for (int w = 0; w < TC_PROD_WARPS; ++w) t += part[w * TC_SLAB];
+                if (p.pool_scale != nullptr) t *= __ldg(p.pool_scale + gi);
+                if (f0 + c < p.n_feat) p.pooled[(int64_t)gi * p.ld_pooled + f0 + c] = t;
+                __syncwarp();
+                if (lane == 0) mbar_arrive(&pool_empty[pb]);
+            }
+            ++pool_it;
         }
         double* const stats_out = ostats ? p.out_stats : (fuse ? p.r_stats : nullptr);
         if (stats_out != nullptr) {
@@ -533,7 +564,23 @@ __global__ void __launch_bounds__(TC_THREADS, 1) aggregate_tc_kernel(const AggTc
         float4 bq[8];
         // affine variant: this thread's column never changes within a slab - its coefficients live in registers
         float4 aff_a = make_float4(0.f, 0.f, 0.f, 0.f), aff_b = aff_a, aff_c = aff_a;
+        float4 bn_sc = aff_a, bn_sh = aff_a;                 // BatchNorm variant: the same, for scale / shift
         int aff_col = -1;
+        // pooling variant: this thread's share of the item's column sums (its column, rows kbase + 8u of the chunks it
+        // converts), folded with lane l ^ 16 and parked per warp for the epilogue (pool_full / pool_empty, by item parity)
+        float4 pacc = aff_a;
+        uint32_t pool_it = 0;
+        auto put_pool = [&](float4 v) -> bool {
+            const uint32_t pb = pool_it & 1, pph = (pool_it >> 1) & 1;
+            ++pool_it;
+            v.x += __shfl_xor_sync(GNM_FULL_MASK, v.x, 16); v.y += __shfl_xor_sync(GNM_FULL_MASK, v.y, 16);
+            v.z += __shfl_xor_sync(GNM_FULL_MASK, v.z, 16); v.w += __shfl_xor_sync(GNM_FULL_MASK, v.w, 16);
+            if (!mbar_wait<32>(&pool_empty[pb], pph ^ 1, abort_flag)) return false;
+            if (lane < 16) *reinterpret_cast<float4*>(sm_pool + pb * (TC_PROD_WARPS * TC_SLAB) + (ptid >> 5) * TC_SLAB + lane * 4) = v;
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&pool_full[pb]);
+            return true;
+        };
         // The second stream (aff_z) lands in shared memory through cp.async and meets the first (registers, bq) only when
         // the chunk is converted: forming cA*src + cB*z + cC right behind the loads made every chunk wait for DRAM
         // (B fill 130 k of 292 k cycles per CTA, 164 us per launch against 96 us for the plain variant).
@@ -548,6 +595,11 @@ __global__ void __launch_bounds__(TC_THREADS, 1) aggregate_tc_kernel(const AggTc
                 aff_a = __ldg(reinterpret_cast<const float4*>(p.aff_coef + col));
                 aff_b = __ldg(reinterpret_cast<const float4*>(p.aff_coef + p.n_feat + col));
                 aff_c = __ldg(reinterpret_cast<const float4*>(p.aff_coef + 2 * p.n_feat + col));
+                aff_col = col;
+            }
+            if (kBn && ok0 && aff_col != col) {
+                bn_sc = __ldg(reinterpret_cast<const float4*>(p.bn_scale + col));
+                bn_sh = __ldg(reinterpret_cast<const float4*>(p.bn_shift + col));
                 aff_col = col;
             }
             // a chunk that was requested but never converted (a group without a chunk in a one-chunk graph) must not
@@ -663,6 +715,22 @@ __global__ void __launch_bounds__(TC_THREADS, 1) aggregate_tc_kernel(const AggTc
                                 bq[u] = v;
                             }
                         }
+                        if (kBn) {
+                            // h = relu(z*scale + shift) with the readout's expression: bit-identical to aggregating the
+                            // materialised h. Rows past the graph and columns past n_feat were loaded as 0, and
+                            // relu(0*scale + shift) is not 0: they are zeroed AFTER the affine, for the planes and the sums
+                            const bool col_in = lb_c4 * 4 + cur.f0 < p.n_feat;
+#pragma unroll
+                            for (int u = 0; u < 8; ++u) {
+                                const int k = kc * TC_KC + lb_kr + u * 8;
+                                float4 v = bq[u];
+                                v.x = fmaxf(fmaf(v.x, bn_sc.x, bn_sh.x), 0.f); v.y = fmaxf(fmaf(v.y, bn_sc.y, bn_sh.y), 0.f);
+                                v.z = fmaxf(fmaf(v.z, bn_sc.z, bn_sh.z), 0.f); v.w = fmaxf(fmaf(v.w, bn_sc.w, bn_sh.w), 0.f);
+                                if (k >= cur.nk || !col_in) v = make_float4(0.f, 0.f, 0.f, 0.f);
+                                if (pool_on) { pacc.x += v.x; pacc.y += v.y; pacc.z += v.z; pacc.w += v.w; }
+                                bq[u] = v;
+                            }
+                        }
 #pragma unroll
                         for (int u = 0; u < 8; ++u) {
                             const int k = kc * TC_KC + lb_kr + u * 8, c4 = lb_c4;
@@ -707,11 +775,16 @@ __global__ void __launch_bounds__(TC_THREADS, 1) aggregate_tc_kernel(const AggTc
                     if (lane == 0) mbar_arrive(&a_full[s]);
                     if (DBG) { const long long tq3 = clock64(); c_st += tq1 - tq0; c_arr += tq3 - tq1; }
                 }
+                if (pool_on && mt == 0 && ok) {
+                    ok = put_pool(pacc);
+                    pacc = make_float4(0.f, 0.f, 0.f, 0.f);
+                }
                 const long long tt1 = DBG ? clock64() : 0;
 #pragma unroll
                 for (int c = 0; c < MYC; ++c) { w_cur[c][0] = w_nxt[c][0]; w_cur[c][1] = w_nxt[c][1]; }
                 if (DBG) c_bload += clock64() - tt1;                // tile tail: the prefetched words must have arrived
             }
+            if (pool_on && n_mt == 0 && ok) ok = put_pool(make_float4(0.f, 0.f, 0.f, 0.f));     // empty graph: sums 0
             prev_nkc = n_kc;
             if (!preloaded) derive_item(nxt);
             cur = nxt;
@@ -747,7 +820,17 @@ int gnm_launch_aggregate_tc(const int64_t* bitmap_addr, const int32_t* node_off,
                             int n_max, const float* src, int64_t ld_src, const int32_t* src_map, float* dst,
                             int64_t ld_dst, int n_feat, int mode, const float* eps, const float* bias,
                             const float* aff_coef, const float* aff_z, int64_t ld_aff_z, const GnmReluBnBwdFuse* fuse,
-                            int b_shared, double* out_stats, const gnm_bn_tail* tail, cudaStream_t stream) {
+                            int b_shared, double* out_stats, const gnm_bn_tail* tail, const float* bn_scale,
+                            const float* bn_shift, float* pooled, int64_t ld_pooled, const float* pool_scale,
+                            cudaStream_t stream) {
+    if (bn_scale != nullptr) {
+        // BatchNorm + ReLU on load (+ pooling): single pass, sum pooling, one slab, no self term / row map / other fusion
+        if (bn_shift == nullptr) return GNM_ERR_BAD_ARG;
+        if (n_max > TC_MAX_NODES || n_feat > TC_SLAB || mode != 0 || eps != nullptr || src_map != nullptr || bias != nullptr ||
+            fuse != nullptr || aff_coef != nullptr || b_shared || out_stats != nullptr || tail != nullptr)
+            return GNM_ERR_TOO_LARGE;
+        if (!gnm_aligned16(bn_scale) || !gnm_aligned16(bn_shift)) return GNM_ERR_ALIGN;
+    }
     // graphs above TC_MAX_NODES nodes: K-split passes (plain / eps / row-map variants of sum pooling and of the transposed
     // average, mode 2); the fused consumers, the shared table and the forward average (division of the TOTAL) stay single-pass
     const bool ksplit = n_max > TC_MAX_NODES;
@@ -792,6 +875,8 @@ int gnm_launch_aggregate_tc(const int64_t* bitmap_addr, const int32_t* node_off,
     }
     p.b_shared = b_shared; p.out_stats = out_stats;
     p.k_lo = 0; p.k_pass = 0; p.accumulate = 0;
+    p.bn_scale = bn_scale; p.bn_shift = bn_shift;
+    p.pooled = bn_scale != nullptr ? pooled : nullptr; p.ld_pooled = ld_pooled; p.pool_scale = pool_scale;
     const int trc = bn_tail_args(tail, out_stats != nullptr ? out_stats : (fuse ? fuse->stats : nullptr), n_feat, &p.tail);
     if (trc != GNM_OK) return trc;
     p.dbg = g_tc_dbg_host;
@@ -799,7 +884,7 @@ int gnm_launch_aggregate_tc(const int64_t* bitmap_addr, const int32_t* node_off,
     p.kcores_max = (((ksplit ? TC_K_PASS : n_max) + 15) / 16) * 2;
     // B planes + staging + LUT (+ the z tiles of the fused relu / BatchNorm backward)
     const int smem = 24 * (p.kcores_max * 128 + 16) + TC_EPI_WARPS * TC_STG + 4096 + 1024 + (fuse ? TC_EPI_WARPS * TC_STG : 0) +
-                     (aff_coef ? TC_PROD_WARPS * 32 * 8 * 16 : 0);
+                     (aff_coef ? TC_PROD_WARPS * 32 * 8 * 16 : 0) + (p.pooled ? 2 * TC_PROD_WARPS * TC_SLAB * 4 : 0);
     if (smem > smem_cap - 1024) return GNM_ERR_TOO_LARGE;
     const int64_t items = (int64_t)n_graphs * p.n_slabs;
     const int grid = (int)(items < sms ? items : sms);
@@ -820,6 +905,10 @@ int gnm_launch_aggregate_tc(const int64_t* bitmap_addr, const int32_t* node_off,
             if (e != cudaSuccess) return (int)e;
         }
         return GNM_OK;
+    }
+    if (bn_scale != nullptr) {
+        e = p.dbg != nullptr ? launch_variant<true, TCV_BN>(p, grid, smem, stream) : launch_variant<false, TCV_BN>(p, grid, smem, stream);
+        return e == cudaSuccess ? GNM_OK : (int)e;
     }
     if (p.dbg != nullptr) {
         e = var == 0 ? launch_variant<true, 0>(p, grid, smem, stream)

@@ -9,14 +9,35 @@ namespace {
 
 constexpr int kMaxFeatPerLane = 32;   // n_h = L*F up to 1024
 
+// bn (nullable): h_all holds each layer's PRE-BatchNorm output z and every value is read as h = relu(z*scale + shift),
+// scale / shift of layer l at bn + l*ld_bn and bn + l*ld_bn + n_feat - gnm_bn_relu_readout's expression, so the result is
+// bit-identical to reading the h it would have written
+__device__ __forceinline__ float bn_relu(float z, float sc, float sh) { return fmaxf(fmaf(z, sc, sh), 0.f); }
+__device__ __forceinline__ float4 bn_relu4(float4 z, float4 sc, float4 sh) {
+    return make_float4(bn_relu(z.x, sc.x, sh.x), bn_relu(z.y, sc.y, sh.y), bn_relu(z.z, sc.z, sh.z), bn_relu(z.w, sc.w, sh.w));
+}
+
 __global__ void gather_nf_rows_kernel(const float* __restrict__ h_all, int64_t layer_stride, int n_layers, int n_feat,
-                                      int64_t ldh, int n_rows, float* __restrict__ table) {
+                                      int64_t ldh, int n_rows, const float* __restrict__ bn, int64_t ld_bn,
+                                      float* __restrict__ table) {
     const int nh = n_layers * n_feat;
     const int64_t total = (int64_t)n_rows * nh;
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int r = (int)(i / nh), c = (int)(i % nh);
         const int l = c / n_feat, f = c % n_feat;
-        table[i] = h_all[l * layer_stride + (int64_t)r * ldh + f];
+        float v = h_all[l * layer_stride + (int64_t)r * ldh + f];
+        if (bn != nullptr) v = bn_relu(v, bn[l * ld_bn + f], bn[l * ld_bn + n_feat + f]);
+        table[i] = v;
+    }
+}
+
+// the [2][nh] table of scale | shift per (layer, feature) in shared memory, laid out like u_g
+__device__ __forceinline__ void stage_bn(const float* __restrict__ bn, int64_t ld_bn, int n_layers, int n_feat, float* sbn) {
+    const int nh = n_layers * n_feat;
+    for (int i = threadIdx.x; i < nh; i += blockDim.x) {
+        const int l = i / n_feat, f = i % n_feat;
+        sbn[i] = bn[l * ld_bn + f];
+        sbn[nh + i] = bn[l * ld_bn + n_feat + f];
     }
 }
 
@@ -35,13 +56,15 @@ __global__ void __launch_bounds__(256)
 dgi_score_fwd_kernel(const float* __restrict__ h_all, int64_t layer_stride, int n_layers, int n_feat, int64_t ldh,
                      int n_rows, const float* __restrict__ u, const float* __restrict__ neg_table,
                      const int32_t* __restrict__ neg_idx, const int32_t* __restrict__ node_off,
-                     const float* __restrict__ bias, float* __restrict__ out) {
-    extern __shared__ __align__(16) float us[];    // [n_layers * n_feat]
+                     const float* __restrict__ bias, const float* __restrict__ bn, int64_t ld_bn, float* __restrict__ out) {
+    extern __shared__ __align__(16) float us[];    // [n_layers * n_feat] (+ [2][n_layers * n_feat] scale | shift with bn)
     __shared__ float s_neg;
     const int g = blockIdx.x;
     const int nh = n_layers * n_feat;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    float* sbn = us + nh;
     for (int i = threadIdx.x; i < nh; i += blockDim.x) us[i] = u[(int64_t)g * nh + i];
+    if (bn != nullptr) stage_bn(bn, ld_bn, n_layers, n_feat, sbn);
     __syncthreads();
     const float b = bias ? __ldg(bias) : 0.f;
     if (warp == 0) {
@@ -66,7 +89,10 @@ dgi_score_fwd_kernel(const float* __restrict__ h_all, int64_t layer_stride, int 
                 const float* ul = us + sub * 4;
 #pragma unroll 5
                 for (int l = 0; l < n_layers; ++l) {
-                    const float4 hv = ld_stream_f4(hr + l * layer_stride);
+                    float4 hv = ld_stream_f4(hr + l * layer_stride);
+                    if (bn != nullptr)
+                        hv = bn_relu4(hv, *reinterpret_cast<const float4*>(sbn + l * n_feat + sub * 4),
+                                      *reinterpret_cast<const float4*>(sbn + nh + l * n_feat + sub * 4));
                     const float4 uv = *reinterpret_cast<const float4*>(ul + l * n_feat);
                     a = fmaf(hv.x, uv.x, a); a = fmaf(hv.y, uv.y, a); a = fmaf(hv.z, uv.z, a); a = fmaf(hv.w, uv.w, a);
                 }
@@ -83,7 +109,11 @@ dgi_score_fwd_kernel(const float* __restrict__ h_all, int64_t layer_stride, int 
             for (int l = 0; l < n_layers; ++l) {
                 const float* hr = h_all + l * layer_stride + (int64_t)r * ldh;
                 const float* ul = us + l * n_feat;
-                for (int f = lane; f < n_feat; f += 32) a = fmaf(hr[f], ul[f], a);
+                for (int f = lane; f < n_feat; f += 32) {
+                    float hv = hr[f];
+                    if (bn != nullptr) hv = bn_relu(hv, sbn[l * n_feat + f], sbn[nh + l * n_feat + f]);
+                    a = fmaf(hv, ul[f], a);
+                }
             }
             a = warp_sum(a);
             if (lane == 0) {
@@ -98,15 +128,21 @@ __global__ void __launch_bounds__(256)
 dgi_score_bwd_kernel(const float* __restrict__ h_all, int64_t layer_stride, int n_layers, int n_feat, int64_t ldh,
                      int n_rows, const float* __restrict__ d_out, const float* __restrict__ neg_table,
                      const int32_t* __restrict__ neg_idx, const int32_t* __restrict__ node_off,
+                     const float* __restrict__ bn, int64_t ld_bn,
                      float* __restrict__ du, float* __restrict__ s2, double* __restrict__ d_bias) {
-    extern __shared__ float acc_s[];   // [8][nh] per-warp partial du
+    extern __shared__ float acc_s[];   // [8][nh] per-warp partial du (+ [2][nh] scale | shift with bn)
     __shared__ float red[2][8];
     const int g = blockIdx.x;
     const int nh = n_layers * n_feat;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int r0 = node_off[g], r1 = node_off[g + 1];
     float* mine = acc_s + warp * nh;
+    float* sbn = acc_s + 8 * nh;
     for (int i = lane; i < nh; i += 32) mine[i] = 0.f;
+    if (bn != nullptr) {
+        stage_bn(bn, ld_bn, n_layers, n_feat, sbn);
+        __syncthreads();
+    }
     __syncwarp();
     float sum1 = 0.f, sum2 = 0.f;
     for (int r = r0 + warp; r < r1; r += 8) {
@@ -115,7 +151,11 @@ dgi_score_bwd_kernel(const float* __restrict__ h_all, int64_t layer_stride, int 
         for (int l = 0; l < n_layers; ++l) {
             const float* hr = h_all + l * layer_stride + (int64_t)r * ldh;
             float* ml = mine + l * n_feat;
-            for (int f = lane; f < n_feat; f += 32) ml[f] = fmaf(d1, hr[f], ml[f]);
+            for (int f = lane; f < n_feat; f += 32) {
+                float hv = hr[f];
+                if (bn != nullptr) hv = bn_relu(hv, sbn[l * n_feat + f], sbn[nh + l * n_feat + f]);
+                ml[f] = fmaf(d1, hv, ml[f]);
+            }
         }
     }
     sum1 = warp_sum(sum1);
@@ -143,14 +183,20 @@ __global__ void __launch_bounds__(256)
 dgi_score_bwd_vec_kernel(const float* __restrict__ h_all, int64_t layer_stride, int64_t ldh, int n_rows,
                          const float* __restrict__ d_out, const float* __restrict__ neg_table,
                          const int32_t* __restrict__ neg_idx, const int32_t* __restrict__ node_off,
+                         const float* __restrict__ bn, int64_t ld_bn,
                          float* __restrict__ du, float* __restrict__ s2, double* __restrict__ d_bias) {
     constexpr int F = 64, NH = NL * F;
     __shared__ __align__(16) float part[8][NH];
+    __shared__ __align__(16) float sbn[2 * NH];
     __shared__ float red[2][8];
     const int g = blockIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int half = lane >> 4, c4 = lane & 15;
     const int r0 = node_off[g], r1 = node_off[g + 1];
+    if (bn != nullptr) {
+        stage_bn(bn, ld_bn, NL, F, sbn);
+        __syncthreads();
+    }
     float4 acc[NL];
 #pragma unroll
     for (int l = 0; l < NL; ++l) acc[l] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -162,6 +208,12 @@ dgi_score_bwd_vec_kernel(const float* __restrict__ h_all, int64_t layer_stride, 
         float4 hv[NL];
 #pragma unroll
         for (int l = 0; l < NL; ++l) hv[l] = ld_stream_f4(hr + l * layer_stride);
+        if (bn != nullptr) {
+#pragma unroll
+            for (int l = 0; l < NL; ++l)
+                hv[l] = bn_relu4(hv[l], *reinterpret_cast<const float4*>(sbn + l * F + c4 * 4),
+                                 *reinterpret_cast<const float4*>(sbn + NH + l * F + c4 * 4));
+        }
 #pragma unroll
         for (int l = 0; l < NL; ++l) {
             acc[l].x = fmaf(d1, hv[l].x, acc[l].x); acc[l].y = fmaf(d1, hv[l].y, acc[l].y);
@@ -205,11 +257,12 @@ __global__ void __launch_bounds__(256)
 dgi_score_train_kernel(const float* __restrict__ h_all, int64_t layer_stride, int64_t ldh, int n_rows,
                        const float* __restrict__ u, const float* __restrict__ neg_table,
                        const int32_t* __restrict__ neg_idx, const int32_t* __restrict__ node_off,
-                       const float* __restrict__ bias, float grad_scale, double loss_scale, float* __restrict__ out,
-                       float* __restrict__ d_score, float* __restrict__ du, float* __restrict__ s2,
-                       double* __restrict__ d_bias, double* __restrict__ loss_acc) {
+                       const float* __restrict__ bias, const float* __restrict__ bn, int64_t ld_bn, float grad_scale,
+                       double loss_scale, float* __restrict__ out, float* __restrict__ d_score, float* __restrict__ du,
+                       float* __restrict__ s2, double* __restrict__ d_bias, double* __restrict__ loss_acc) {
     constexpr int F = 64, NH = NL * F;
     __shared__ __align__(16) float us[NH];
+    __shared__ __align__(16) float sbn[2 * NH];     // bn: scale | shift (shared memory, not 2 NL float4 registers)
     __shared__ __align__(16) float part[8][NH];
     __shared__ float red[2][8];
     __shared__ double lred[8];
@@ -218,6 +271,7 @@ dgi_score_train_kernel(const float* __restrict__ h_all, int64_t layer_stride, in
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int half = lane >> 4, c4 = lane & 15;
     for (int i = threadIdx.x; i < NH; i += blockDim.x) us[i] = u[(int64_t)g * NH + i];
+    if (bn != nullptr) stage_bn(bn, ld_bn, NL, F, sbn);
     __syncthreads();
     const float b = bias ? __ldg(bias) : 0.f;
     const float* nr = neg_table + (int64_t)neg_idx[g] * NH;
@@ -246,6 +300,12 @@ dgi_score_train_kernel(const float* __restrict__ h_all, int64_t layer_stride, in
             const float* hr = h_all + (int64_t)r * ldh + c4 * 4;
 #pragma unroll
             for (int l = 0; l < NL; ++l) hv[l] = ld_stream_f4(hr + l * layer_stride);
+            if (bn != nullptr) {
+#pragma unroll
+                for (int l = 0; l < NL; ++l)
+                    hv[l] = bn_relu4(hv[l], *reinterpret_cast<const float4*>(sbn + l * F + c4 * 4),
+                                     *reinterpret_cast<const float4*>(sbn + NH + l * F + c4 * 4));
+            }
 #pragma unroll
             for (int l = 0; l < NL; ++l) {
                 const float4 uv = *reinterpret_cast<const float4*>(us + l * F + c4 * 4);
@@ -318,7 +378,7 @@ rowdot_score_kernel(const float* __restrict__ h, int64_t ldh, int n_rows, int n_
 }  // namespace
 
 extern "C" int gnm_gather_nf_rows(const float* h_all, int64_t layer_stride, int n_layers, int n_feat, int64_t ldh,
-                                  int n_rows, float* table, gnm_stream_t stream) {
+                                  int n_rows, const float* bn, int64_t ld_bn, float* table, gnm_stream_t stream) {
     if (n_layers < 0 || n_feat < 0 || n_rows < 0) return GNM_ERR_BAD_ARG;
     if (n_layers == 0 || n_feat == 0 || n_rows == 0) return GNM_OK;
     if (!h_all || !table) return GNM_ERR_BAD_ARG;
@@ -327,19 +387,19 @@ extern "C" int gnm_gather_nf_rows(const float* h_all, int64_t layer_stride, int 
     if (blocks > 148 * 8) blocks = 148 * 8;
     gnm_count_launch(GNM_K_OTHER);
     gather_nf_rows_kernel<<<(int)blocks, 256, 0, gnm_cast_stream(stream)>>>(h_all, layer_stride, n_layers, n_feat, ldh,
-                                                                            n_rows, table);
+                                                                            n_rows, bn, ld_bn, table);
     GNM_RETURN_IF_LAUNCH_FAILED();
     return GNM_OK;
 }
 
 extern "C" int gnm_dgi_score_fwd(const float* h_all, int64_t layer_stride, int n_layers, int n_feat, int64_t ldh,
                                  int n_rows, const float* u, const float* neg_table, const int32_t* neg_idx,
-                                 const int32_t* node_off, int n_graphs, const float* bias, float* out,
-                                 gnm_stream_t stream) {
+                                 const int32_t* node_off, int n_graphs, const float* bias, const float* bn, int64_t ld_bn,
+                                 float* out, gnm_stream_t stream) {
     if (n_layers < 0 || n_feat < 0 || n_rows < 0 || n_graphs < 0) return GNM_ERR_BAD_ARG;
     if (n_graphs == 0 || n_rows == 0) return GNM_OK;
     if (!h_all || !u || !neg_table || !neg_idx || !node_off || !out) return GNM_ERR_BAD_ARG;
-    const size_t smem = (size_t)n_layers * n_feat * 4;
+    const size_t smem = (size_t)n_layers * n_feat * 4 * (bn != nullptr ? 3 : 1);
     if (smem > 48 * 1024) return GNM_ERR_TOO_LARGE;
     const int q = n_feat / 4;
     const bool vec = (n_feat % 4 == 0) && (q & (q - 1)) == 0 && q <= 32 && (ldh % 4 == 0) && (layer_stride % 4 == 0) &&
@@ -348,7 +408,7 @@ extern "C" int gnm_dgi_score_fwd(const float* h_all, int64_t layer_stride, int n
     do { gnm_count_launch(GNM_K_OTHER); \
     dgi_score_fwd_kernel<LPR><<<n_graphs, 256, smem, gnm_cast_stream(stream)>>>(h_all, layer_stride, n_layers, n_feat, \
                                                                                  ldh, n_rows, u, neg_table, neg_idx,   \
-                                                                                 node_off, bias, out); } while (0)
+                                                                                 node_off, bias, bn, ld_bn, out); } while (0)
     if (!vec) GNM_DGI_FWD(0);
     else if (q == 1) GNM_DGI_FWD(1);
     else if (q == 2) GNM_DGI_FWD(2);
@@ -363,8 +423,8 @@ extern "C" int gnm_dgi_score_fwd(const float* h_all, int64_t layer_stride, int n
 
 extern "C" int gnm_dgi_score_bwd(const float* h_all, int64_t layer_stride, int n_layers, int n_feat, int64_t ldh,
                                  int n_rows, const float* d_out, const float* neg_table, const int32_t* neg_idx,
-                                 const int32_t* node_off, int n_graphs, float* du, float* s2, double* d_bias,
-                                 gnm_stream_t stream) {
+                                 const int32_t* node_off, int n_graphs, const float* bn, int64_t ld_bn, float* du, float* s2,
+                                 double* d_bias, gnm_stream_t stream) {
     if (n_layers < 0 || n_feat < 0 || n_rows < 0 || n_graphs < 0) return GNM_ERR_BAD_ARG;
     if (n_graphs == 0 || n_rows == 0) return GNM_OK;
     if (!h_all || !d_out || !neg_table || !neg_idx || !node_off || !du || !s2) return GNM_ERR_BAD_ARG;
@@ -372,7 +432,8 @@ extern "C" int gnm_dgi_score_bwd(const float* h_all, int64_t layer_stride, int n
 #define GNM_DGI_BWD(NL) \
     do { gnm_count_launch(GNM_K_OTHER); \
     dgi_score_bwd_vec_kernel<NL><<<n_graphs, 256, 0, gnm_cast_stream(stream)>>>(h_all, layer_stride, ldh, n_rows, d_out, \
-                                                                             neg_table, neg_idx, node_off, du, s2, d_bias); } while (0)
+                                                                             neg_table, neg_idx, node_off, bn, ld_bn, du, s2, \
+                                                                             d_bias); } while (0)
         switch (n_layers) {
             case 1: GNM_DGI_BWD(1); break;
             case 2: GNM_DGI_BWD(2); break;
@@ -384,7 +445,7 @@ extern "C" int gnm_dgi_score_bwd(const float* h_all, int64_t layer_stride, int n
         GNM_RETURN_IF_LAUNCH_FAILED();
         return GNM_OK;
     }
-    const size_t smem = (size_t)8 * n_layers * n_feat * 4;
+    const size_t smem = (size_t)(bn != nullptr ? 10 : 8) * n_layers * n_feat * 4;
     if (smem > 200 * 1024) return GNM_ERR_TOO_LARGE;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(dgi_score_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -393,15 +454,15 @@ extern "C" int gnm_dgi_score_bwd(const float* h_all, int64_t layer_stride, int n
     gnm_count_launch(GNM_K_OTHER);
     dgi_score_bwd_kernel<<<n_graphs, 256, smem, gnm_cast_stream(stream)>>>(h_all, layer_stride, n_layers, n_feat, ldh,
                                                                            n_rows, d_out, neg_table, neg_idx, node_off,
-                                                                           du, s2, d_bias);
+                                                                           bn, ld_bn, du, s2, d_bias);
     GNM_RETURN_IF_LAUNCH_FAILED();
     return GNM_OK;
 }
 
 extern "C" int gnm_dgi_score_train(const float* h_all, int64_t layer_stride, int n_layers, int n_feat, int64_t ldh,
                                    int n_rows, const float* u, const float* neg_table, const int32_t* neg_idx,
-                                   const int32_t* node_off, int n_graphs, const float* bias, float grad_scale,
-                                   double loss_scale, float* out, float* d_score, float* du, float* s2, double* d_bias,
+                                   const int32_t* node_off, int n_graphs, const float* bias, const float* bn,
+                                   int64_t ld_bn, float grad_scale, double loss_scale, float* out, float* d_score, float* du, float* s2, double* d_bias,
                                    double* loss_acc, gnm_stream_t stream) {
     if (n_layers < 0 || n_feat < 0 || n_rows < 0 || n_graphs < 0) return GNM_ERR_BAD_ARG;
     if (n_graphs == 0 || n_rows == 0) return GNM_OK;
@@ -412,7 +473,7 @@ extern "C" int gnm_dgi_score_train(const float* h_all, int64_t layer_stride, int
 #define GNM_DGI_TRAIN(NL) \
     do { gnm_count_launch(GNM_K_OTHER); \
     dgi_score_train_kernel<NL><<<n_graphs, 256, 0, gnm_cast_stream(stream)>>>(h_all, layer_stride, ldh, n_rows, u, neg_table, \
-        neg_idx, node_off, bias, grad_scale, loss_scale, out, d_score, du, s2, d_bias, loss_acc); } while (0)
+        neg_idx, node_off, bias, bn, ld_bn, grad_scale, loss_scale, out, d_score, du, s2, d_bias, loss_acc); } while (0)
     switch (n_layers) {
         case 1: GNM_DGI_TRAIN(1); break;
         case 2: GNM_DGI_TRAIN(2); break;

@@ -334,6 +334,16 @@ class BatchStructure(object):
                                             src, src_map, dst, mode, eps, bias)
         return _ops.aggregate(self.rowptr, self.colidx, src, src_map, dst, mode, eps, bias)
 
+    def aggregate_bn(self, z, scale, shift, dst, pooled):
+        """dst = Agg(relu(z*scale + shift)) (sum pooling, no self term) with the activated rows never written, and pooled
+        (nullable) = their graph readout - the tcgen05 kernel's BatchNorm + ReLU on load. False, nothing launched, when
+        the batch does not run on that kernel (the caller materialises h then)."""
+        if self.bitmap_addr is None or FORCE_CSR_AGGREGATE or not _ops.dense_aggregate_ok(z, dst):
+            return False
+        return _ops.aggregate_dense(self.bitmap_addr, self.node_off, self.rowptr, self.n_graphs, self.n_max, z, None, dst,
+                                    0, None, None, bn_scale=scale, bn_shift=shift, pooled=pooled,
+                                    pool_scale=self.pool_scale)
+
     def aggregate_relu_bn_bwd(self, src, mode, eps, unit, d_pooled, d_score, u, d_neg, n_neg, dy, stats, tail=None):
         """Backward aggregation of `src` fused with the relu / BatchNorm backward reduction of `unit` (the last unit of
         the layer below) when the batch runs on the tcgen05 dense-block kernel; False, nothing launched, otherwise."""
@@ -474,13 +484,15 @@ class _ZeroPool(object):
 FOLD_BN_TAILS = True           # A/B switch: BatchNorm finalisation in the last CTA of the kernel producing the statistics
 
 
-def _bn_forward_tail(unit, stats, count, training, comm):
-    """Prepare the BatchNorm of `unit` (its Linear's output z is about to be produced together with `stats`): allocates
-    scale / shift / mean / rstd and returns the ops.BnTail the producer kernel may run in its last CTA - or None when
-    this BatchNorm uses running statistics or the exchange needs NCCL. `_bn_affine(..., done=taken)` completes it."""
+def _bn_forward_tail(unit, stats, count, training, comm, buf=None):
+    """Prepare the BatchNorm of `unit` (its Linear's output z is about to be produced together with `stats`): places
+    scale / shift / mean / rstd in `buf` ([4, F], allocated when None) and returns the ops.BnTail the producer kernel may
+    run in its last CTA - or None when this BatchNorm uses running statistics or the exchange needs NCCL.
+    `_bn_affine(..., done=taken)` completes it."""
     dev = unit.z.device
     f = unit.z.shape[1]
-    buf = torch.empty(4, f, dtype=torch.float32, device=dev)
+    if buf is None:
+        buf = torch.empty(4, f, dtype=torch.float32, device=dev)
     unit.scale, unit.shift, unit.mean, unit.rstd = buf[0], buf[1], buf[2], buf[3]
     bn = unit.bn
     use_batch = training or not bn.track_running_stats
@@ -561,6 +573,26 @@ def first_argmax_from_padded(h, padded, cmin_values):
     return idx.gather(1, pos).to(torch.int32)
 
 
+BN_ON_LOAD = True              # A/B switch: layers' h formed on load from z by its consumers instead of materialised
+
+
+def _materialise_plan(model, bs, with_dgi):
+    """Which layers' h = relu(BN(z)) must be written to memory ([L] bools), and whether the DGI kernels read z with the
+    BatchNorm on load. A layer's h is materialised only when one of its consumers cannot form it on load: the next
+    layer's aggregation off the tcgen05 single-pass kernel (CSR, mma.sync, more than TC_MAX_NODES nodes, max / average
+    pooling, the eps self term, F > 64), learn_eps (the backward's d eps reads h), or a DGI shape off the 64-wide kernels."""
+    L, F = model.num_layers, model.hidden_dim
+    on_load = BN_ON_LOAD and getattr(_ops, "BN_ON_LOAD", False)
+    agg_ok = (on_load and not FORCE_CSR_AGGREGATE and bs.bitmap_addr is not None and bs.n_max <= _ops.TC_MAX_NODES and
+              _ops.DENSE_IMPL[0] != 1 and model.neighbor_pooling_type == "sum" and not model.learn_eps and
+              F % 4 == 0 and F <= 64)
+    dgi_ok = on_load and F == 64 and L <= 5
+    need = [not agg_ok if layer < L - 1 else False for layer in range(L)]
+    if with_dgi and not dgi_ok:
+        need = [True] * L
+    return need, on_load and with_dgi and dgi_ok
+
+
 def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, max_padded=None, bce=None):
     """graphcnn.py:194-251 (and :254-294 when with_dgi is False). Returns (g_f, d_logit, saved).
     bce = (grad_scale, loss_scale, loss_acc): the caller's loss on d_logit is BCEWithLogits against main.py:32's targets
@@ -581,7 +613,14 @@ def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, m
     sv.with_dgi = with_dgi
     sv.x_dense = x_dense
     sv.scored = None
-    h_all = torch.empty(L, M, F, dtype=torch.float32, device=dev)
+    sv.F = F
+    # Each layer's h = relu(BN(z_last)) is read on load from its last unit's z (z_all[layer]) with that unit's scale /
+    # shift (bn_all[layer, :2]) by the next layer's aggregation - which also forms the layer's readout - and by the DGI
+    # kernels; h_all exists only when some layer's h has a consumer that cannot do that (_materialise_plan).
+    need_h, dgi_on_load = _materialise_plan(model, bs, with_dgi)
+    h_all = torch.empty(L, M, F, dtype=torch.float32, device=dev) if any(need_h) else None
+    z_all = torch.empty(L, M, F, dtype=torch.float32, device=dev) if not all(need_h) else None
+    bn_all = torch.empty(L, 4, F, dtype=torch.float32, device=dev) if z_all is not None else None
     g_f = torch.empty(B, L * F, dtype=torch.float32, device=dev)
     sv.h_all = h_all
     use_gather0 = x_dense is None
@@ -602,14 +641,15 @@ def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, m
             u.bn = bn
             units.append(u)
         eps_l = eps_p[layer:layer + 1] if learn_eps else None
-        h_prev = h_all[layer - 1] if layer > 0 else None
+        h_prev = h_all[layer - 1] if layer > 0 and need_h[layer - 1] else None
         pooled = None
         for j, u in enumerate(units):
             n_out = u.w.shape[0]
-            u.z = torch.empty(M, n_out, dtype=torch.float32, device=dev)
+            last_unit = j == len(units) - 1 and z_all is not None
+            u.z = z_all[layer] if last_unit else torch.empty(M, n_out, dtype=torch.float32, device=dev)
             u.scale = None
             stats = zp.f64(2 * n_out)[0]
-            tail = _bn_forward_tail(u, stats, M, training, comm)
+            tail = _bn_forward_tail(u, stats, M, training, comm, buf=bn_all[layer] if last_unit else None)
             done = False
             if j == 0:
                 if layer == 0 and use_gather0:
@@ -621,6 +661,18 @@ def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, m
                         bs.aggregate(w1t, bs.tags, u.z, 1 if average else 0, eps_l, u.b)
                         _ops.col_stats(u.z, stats)
                     u.x_in = None
+                elif layer > 0 and h_prev is None:
+                    # h of the layer below formed on load from its z, and that layer's readout formed with it
+                    below = sv.layers[layer - 1][-1]
+                    pooled = torch.empty(M, F, dtype=torch.float32, device=dev)
+                    g_below = g_f[:, (layer - 1) * F:layer * F]
+                    if not bs.aggregate_bn(below.z, below.scale, below.shift, pooled, g_below):
+                        h_tmp = torch.empty(M, F, dtype=torch.float32, device=dev)
+                        _ops.bn_relu_readout(below.z, below.scale, below.shift, h_tmp, bs.node_off, B, bs.pool_scale,
+                                             g_below)
+                        bs.aggregate(h_tmp, None, pooled, 0, None, None)
+                    done = bool(_ops.linear(pooled, u.w, False, u.b, None, None, u.z, stats, tail))
+                    u.x_in = pooled
                 else:
                     src = x_dense if layer == 0 else h_prev
                     pooled = torch.empty(M, src.shape[1], dtype=torch.float32, device=dev)
@@ -643,9 +695,16 @@ def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, m
                 u.x_in = None          # recomputed from p.z with p's affine + ReLU
             _bn_affine(u, stats, M, training, comm, done=done)
         last = units[-1]
-        _ops.bn_relu_readout(last.z, last.scale, last.shift, h_all[layer], bs.node_off, B, bs.pool_scale,
-                             g_f[:, layer * F:(layer + 1) * F])
+        if need_h[layer] or layer == L - 1:
+            # the readout (writing h only where a consumer needs it); the other layers' readouts come with the next
+            # layer's aggregation
+            _ops.bn_relu_readout(last.z, last.scale, last.shift, h_all[layer] if need_h[layer] else None, bs.node_off, B,
+                                 bs.pool_scale, g_f[:, layer * F:(layer + 1) * F])
         sv.layers.append(units)
+    # what the DGI kernels read: the pre-BatchNorm z with scale | shift applied on load, or the materialised h
+    nf, nf_bn = (z_all, bn_all[:, :2]) if dgi_on_load else (h_all, None)
+    sv.nf, sv.nf_bn = nf, nf_bn
+    bn_kw = {"bn": nf_bn} if nf_bn is not None else {}
     d_logit = None
     if with_dgi:
         # discriminator.py:19-38 refactored: sc = <h, u_g> + b with u_g = W c_g (c = sigmoid(g_f), graphcnn.py:238-239)
@@ -667,15 +726,15 @@ def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, m
                 # at B = 1024 instead of a broadcast of the whole [B_global, L*F] table)
                 neg_table = reg.tensor(0, 0, (b_neg, lf))
                 if comm.rank == 0:
-                    _ops.gather_nf_rows(h_all, b_neg, out=neg_table)
+                    _ops.gather_nf_rows(nf, b_neg, out=neg_table, **bn_kw)
                 comm.p2p_barrier()
                 sv.rows_region = reg
             else:
-                neg_table = _ops.gather_nf_rows(h_all, b_neg) if comm.rank == 0 else \
+                neg_table = _ops.gather_nf_rows(nf, b_neg, **bn_kw) if comm.rank == 0 else \
                     torch.empty(b_neg, lf, dtype=torch.float32, device=dev)
                 comm.broadcast(neg_table, 0)
         else:
-            neg_table = _ops.gather_nf_rows(h_all, b_neg)
+            neg_table = _ops.gather_nf_rows(nf, b_neg, **bn_kw)
             my_neg = neg_idx
         d_logit = torch.empty(2 * M, 1, dtype=torch.float32, device=dev)
         scored = False
@@ -686,12 +745,12 @@ def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, m
             du = torch.empty(B, lf, dtype=torch.float32, device=dev)
             s2 = torch.empty(B, dtype=torch.float32, device=dev)
             d_bias = zp.f64(1)[0]
-            scored = _ops.dgi_score_train(h_all, u_mat, neg_table, my_neg, bs.node_off, B, disc_b, bce[0], bce[1],
-                                          d_logit, d_score, du, s2, d_bias, bce[2])
+            scored = _ops.dgi_score_train(nf, u_mat, neg_table, my_neg, bs.node_off, B, disc_b, bce[0], bce[1],
+                                          d_logit, d_score, du, s2, d_bias, bce[2], **bn_kw)
             if scored:
                 sv.scored = (d_score, du, s2, d_bias)
         if not scored:
-            _ops.dgi_score_fwd(h_all, u_mat, neg_table, my_neg, bs.node_off, B, disc_b, d_logit)
+            _ops.dgi_score_fwd(nf, u_mat, neg_table, my_neg, bs.node_off, B, disc_b, d_logit, **bn_kw)
         sv.c, sv.u_mat, sv.neg_table, sv.my_neg, sv.neg_idx = c, u_mat, neg_table, my_neg, neg_idx
     return g_f, d_logit, sv
 
@@ -731,7 +790,7 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
     dev = params[0].device
     L = model.num_layers
     M, B = bs.n_rows, bs.n_graphs
-    F = sv.h_all.shape[2]
+    F = sv.F
     learn_eps = model.learn_eps
     average = model.neighbor_pooling_type == "average"
     bwd_mode = 2 if average else 0
@@ -758,7 +817,8 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
             s2 = torch.empty(B, dtype=torch.float32, device=dev)
             d_bias, c_, o_ = zp.f64(1)
             from_f64.append((2, c_, o_, 1, False))
-            _ops.dgi_score_bwd(sv.h_all, dd, sv.neg_table, sv.my_neg, bs.node_off, B, du, s2, d_bias)
+            bn_kw = {"bn": sv.nf_bn} if sv.nf_bn is not None else {}
+            _ops.dgi_score_bwd(sv.nf, dd, sv.neg_table, sv.my_neg, bs.node_off, B, du, s2, d_bias, **bn_kw)
         # [B, L*F]-sized glue of u = c W^T, c = sigmoid(g_f): dW[i,j] = sum_b du[b,i] c[b,j];
         # d g_f = dg_f (heads) + (du W) c (1 - c); gradient reaching the shuffled rows n_f[perm[g]]
         lf = L * F
@@ -822,7 +882,7 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
         pidx -= 4 * len(units)
         sl = slice(layer * F, (layer + 1) * F)
         eps_l = eps_p[layer:layer + 1] if learn_eps else None
-        h_prev = sv.h_all[layer - 1] if layer > 0 else None
+        h_prev = sv.h_all[layer - 1] if layer > 0 and learn_eps else None      # materialised under learn_eps
         dz = None
         pending = None        # (dy, stats) of the current unit when the previous fused call already produced them
         for j in range(len(units) - 1, -1, -1):

@@ -11,7 +11,7 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.path.join(CSRC, "libgnm.so")
-ABI_VERSION = 23
+ABI_VERSION = 24
 
 _c_i32 = ctypes.c_int
 _c_i64 = ctypes.c_int64
@@ -31,7 +31,8 @@ SIGNATURES = {
     "gnm_csr_batch_gather": [_p, _p, _p, _p, _p, _c_i32, _p, _p, _p, _p],
     "gnm_aggregate": [_p, _p, _c_i32, _p, _c_i64, _p, _p, _c_i64, _c_i32, _c_i32, _p, _p, _p],
     "gnm_bitmap_build": [_p, _p, _p, _p, _c_i32, _p, _p, _p],
-    "gnm_aggregate_dense": [_p, _p, _p, _c_i32, _c_i32, _p, _c_i64, _p, _p, _c_i64, _c_i32, _c_i32, _p, _p, _c_i32, _p],
+    "gnm_aggregate_dense": [_p, _p, _p, _c_i32, _c_i32, _p, _c_i64, _p, _p, _c_i64, _c_i32, _c_i32, _p, _p, _c_i32, _p, _p,
+                            _p, _c_i64, _p, _p],
     "gnm_aggregate_dense_table": [_p, _p, _p, _c_i32, _c_i32, _p, _c_i64, _p, _p, _c_i64, _c_i32, _c_i32, _p, _p, _p, _p, _p],
     "gnm_aggregate_tc_status": [_p],
     "gnm_aggregate_tc_set_debug": [_p],
@@ -69,11 +70,11 @@ SIGNATURES = {
     "gnm_relu_bn_bwd_reduce": [_p, _c_i64, _c_i32, _c_i32, _p, _p, _p, _p, _p, _c_i64, _p, _c_i64, _p, _p, _p,
                                _c_i64, _p, _c_i64, _c_i32, _p, _c_i32, _p, _c_i64, _p, _p, _p],
     "gnm_bn_bwd_apply": [_p, _c_i64, _c_i32, _c_i32, _p, _p, _p, _p, _c_f64, _p, _c_i64, _p],
-    "gnm_gather_nf_rows": [_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i32, _p, _p],
-    "gnm_dgi_score_fwd": [_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i32, _p, _p, _p, _p, _c_i32, _p, _p, _p],
-    "gnm_dgi_score_bwd": [_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i32, _p, _p, _p, _p, _c_i32, _p, _p, _p, _p],
-    "gnm_dgi_score_train": [_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i32, _p, _p, _p, _p, _c_i32, _p, _c_f32, _c_f64, _p, _p,
-                            _p, _p, _p, _p, _p],
+    "gnm_gather_nf_rows": [_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i32, _p, _c_i64, _p, _p],
+    "gnm_dgi_score_fwd": [_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i32, _p, _p, _p, _p, _c_i32, _p, _p, _c_i64, _p, _p],
+    "gnm_dgi_score_bwd": [_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i32, _p, _p, _p, _p, _c_i32, _p, _c_i64, _p, _p, _p, _p],
+    "gnm_dgi_score_train": [_p, _c_i64, _c_i32, _c_i32, _c_i64, _c_i32, _p, _p, _p, _p, _c_i32, _p, _p, _c_i64, _c_f32, _c_f64,
+                            _p, _p, _p, _p, _p, _p, _p],
     "gnm_heads_ce_workspace": [_c_i32, _c_i32, _c_i32, _c_i32],
     "gnm_heads_ce": [_p, _c_i64, _c_i32, _c_i32, _c_i32, _c_i32, _p, _p, _p, _p, _c_f32, _p, _p, _p, _c_i64, _p, _p, _p,
                      _c_i64, _p, _p],

@@ -202,16 +202,31 @@ def aggregate_tc_status():
     return bool(v.value)
 
 
-def aggregate_dense(bitmap_addr, node_off, rowptr, n_graphs, n_max, src, src_map, dst, mode, eps, bias=None, impl=None):
+BN_ON_LOAD = True    # this module's aggregation and DGI entry points take bn_scale= / bn= (engine checks for it)
+
+
+def aggregate_dense(bitmap_addr, node_off, rowptr, n_graphs, n_max, src, src_map, dst, mode, eps, bias=None, impl=None, *,
+                    bn_scale=None, bn_shift=None, pooled=None, pool_scale=None):
+    """dst = Agg(src) (include/gnm.h: gnm_aggregate_dense); returns dst. With bn_scale / bn_shift, src is the layer
+    below's pre-BatchNorm output z and the kernel aggregates relu(z*bn_scale + bn_shift) without writing it, and pooled
+    (optional, [B, >= F] view) receives that layer's graph readout (times pool_scale). Returns True then, or False with
+    nothing launched when the batch does not fit that kernel (materialise h with bn_relu_readout instead)."""
     sp, lds = _mat(src)
     dp, ldd = _mat(dst)
-    _libmod.check(_lib().gnm_aggregate_dense(_ptr(bitmap_addr, torch.int64), _ptr(node_off, torch.int32),
-                                             _ptr(rowptr, torch.int32), n_graphs, n_max, sp, lds,
-                                             _ptr(src_map, torch.int32) if src_map is not None else None, dp, ldd,
-                                             int(dst.shape[1]), int(mode), _ptr(eps, torch.float32),
-                                             _ptr(bias, torch.float32), DENSE_IMPL[0] if impl is None else int(impl),
-                                             _stream(dst)), "gnm_aggregate_dense")
-    return dst
+    pp, ldp = _mat(pooled)
+    on_load = bn_scale is not None
+    rc = _lib().gnm_aggregate_dense(_ptr(bitmap_addr, torch.int64), _ptr(node_off, torch.int32),
+                                    _ptr(rowptr, torch.int32), n_graphs, n_max, sp, lds,
+                                    _ptr(src_map, torch.int32) if src_map is not None else None, dp, ldd,
+                                    int(dst.shape[1]), int(mode), _ptr(eps, torch.float32),
+                                    _ptr(bias, torch.float32), DENSE_IMPL[0] if impl is None else int(impl),
+                                    _ptr(bn_scale, torch.float32), _ptr(bn_shift, torch.float32), pp, ldp,
+                                    _ptr(pool_scale, torch.float32), _stream(dst))
+    if on_load and rc in (-2, -3):          # GNM_ERR_TOO_LARGE / GNM_ERR_ALIGN: not a tcgen05 batch
+        LAUNCHES[0] -= 1
+        return False
+    _libmod.check(rc, "gnm_aggregate_dense")
+    return True if on_load else dst
 
 
 def aggregate_dense_table(bitmap_addr, node_off, rowptr, n_graphs, n_max, table, tags, dst, mode, eps, bias, out_stats,
@@ -647,42 +662,57 @@ def _hall(h_all):
     return _ptr(h_all, torch.float32), int(h_all.stride(0)), int(h_all.shape[0]), int(h_all.shape[2]), int(h_all.stride(1))
 
 
-def gather_nf_rows(h_all, n_rows, out=None):
+def _bn_table(bn, h_all):
+    """bn: None, or per-layer scale | shift as an [L, >= 2, F] view with contiguous rows (e.g. the first two rows of each
+    layer's [4, F] BatchNorm buffers): h_all then holds the pre-BatchNorm z and h = relu(z*scale + shift) on load."""
+    if bn is None:
+        return None, 0
+    if (bn.dim() != 3 or bn.shape[0] != h_all.shape[0] or bn.shape[1] < 2 or bn.shape[2] != h_all.shape[2] or
+            bn.stride(2) != 1 or bn.stride(1) != bn.shape[2] or bn.dtype != torch.float32):
+        raise RuntimeError("bn must be an [L, 2, F] float32 table with contiguous scale | shift rows")
+    return _ptr(bn), int(bn.stride(0))
+
+
+def gather_nf_rows(h_all, n_rows, out=None, bn=None):
     hp, ls, nl, nf, ldh = _hall(h_all)
+    bp, ldb = _bn_table(bn, h_all)
     table = out if out is not None else torch.empty(n_rows, nl * nf, dtype=torch.float32, device=h_all.device)
     if tuple(table.shape) != (n_rows, nl * nf) or not table.is_contiguous():
         raise RuntimeError("gather_nf_rows: out must be a contiguous [%d, %d] tensor" % (n_rows, nl * nf))
-    _libmod.check(_lib().gnm_gather_nf_rows(hp, ls, nl, nf, ldh, n_rows, _ptr(table), _stream(h_all)),
+    _libmod.check(_lib().gnm_gather_nf_rows(hp, ls, nl, nf, ldh, n_rows, bp, ldb, _ptr(table), _stream(h_all)),
                   "gnm_gather_nf_rows")
     return table
 
 
-def dgi_score_fwd(h_all, u, neg_table, neg_idx, node_off, n_graphs, bias, out):
+def dgi_score_fwd(h_all, u, neg_table, neg_idx, node_off, n_graphs, bias, out, bn=None):
     hp, ls, nl, nf, ldh = _hall(h_all)
+    bp, ldb = _bn_table(bn, h_all)
     _libmod.check(_lib().gnm_dgi_score_fwd(hp, ls, nl, nf, ldh, int(h_all.shape[1]), _ptr(u.contiguous(), torch.float32),
                                            _ptr(neg_table, torch.float32), _ptr(neg_idx, torch.int32),
-                                           _ptr(node_off, torch.int32), n_graphs, _ptr(bias, torch.float32),
+                                           _ptr(node_off, torch.int32), n_graphs, _ptr(bias, torch.float32), bp, ldb,
                                            _ptr(out, torch.float32), _stream(out)), "gnm_dgi_score_fwd")
     return out
 
 
-def dgi_score_bwd(h_all, d_out, neg_table, neg_idx, node_off, n_graphs, du, s2, d_bias):
+def dgi_score_bwd(h_all, d_out, neg_table, neg_idx, node_off, n_graphs, du, s2, d_bias, bn=None):
     hp, ls, nl, nf, ldh = _hall(h_all)
+    bp, ldb = _bn_table(bn, h_all)
     _libmod.check(_lib().gnm_dgi_score_bwd(hp, ls, nl, nf, ldh, int(h_all.shape[1]), _ptr(d_out, torch.float32),
                                            _ptr(neg_table, torch.float32), _ptr(neg_idx, torch.int32),
-                                           _ptr(node_off, torch.int32), n_graphs, _ptr(du, torch.float32),
+                                           _ptr(node_off, torch.int32), n_graphs, bp, ldb, _ptr(du, torch.float32),
                                            _ptr(s2, torch.float32), _ptr(d_bias, torch.float64), _stream(du)),
                   "gnm_dgi_score_bwd")
 
 
 def dgi_score_train(h_all, u, neg_table, neg_idx, node_off, n_graphs, bias, grad_scale, loss_scale, out, d_score, du, s2,
-                    d_bias, loss_acc):
+                    d_bias, loss_acc, bn=None):
     """dgi_score_fwd + bce_logits + dgi_score_bwd in one pass (include/gnm.h: gnm_dgi_score_train). Returns False, with
     nothing launched, when the shape does not fit the kernel - make the three calls then."""
     hp, ls, nl, nf, ldh = _hall(h_all)
+    bp, ldb = _bn_table(bn, h_all)
     rc = _lib().gnm_dgi_score_train(hp, ls, nl, nf, ldh, int(h_all.shape[1]), _ptr(u.contiguous(), torch.float32),
                                     _ptr(neg_table, torch.float32), _ptr(neg_idx, torch.int32), _ptr(node_off, torch.int32),
-                                    n_graphs, _ptr(bias, torch.float32), float(grad_scale), float(loss_scale),
+                                    n_graphs, _ptr(bias, torch.float32), bp, ldb, float(grad_scale), float(loss_scale),
                                     _ptr(out, torch.float32), _ptr(d_score, torch.float32), _ptr(du, torch.float32),
                                     _ptr(s2, torch.float32), _ptr(d_bias, torch.float64), _ptr(loss_acc, torch.float64),
                                     _stream(out))

@@ -33,7 +33,7 @@ extern "C" {
 #define GNM_ERR_TOO_LARGE (-2)
 #define GNM_ERR_ALIGN (-3)
 
-#define GNM_ABI_VERSION 23
+#define GNM_ABI_VERSION 24
 
 typedef void* gnm_stream_t;
 
@@ -163,11 +163,20 @@ int gnm_bitmap_build(const int32_t* rowptr, const int32_t* colidx, const int32_t
  * accumulation. rowptr (batch CSR row pointers) supplies the degrees for mode 1 / 2 and may be NULL for mode 0.
  * Needs n_feat % 4 == 0 and 16-byte aligned rows (else GNM_ERR_ALIGN: use gnm_aggregate).
  * impl: 0 = auto (tcgen05/TMEM kernel when every graph has <= 416 nodes, else the mma.sync kernel),
- *       1 = mma.sync kernel, 2 = tcgen05 kernel only (GNM_ERR_TOO_LARGE if it does not fit). */
+ *       1 = mma.sync kernel, 2 = tcgen05 kernel only (GNM_ERR_TOO_LARGE if it does not fit).
+ * BatchNorm + ReLU on load: with bn_scale / bn_shift (nullable, [n_feat] each) src is the PRE-BatchNorm output z of the
+ * layer below and the kernel aggregates h = relu(z*bn_scale + bn_shift) - graphcnn.py:162-166's h of that layer, the
+ * expression of gnm_bn_relu_readout, so dst is bit-identical to gnm_bn_relu_readout(z -> h) + gnm_aggregate_dense(h)
+ * without h ever being written. pooled (nullable, ld_pooled) then also receives that layer's readout
+ * (graphcnn.py:225-228: pooled[g] = pool_scale[g] (nullable) * sum of the graph's rows of h), i.e. gnm_bn_relu_readout's
+ * pooled output, summed in a different order. tcgen05 kernel only, single pass: n_max <= 416, n_feat <= 64, mode 0, no
+ * eps / src_map / bias, impl != 1; GNM_ERR_TOO_LARGE / GNM_ERR_ALIGN otherwise, nothing launched (materialise h with
+ * gnm_bn_relu_readout and aggregate it then). */
 int gnm_aggregate_dense(const int64_t* bitmap_addr, const int32_t* node_off, const int32_t* rowptr,
                         int n_graphs, int n_max, const float* src, int64_t ld_src, const int32_t* src_map,
                         float* dst, int64_t ld_dst, int n_feat, int mode, const float* eps, const float* bias,
-                        int impl, gnm_stream_t stream);
+                        int impl, const float* bn_scale, const float* bn_shift, float* pooled, int64_t ld_pooled,
+                        const float* pool_scale, gnm_stream_t stream);
 /* dst = Agg(cA*dy + cB*z + cC): the aggregation of a BatchNorm-backward result (autograd of graphcnn.py:162-166 feeding
  * the transpose of :154-161 at layer 0) without materialising it - coef = [cA | cB | cC] from gnm_bn_bwd_coeffs is
  * applied to the rows as the tcgen05 kernel loads them. Returns GNM_ERR_TOO_LARGE / GNM_ERR_ALIGN when the batch does
@@ -324,10 +333,15 @@ int gnm_bn_bwd_apply(const float* z, int64_t ldz, int n_rows, int n_feat, const 
 
 /* ---- DGI discriminator ------------------------------------------------------------------- */
 
+/* BatchNorm + ReLU on load (the four entry points below): bn (nullable) = per-layer scale | shift, layer l's scale at
+ * bn + l*ld_bn and its shift at bn + l*ld_bn + n_feat. With bn, h_all holds each layer's PRE-BatchNorm output z and
+ * every value is read as h = relu(z*scale + shift) - graphcnn.py:162-166, gnm_bn_relu_readout's expression - so the
+ * results are bit-identical to the same call on the h that gnm_bn_relu_readout would have written. */
+
 /* Copy rows [0, n_rows) of n_f = cat(hidden_rep, 1) (graphcnn.py:233) into a dense [n_rows, L*F] table:
  * the only rows the "shuffled" negatives ever read (graphcnn.py:198-201,241-242). */
 int gnm_gather_nf_rows(const float* h_all, int64_t layer_stride, int n_layers, int n_feat, int64_t ldh,
-                       int n_rows, float* table, gnm_stream_t stream);
+                       int n_rows, const float* bn, int64_t ld_bn, float* table, gnm_stream_t stream);
 
 /* discriminator.py:19-38 with f_k = nn.Bilinear(n_h, n_h, 1) refactored as sc = <h, u_g> + b, u_g = W c_g:
  *   out[r]     = <n_f[r], u[g(r)]> + *bias                    (sc_1, positives)
@@ -335,7 +349,8 @@ int gnm_gather_nf_rows(const float* h_all, int64_t layer_stride, int n_layers, i
  * h_all holds the L hidden representations as [L][M, ldh]; n_f[r] is their concatenation. */
 int gnm_dgi_score_fwd(const float* h_all, int64_t layer_stride, int n_layers, int n_feat, int64_t ldh, int n_rows,
                       const float* u, const float* neg_table, const int32_t* neg_idx,
-                      const int32_t* node_off, int n_graphs, const float* bias, float* out, gnm_stream_t stream);
+                      const int32_t* node_off, int n_graphs, const float* bias, const float* bn, int64_t ld_bn,
+                      float* out, gnm_stream_t stream);
 
 /* Backward of the scores wrt u, bias and the negative rows:
  *   s2[g]   = sum_{r in g} d_out[M + r]
@@ -344,8 +359,8 @@ int gnm_dgi_score_fwd(const float* h_all, int64_t layer_stride, int n_layers, in
  * (the gradient wrt n_f itself is fused into gnm_relu_bn_bwd_reduce via d_score/u/d_neg). */
 int gnm_dgi_score_bwd(const float* h_all, int64_t layer_stride, int n_layers, int n_feat, int64_t ldh, int n_rows,
                       const float* d_out, const float* neg_table, const int32_t* neg_idx,
-                      const int32_t* node_off, int n_graphs, float* du, float* s2, double* d_bias,
-                      gnm_stream_t stream);
+                      const int32_t* node_off, int n_graphs, const float* bn, int64_t ld_bn, float* du, float* s2,
+                      double* d_bias, gnm_stream_t stream);
 
 /* gnm_dgi_score_fwd, BCEWithLogits against the targets of main.py:32 (positives 1, negatives 0) and gnm_dgi_score_bwd
  * in ONE pass over n_f, for a training step whose loss is the BCE mean (the gradient of a score is local):
@@ -358,8 +373,9 @@ int gnm_dgi_score_bwd(const float* h_all, int64_t layer_stride, int n_layers, in
  * 16-byte aligned rows (GNM_ERR_ALIGN); nothing is launched then - make the three calls instead. */
 int gnm_dgi_score_train(const float* h_all, int64_t layer_stride, int n_layers, int n_feat, int64_t ldh, int n_rows,
                         const float* u, const float* neg_table, const int32_t* neg_idx, const int32_t* node_off,
-                        int n_graphs, const float* bias, float grad_scale, double loss_scale, float* out, float* d_score,
-                        float* du, float* s2, double* d_bias, double* loss_acc, gnm_stream_t stream);
+                        int n_graphs, const float* bias, const float* bn, int64_t ld_bn, float grad_scale,
+                        double loss_scale, float* out, float* d_score, float* du, float* s2, double* d_bias,
+                        double* loss_acc, gnm_stream_t stream);
 
 /* Standalone Discriminator.forward on materialised tensors (discriminator.py:19-38):
  * out[r] = <h[r], u[r / rows_per_graph]> + *bias (+ s_bias[r] if non-NULL). */

@@ -402,6 +402,19 @@ def saliency_maps(model, graphs, cls, batch=64):
     return out.get("a", np.zeros((0, 0, 0), dtype=np.float32))
 
 
+def roi_saliency(model, graphs, classes=(0, 1), batch=1024):
+    """ROI saliency: float32 [G, len(classes), D], entry [i, k] = the node average of `compute_saliency([graphs[i]],
+    classes[k])` - what evaluate/plot_saliency_nii.py reduces each map to - computed by
+    `compute_roi_saliency_batched` in batches of `batch` graphs (one forward per batch for all classes, one D2H copy
+    per batch; 1.6 KB per graph and class instead of a 640 KB map at N = D = 400). Graphs may differ in size."""
+    d = int(_engine.layer_units(model, 0)[0][0].weight.shape[1])          # input_dim
+    out = np.empty((len(graphs), len(classes), d), dtype=np.float32)
+    for i in range(0, len(graphs), batch):
+        chunk = graphs[i:i + batch]
+        out[i:i + len(chunk)] = model.compute_roi_saliency_batched(chunk, classes).cpu().numpy()
+    return out
+
+
 def saliency_maps_to_npy(model, graphs, cls, path, batch=64):
     """`np.save(path, get_saliency_map(model, graphs, cls))` (main.py:168-172) without holding the array: the `.npy`
     file is created as a memory map of its final shape [G, N, D] and filled batch by batch from the pinned double

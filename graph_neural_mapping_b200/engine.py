@@ -784,8 +784,12 @@ def max_pool_onehot_input_grad(bs, p, first, eps):
     return d_x
 
 
-def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first=None):
-    """Hand-derived backward of `run_forward`. Returns (dX or None, [grad per flat param])."""
+def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first=None, roi=None):
+    """Hand-derived backward of `run_forward`. Returns (dX or None, [grad per flat param]).
+    roi ([B, D] view, nullable): ROI mode - roi[g] receives the node average of graph g's input gradient,
+    (1/n_g) sum_{n in g} dX[n], formed without dX where the layer-0 aggregation is linear (ops.segment_weighted_colsum:
+    mean_n (Agg^T dz)[n] = (1/n_g) sum_m w_m dz[m], w_m the operator's row sums). Layer 0's parameter gradients are not
+    formed then. Nothing here writes the saved forward state, so one forward serves a backward per class."""
     bs = sv.bs
     dev = params[0].device
     L = model.num_layers
@@ -855,6 +859,17 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
     d_h = None        # gradient reaching h_all[layer] from layer+1's aggregation
     carry = None      # (dy, stats) of this layer's last unit when layer+1's aggregation kernel already produced them
     d_x = None
+
+    def roi_from_dp(dp, eps_l):
+        """ROI mode, layer 0 on a dense input: the node average of d_x = Agg^T dp (the reduction of dp itself with the
+        operator's row sums; under max pooling, which is not linear, of d_x - the [M, D] route)."""
+        if 0 in sv.max_state:
+            amax, cmin = sv.max_state[0]
+            d_in = torch.empty(M, dp.shape[1], dtype=torch.float32, device=dev)
+            _ops.aggregate_max_bwd(bs.rowptr, bs.colidx, dp, amax, cmin, eps_l, d_in)
+            _ops.segment_weighted_colsum(d_in, bs.node_off, roi)
+        else:
+            _ops.segment_weighted_colsum(dp, bs.node_off, roi, rowptr=bs.rowptr, mode=1 if average else 0, eps=eps_l)
 
     def aggregate_into_layer_below(layer, dp, eps_l):
         """d_h of layer-1 = Agg^T(dp); fused with layer-1's relu / BatchNorm backward reduction when possible."""
@@ -930,6 +945,28 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
             from_f64.append((gi + 2, st_chunk, st_off + n_out, n_out, scaled))
             dw = zp.f32(*u.w.shape)
             db = zp.f32(*u.b.shape)
+            if gather0 and roi is not None:
+                # ROI mode, one-hot input: saliency = (Agg^T dz) W1, so its node average is (1/n_g)(sum_m w_m dz[m]) W1 -
+                # one streaming reduction of dy with the BatchNorm-backward affine on load, then a [B, F] x [F, D] product
+                if model.neighbor_pooling_type == "max":
+                    # max pooling is not linear: the input gradient itself, then its average
+                    if max_first is None:
+                        raise RuntimeError("input gradients under max pooling need the neighbour-list order")
+                    _ops.bn_bwd_apply(u.z, u.mean, u.rstd, u.gamma, stats if use_batch else None, u.count, dy)
+                    dp0 = torch.empty(M, n_in, dtype=torch.float32, device=dev)
+                    _ops.linear(dy, u.w, True, None, None, None, dp0, None)
+                    _ops.segment_weighted_colsum(max_pool_onehot_input_grad(bs, dp0, max_first, eps_l), bs.node_off, roi)
+                    continue
+                if coef_ready is not None:
+                    coef0 = coef_ready
+                else:
+                    coef0 = torch.empty(3, n_out, dtype=torch.float32, device=dev)
+                    _ops.bn_bwd_coeffs(stats if use_batch else None, u.count, u.gamma, u.mean, u.rstd, coef0)
+                dz_sum = torch.empty(B, n_out, dtype=torch.float32, device=dev)
+                _ops.segment_weighted_colsum(dy, bs.node_off, dz_sum, z=u.z if use_batch else None, coef=coef0,
+                                             rowptr=bs.rowptr, mode=1 if average else 0, eps=eps_l)
+                _ops.small_gemm(dz_sum, (dz_sum.stride(0), 1), u.w, (u.w.stride(0), 1), roi, B, n_in, n_out)
+                continue
             if fused:
                 # one pass: BatchNorm-backward apply (folded into the load as dz = A*dy + B*z + C), dW, db, dX and -
                 # for an inner unit - the ReLU mask + BatchNorm-backward reduction of the unit below
@@ -947,15 +984,17 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
                                            stats_prev[0], tail=tail_p)
                     pending = (dy_prev, stats_prev, coef_p if took is True else None)
                 else:
-                    need_dp = layer > 0 or need_x_grad or learn_eps
+                    need_dp = layer > 0 or need_x_grad or learn_eps or roi is not None
                     dp = torch.empty(M, n_in, dtype=torch.float32, device=dev) if need_dp else None
                     _ops.linear_bwd(dy, u.z, coef, u.x_in, None, None, None, None, u.w, dw, db, dp, None)
                     if need_dp:
                         src = sv.x_dense if layer == 0 else h_prev
-                        if learn_eps:
+                        if learn_eps and not (layer == 0 and roi is not None):
                             _ops.dot_rows(dp, src, None, d_eps[layer:layer + 1])
                         if layer > 0:
                             d_h, carry = aggregate_into_layer_below(layer, dp, eps_l)
+                        elif roi is not None:
+                            roi_from_dp(dp, eps_l)
                         elif need_x_grad:
                             d_x = torch.empty(M, n_in, dtype=torch.float32, device=dev)
                             if layer in sv.max_state:
@@ -1025,16 +1064,20 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
                     d_x = torch.empty(M, n_in, dtype=torch.float32, device=dev)
                     _ops.linear(g_agg, u.w, True, None, None, None, d_x, None)   # (Agg^T dz) @ W1
             else:
-                _ops.linear_wgrad(dz_u, u.x_in, None, None, dw, db)
-                need_dp = layer > 0 or need_x_grad or learn_eps
+                roi0 = layer == 0 and roi is not None
+                if not roi0:
+                    _ops.linear_wgrad(dz_u, u.x_in, None, None, dw, db)
+                need_dp = layer > 0 or need_x_grad or learn_eps or roi0
                 if need_dp:
                     src = sv.x_dense if layer == 0 else h_prev
                     dp = torch.empty(M, n_in, dtype=torch.float32, device=dev)
                     _ops.linear(dz_u, u.w, True, None, None, None, dp, None)
-                    if learn_eps:
+                    if learn_eps and not roi0:
                         _ops.dot_rows(dp, src, None, d_eps[layer:layer + 1])
                     if layer > 0:
                         d_h, carry = aggregate_into_layer_below(layer, dp, eps_l)
+                    elif roi0:
+                        roi_from_dp(dp, eps_l)
                     elif need_x_grad:
                         d_x = torch.empty(M, n_in, dtype=torch.float32, device=dev)
                         if layer in sv.max_state:

@@ -284,5 +284,40 @@ class GIN_InfoMaxReg(nn.Module):
         score_over_layer.backward(predicting_class)
         return runner.x_grad if x is None else x.grad
 
+    def compute_roi_saliency_batched(self, batch_graph, classes):
+        """ROI saliency: float32 [B, len(classes), D] device tensor whose entry [i, k] is
+        `compute_saliency([batch_graph[i]], classes[k]).mean(0)` (up to fp32 rounding) - the node average that
+        evaluate/plot_saliency_nii.py paints onto ROI volumes, without the [N, D] maps. One eval forward serves every
+        class; each class then runs the hand-derived backward from the same saved state, and layer 0 reduces its
+        gradient per graph instead of forming the map (engine.run_backward's ROI mode). Graphs may differ in size:
+        each mean is over that graph's own nodes. Puts the model in eval() like compute_saliency but, unlike it, leaves
+        every parameter's .grad untouched (no autograd pass runs)."""
+        self.eval()
+        classes = [int(c) for c in classes]
+        n_cls = self.linears_prediction[0].weight.shape[0]
+        if any(c < 0 or c >= n_cls for c in classes):
+            raise ValueError("classes must lie in [0, %d), got %s" % (n_cls, classes))
+        dev = self.eps.device
+        d_in = _engine.layer_units(self, 0)[0][0].weight.shape[1]
+        b = len(batch_graph)
+        out = torch.empty(b, len(classes), d_in, dtype=torch.float32, device=dev)
+        if b == 0 or not classes:
+            return out
+        bs = self._structure(batch_graph)
+        max_padded = max_first = None
+        if self.neighbor_pooling_type == "max":
+            padded, first = self._padded_neighbours(batch_graph)
+            max_padded, max_first = padded.to(dev), first.to(dev)
+        x = self._dense_features(batch_graph, bs)
+        params = [p.detach() for p in _engine.flat_params(self)]
+        with torch.no_grad():
+            _, _, sv = _engine.run_forward(self, bs, None, False, False, x, params, _dist.SINGLE, max_padded=max_padded)
+            heads = [lin.weight.detach() for lin in self.linears_prediction]
+            for k, c in enumerate(classes):
+                # d score_c / d g_f: the class-c rows of the prediction heads (graphcnn.py:228-231 in eval, no dropout)
+                dg_f = torch.cat([w[c] for w in heads]).expand(b, -1).contiguous()
+                _engine.run_backward(self, sv, params, dg_f, None, False, _dist.SINGLE, max_first=max_first, roi=out[:, k])
+        return out
+
 
 GraphCNN = GIN_InfoMaxReg      # the name BASELINE.json's north_star uses for this class

@@ -57,7 +57,8 @@ def device_info():
 
 
 KERNEL_FAMILIES = ("aggregate_csr", "aggregate_mma_sync", "aggregate_tc", "linear_ffma", "linear_tc", "linear_bwd_ffma",
-                   "linear_bwd_dx_tc", "linear_wgrad_tc", "linear_wgrad_ffma", "other", "linear_bwd_onepass_tc")
+                   "linear_bwd_dx_tc", "linear_wgrad_tc", "linear_wgrad_ffma", "other", "linear_bwd_onepass_tc",
+                   "segment_colsum")
 
 
 def launch_counts():
@@ -326,6 +327,21 @@ def rows_period_sum(g, period, tags, table_grad):
                                              int(table_grad.shape[0]), _ptr(ws), need, _stream(g)),
                   "gnm_rows_period_sum")
     return table_grad
+
+
+def segment_weighted_colsum(x, node_off, out, z=None, coef=None, rowptr=None, mode=0, eps=None):
+    """out[g] = (1/n_g) sum over graph g's rows m of w_m * v[m] (include/gnm.h: gnm_segment_weighted_colsum): v = x, or
+    coef[0]*x + coef[1]*z + coef[2] with coef given (z None: coef[1] = coef[2] = 0); w_m = the row sums of the
+    aggregation `mode` (0 sum, 1 average) with the optional eps self term as its backward applies them, or 1 without
+    rowptr. out [B, W] may be a strided view. Returns out."""
+    xp, ldx = _mat(x)
+    zp, ldz = _mat(z)
+    op, ldo = _mat(out)
+    _libmod.check(_lib().gnm_segment_weighted_colsum(xp, ldx, zp, ldz, _ptr(coef, torch.float32), _ptr(node_off, torch.int32),
+                                                     int(out.shape[0]), int(out.shape[1]), _ptr(rowptr, torch.int32),
+                                                     int(mode), _ptr(eps, torch.float32), op, ldo, _stream(out)),
+                  "gnm_segment_weighted_colsum")
+    return out
 
 
 # ---- max pooling over neighbours ----------------------------------------------------------------

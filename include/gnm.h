@@ -33,7 +33,7 @@ extern "C" {
 #define GNM_ERR_TOO_LARGE (-2)
 #define GNM_ERR_ALIGN (-3)
 
-#define GNM_ABI_VERSION 24
+#define GNM_ABI_VERSION 25
 
 typedef void* gnm_stream_t;
 
@@ -92,7 +92,8 @@ int gnm_device_info(int* sm_count, int* cc_major, int* cc_minor, int64_t* smem_o
  * (a kernel recorded during CUDA-graph capture counts once, its replays are the caller's to count). Families:
  * 0 aggregate (CSR warp-per-row), 1 aggregate (mma.sync dense blocks), 2 aggregate (tcgen05), 3 linear (FFMA),
  * 4 linear (tcgen05), 5 linear_bwd (fused FFMA), 6 linear_bwd dX (tcgen05), 7 linear_bwd dW (tcgen05),
- * 8 linear_wgrad (FFMA), 9 every other kernel, 10 linear_bwd one-pass dX + dW (tcgen05). Returns the number of families (>= 0) or GNM_ERR_BAD_ARG.
+ * 8 linear_wgrad (FFMA), 9 every other kernel, 10 linear_bwd one-pass dX + dW (tcgen05), 11 segment_weighted_colsum.
+ * Returns the number of families (>= 0) or GNM_ERR_BAD_ARG.
  * Tests use it to prove WHICH kernel family a code path ran; bench.py to count launches. */
 int gnm_launch_counts(int64_t* out, int n);
 /* Programmatic dependent launch of the persistent tcgen05 kernels (aggregation, Linear forward / dX / dW): off by default
@@ -454,6 +455,26 @@ int gnm_adam_step(float* const* params, const float* const* grads, const int32_t
                   int n_tensors, float* exp_avg, float* exp_avg_sq, float* step, const float* lr, double beta1, double beta2,
                   float eps, float weight_decay, float grad_scale, const double* loss_terms, int n_loss_terms,
                   float* loss_out, gnm_stream_t stream);
+
+/* ---- ROI saliency ----------------------------------------------------------------------------------------------
+ * The node average of the saliency maps (graphcnn.py:254-299 averaged over the node axis, as evaluate/
+ * plot_saliency_nii.py does before painting ROI volumes) without the [N, D] maps: mean_n (Agg^T dz W1)[n] =
+ * (1/n_g) (sum_m w_m dz[m]) W1 with w_m the row sums of the aggregation operator. Per graph g (rows node_off[g] ..
+ * node_off[g+1]):
+ *   out[g, c] = scale_g * sum_{m in g} w_m * v[m, c],   c < width,   scale_g = 1/n_g (an empty graph yields zeros)
+ * v = x (coef NULL), or the BatchNorm-backward affine formed on load as gnm_aggregate_dense_affine forms it: v = cA*x +
+ *   cB*z + cC with coef = [cA | cB | cC] ([3*width], gnm_bn_bwd_coeffs' output); z NULL means cB = cC = 0 (eval with
+ *   running statistics) and z is not read.
+ * w_m = the row sum of the aggregation operator of gnm_aggregate (mode 0 sum / 1 average, eps nullable) as its backward
+ *   (mode 0 / 2) applies it: rowptr NULL: 1; mode 0: deg_m (the CSR row length: self loop included, duplicate edges with
+ *   their multiplicity) [+ 1 + *eps]; mode 1: 1, or 0 for an isolated node [+ 1 + *eps]. The transpose of the average
+ *   gathers nothing from an isolated node, so the forward's 0/0 = NaN does not reach the input gradient through it and
+ *   is not invented here; a NaN in v still propagates.
+ * Rows are summed in a fixed order (deterministic, no atomics). Vectorised when width and the leading dimensions are
+ * multiples of 4 and x, z are 16-byte aligned; any width >= 1 and stride otherwise. */
+int gnm_segment_weighted_colsum(const float* x, int64_t ldx, const float* z, int64_t ldz, const float* coef,
+                                const int32_t* node_off, int n_graphs, int width, const int32_t* rowptr, int mode,
+                                const float* eps, float* out, int64_t ld_out, gnm_stream_t stream);
 
 /* ---- data parallel: synchronised BatchNorm sums over NVLink peer memory ------------------------------
  * The reference is single-process; a global-batch BatchNorm needs the per-channel sums of all ranks before the next

@@ -323,22 +323,26 @@ class BatchStructure(object):
             _, self._colidx, _ = _ops.csr_batch_gather(*self._gather_args)
         return self._colidx
 
+    def _on_tc(self, src, dst, bias, mode):
+        """Whether the batch runs on the tcgen05 dense-block kernel for these operands. Average pooling divides by the
+        degree: an isolated node yields 0/0 = NaN in the reference, and a NaN row would poison its whole dense block
+        (0 * NaN), so such batches keep the gather kernel."""
+        return (self.bitmap_addr is not None and not FORCE_CSR_AGGREGATE and _ops.dense_aggregate_ok(src, dst, bias)
+                and (mode == 0 or not self.has_isolated))
+
     def aggregate(self, src, src_map, dst, mode, eps, bias=None):
         """graphcnn.py:154-161 / :178-182 (and the transpose for backward): tensor-core dense-block kernel when
         the batch qualifies, CSR warp-per-row kernel otherwise."""
-        if self.bitmap_addr is not None and not FORCE_CSR_AGGREGATE and _ops.dense_aggregate_ok(src, dst, bias):
-            # average pooling divides by the degree: an isolated node yields 0/0 = NaN in the reference, and a
-            # NaN row would poison its whole dense block (0 * NaN); keep such batches on the gather kernel
-            if mode == 0 or not self.has_isolated:
-                return _ops.aggregate_dense(self.bitmap_addr, self.node_off, self.rowptr, self.n_graphs, self.n_max,
-                                            src, src_map, dst, mode, eps, bias)
+        if self._on_tc(src, dst, bias, mode):
+            return _ops.aggregate_dense(self.bitmap_addr, self.node_off, self.rowptr, self.n_graphs, self.n_max,
+                                        src, src_map, dst, mode, eps, bias)
         return _ops.aggregate(self.rowptr, self.colidx, src, src_map, dst, mode, eps, bias)
 
     def aggregate_bn(self, z, scale, shift, dst, pooled):
         """dst = Agg(relu(z*scale + shift)) (sum pooling, no self term) with the activated rows never written, and pooled
         (nullable) = their graph readout - the tcgen05 kernel's BatchNorm + ReLU on load. False, nothing launched, when
         the batch does not run on that kernel (the caller materialises h then)."""
-        if self.bitmap_addr is None or FORCE_CSR_AGGREGATE or not _ops.dense_aggregate_ok(z, dst):
+        if not self._on_tc(z, dst, None, 0):
             return False
         return _ops.aggregate_dense(self.bitmap_addr, self.node_off, self.rowptr, self.n_graphs, self.n_max, z, None, dst,
                                     0, None, None, bn_scale=scale, bn_shift=shift, pooled=pooled,
@@ -347,9 +351,7 @@ class BatchStructure(object):
     def aggregate_relu_bn_bwd(self, src, mode, eps, unit, d_pooled, d_score, u, d_neg, n_neg, dy, stats, tail=None):
         """Backward aggregation of `src` fused with the relu / BatchNorm backward reduction of `unit` (the last unit of
         the layer below) when the batch runs on the tcgen05 dense-block kernel; False, nothing launched, otherwise."""
-        if self.bitmap_addr is None or FORCE_CSR_AGGREGATE or FORCE_UNFUSED_BACKWARD or not _ops.dense_aggregate_ok(src, dy):
-            return False
-        if mode != 0 and self.has_isolated:
+        if FORCE_UNFUSED_BACKWARD or not self._on_tc(src, dy, None, mode):
             return False
         return _ops.aggregate_dense_relu_bn_bwd(self.bitmap_addr, self.node_off, self.rowptr, self.n_graphs, self.n_max,
                                                 src, mode, eps, unit.z, unit.scale, unit.shift, unit.mean, unit.rstd,
@@ -359,10 +361,7 @@ class BatchStructure(object):
         """Layer 0 as a row gather of `table` when every graph carries the same tag sequence: dst = Agg(table[tags]) (+ self
         term) + bias and stats += its column statistics, the table staying resident in the kernel's shared memory
         (ops.aggregate_dense_table); False, nothing launched, when the batch does not run on the tcgen05 kernel."""
-        if (self.bitmap_addr is None or FORCE_CSR_AGGREGATE or not self.same_tags or self.uniform_n is None or mode == 2
-                or not _ops.dense_aggregate_ok(table, dst, bias)):
-            return False
-        if mode != 0 and self.has_isolated:
+        if not (self.same_tags and self.uniform_n is not None and mode != 2 and self._on_tc(table, dst, bias, mode)):
             return False
         return _ops.aggregate_dense_table(self.bitmap_addr, self.node_off, self.rowptr, self.n_graphs, self.n_max, table,
                                           self.tags[:self.uniform_n], dst, mode, eps, bias, stats, tail)
@@ -370,9 +369,7 @@ class BatchStructure(object):
     def aggregate_affine(self, dy, z, coef, dst, mode):
         """dst = Agg(coef[0]*dy + coef[1]*z + coef[2]) when the batch runs on the tcgen05 dense-block kernel (the affine
         is applied to the rows as they are loaded); False, with nothing launched, otherwise."""
-        if self.bitmap_addr is None or FORCE_CSR_AGGREGATE or not _ops.dense_aggregate_ok(dy, dst):
-            return False
-        if mode != 0 and self.has_isolated:
+        if not self._on_tc(dy, dst, None, mode):
             return False
         return _ops.aggregate_dense_affine(self.bitmap_addr, self.node_off, self.rowptr, self.n_graphs, self.n_max, dy, z,
                                            coef, dst, mode)
@@ -857,73 +854,94 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
     d_pooled = d_pooled.contiguous()
 
     d_h = None        # gradient reaching h_all[layer] from layer+1's aggregation
-    carry = None      # (dy, stats) of this layer's last unit when layer+1's aggregation kernel already produced them
+    ready = None      # (dy, stats, coef) of the next unit when the kernel that ran the unit above already produced them
     d_x = None
+    # per layer: the slices of the readout gradient and of the DGI terms that reach its h directly
+    side = [(d_pooled[:, s], u_mat[:, s] if u_mat is not None else None, d_neg[:, s] if d_neg is not None else None)
+            for s in (slice(layer * F, (layer + 1) * F) for layer in range(L))]
 
-    def roi_from_dp(dp, eps_l):
-        """ROI mode, layer 0 on a dense input: the node average of d_x = Agg^T dp (the reduction of dp itself with the
-        operator's row sums; under max pooling, which is not linear, of d_x - the [M, D] route)."""
-        if 0 in sv.max_state:
-            amax, cmin = sv.max_state[0]
-            d_in = torch.empty(M, dp.shape[1], dtype=torch.float32, device=dev)
-            _ops.aggregate_max_bwd(bs.rowptr, bs.colidx, dp, amax, cmin, eps_l, d_in)
-            _ops.segment_weighted_colsum(d_in, bs.node_off, roi)
-        else:
-            _ops.segment_weighted_colsum(dp, bs.node_off, roi, rowptr=bs.rowptr, mode=1 if average else 0, eps=eps_l)
-
-    def aggregate_into_layer_below(layer, dp, eps_l):
-        """d_h of layer-1 = Agg^T(dp); fused with layer-1's relu / BatchNorm backward reduction when possible."""
-        below = sv.layers[layer - 1][-1]
-        slb = slice((layer - 1) * F, layer * F)
-        if layer not in sv.max_state and below.z.shape[1] == dp.shape[1]:
-            dy_b = torch.empty(M, dp.shape[1], dtype=torch.float32, device=dev)
-            st_b = zp.f64(2 * dp.shape[1])
-            coef_b, tail_b = _bn_backward_tail(below, st_b[0], comm)
-            if bs.aggregate_relu_bn_bwd(dp, bwd_mode, eps_l, below, d_pooled[:, slb], d_score,
-                                        u_mat[:, slb] if u_mat is not None else None,
-                                        d_neg[:, slb] if d_neg is not None else None, n_neg, dy_b, st_b[0], tail_b):
-                return None, (dy_b, st_b, coef_b)
-        d_prev = torch.empty(M, dp.shape[1], dtype=torch.float32, device=dev)
+    def agg_transpose(layer, dp, eps_l):
+        """Agg^T dp for the aggregation that feeds `layer` (its max-pooling backward when that layer ran max pooling)."""
+        out = torch.empty(M, dp.shape[1], dtype=torch.float32, device=dev)
         if layer in sv.max_state:
             amax, cmin = sv.max_state[layer]
-            _ops.aggregate_max_bwd(bs.rowptr, bs.colidx, dp, amax, cmin, eps_l, d_prev)
+            _ops.aggregate_max_bwd(bs.rowptr, bs.colidx, dp, amax, cmin, eps_l, out)
         else:
-            bs.aggregate(dp, None, d_prev, bwd_mode, eps_l, None)
-        return d_prev, None
+            bs.aggregate(dp, None, out, bwd_mode, eps_l, None)
+        return out
+
+    def bn_coef(u, stats, coef_ready, p2p=None):
+        """[3, F] BatchNorm-backward coefficients of `u`, dz = A*dy + B*z + C: coef_ready when the kernel that produced
+        `stats` already formed them in its last CTA."""
+        if coef_ready is not None:
+            return coef_ready
+        coef = torch.empty(3, u.w.shape[0], dtype=torch.float32, device=dev)
+        _ops.bn_bwd_coeffs(stats if u.count > 0.0 else None, u.count, u.gamma, u.mean, u.rstd, coef, p2p=p2p)
+        return coef
+
+    def max_pool_x_grad(dz, w, eps_l):
+        """Input gradient of the one-hot layer 0 under max pooling, from dz = d loss / d z_0."""
+        if max_first is None:
+            raise RuntimeError("input gradients under max pooling need the neighbour-list order "
+                               "(use compute_saliency / compute_saliency_batched)")
+        dp0 = torch.empty(M, w.shape[1], dtype=torch.float32, device=dev)
+        _ops.linear(dz, w, True, None, None, None, dp0, None)         # d loss / d pooled_0 = dz @ W1
+        return max_pool_onehot_input_grad(bs, dp0, max_first, eps_l)
+
+    def through_aggregation(layer, dp, eps_l):
+        """dp = d loss / d pooled_layer, the output of the layer's neighbour aggregation: d eps, then the gradient of the
+        aggregation's input. Above layer 0 that sets d_h of the layer below = Agg^T dp - or, when the aggregation kernel
+        also ran that layer's relu / BatchNorm backward reduction, `ready`. At layer 0 it forms the ROI reduction or d_x."""
+        nonlocal d_h, ready, d_x
+        roi0 = layer == 0 and roi is not None
+        if learn_eps and not roi0:
+            _ops.dot_rows(dp, sv.x_dense if layer == 0 else sv.h_all[layer - 1], None, d_eps[layer:layer + 1])
+        if layer > 0:
+            below = sv.layers[layer - 1][-1]
+            if layer not in sv.max_state and below.z.shape[1] == dp.shape[1]:
+                dy_b = torch.empty(M, dp.shape[1], dtype=torch.float32, device=dev)
+                st_b = zp.f64(2 * dp.shape[1])
+                coef_b, tail_b = _bn_backward_tail(below, st_b[0], comm)
+                d_pool_b, u_b, d_neg_b = side[layer - 1]
+                if bs.aggregate_relu_bn_bwd(dp, bwd_mode, eps_l, below, d_pool_b, d_score, u_b, d_neg_b, n_neg, dy_b,
+                                            st_b[0], tail_b):
+                    d_h, ready = None, (dy_b, st_b, coef_b)
+                    return
+            d_h = agg_transpose(layer, dp, eps_l)
+        elif roi0:
+            # the node average of d_x = Agg^T dp: the reduction of dp itself with the operator's row sums; under max
+            # pooling, which is not linear, of d_x - the [M, D] route
+            if 0 in sv.max_state:
+                _ops.segment_weighted_colsum(agg_transpose(0, dp, eps_l), bs.node_off, roi)
+            else:
+                _ops.segment_weighted_colsum(dp, bs.node_off, roi, rowptr=bs.rowptr, mode=1 if average else 0, eps=eps_l)
+        elif need_x_grad:
+            d_x = agg_transpose(0, dp, eps_l)
 
     pidx = 3 + 4 * sum(len(u) for u in sv.layers)
     for layer in range(L - 1, -1, -1):
         units = sv.layers[layer]
         pidx -= 4 * len(units)
-        sl = slice(layer * F, (layer + 1) * F)
         eps_l = eps_p[layer:layer + 1] if learn_eps else None
-        h_prev = sv.h_all[layer - 1] if layer > 0 and learn_eps else None      # materialised under learn_eps
+        need_dp = layer > 0 or need_x_grad or learn_eps or roi is not None      # d loss / d pooled_layer has a use
         dz = None
-        pending = None        # (dy, stats) of the current unit when the previous fused call already produced them
         for j in range(len(units) - 1, -1, -1):
             u = units[j]
             n_out, n_in = u.w.shape[0], u.w.shape[1]
-            coef_ready = None      # gnm_bn_bwd_coeffs' output when the kernel that produced `stats` already ran it (tail)
-            if pending is not None:
-                dy, (stats, st_chunk, st_off), coef_ready = pending
-                pending = None
-            elif j == len(units) - 1 and carry is not None:
-                dy, (stats, st_chunk, st_off), coef_ready = carry
-                carry = None
+            if ready is not None:
+                (dy, (stats, st_chunk, st_off), coef_ready), ready = ready, None
             else:
                 dy = torch.empty(M, n_out, dtype=torch.float32, device=dev)
                 stats, st_chunk, st_off = zp.f64(2 * n_out)
                 coef_t, tail_t = _bn_backward_tail(u, stats, comm)
                 if j == len(units) - 1:
-                    took = _ops.relu_bn_bwd_reduce(u.z, u.scale, u.shift, u.mean, u.rstd, d_h, d_pooled[:, sl],
-                                                   bs.pool_scale, d_score, u_mat[:, sl] if u_mat is not None else None,
-                                                   d_neg[:, sl] if d_neg is not None else None, n_neg, bs.node_off, B, dy,
-                                                   stats, tail=tail_t)
+                    d_pool_l, u_l, d_neg_l = side[layer]
+                    d_out = (d_h, d_pool_l, bs.pool_scale, d_score, u_l, d_neg_l, n_neg)
                 else:
-                    took = _ops.relu_bn_bwd_reduce(u.z, u.scale, u.shift, u.mean, u.rstd, dz, None, None, None, None, None,
-                                                   0, bs.node_off, B, dy, stats, tail=tail_t)
-                if took is True:
-                    coef_ready = coef_t
+                    d_out = (dz, None, None, None, None, None, 0)
+                took = _ops.relu_bn_bwd_reduce(u.z, u.scale, u.shift, u.mean, u.rstd, *d_out, bs.node_off, B, dy, stats,
+                                               tail=tail_t)
+                coef_ready = coef_t if took is True else None
             use_batch = u.count > 0.0
             gather0 = j == 0 and layer == 0 and sv.use_gather0
             fused = (not gather0) and (not FORCE_UNFUSED_BACKWARD) and n_out <= FUSED_BWD_MAX and n_in <= FUSED_BWD_MAX
@@ -950,18 +968,10 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
                 # one streaming reduction of dy with the BatchNorm-backward affine on load, then a [B, F] x [F, D] product
                 if model.neighbor_pooling_type == "max":
                     # max pooling is not linear: the input gradient itself, then its average
-                    if max_first is None:
-                        raise RuntimeError("input gradients under max pooling need the neighbour-list order")
                     _ops.bn_bwd_apply(u.z, u.mean, u.rstd, u.gamma, stats if use_batch else None, u.count, dy)
-                    dp0 = torch.empty(M, n_in, dtype=torch.float32, device=dev)
-                    _ops.linear(dy, u.w, True, None, None, None, dp0, None)
-                    _ops.segment_weighted_colsum(max_pool_onehot_input_grad(bs, dp0, max_first, eps_l), bs.node_off, roi)
+                    _ops.segment_weighted_colsum(max_pool_x_grad(dy, u.w, eps_l), bs.node_off, roi)
                     continue
-                if coef_ready is not None:
-                    coef0 = coef_ready
-                else:
-                    coef0 = torch.empty(3, n_out, dtype=torch.float32, device=dev)
-                    _ops.bn_bwd_coeffs(stats if use_batch else None, u.count, u.gamma, u.mean, u.rstd, coef0)
+                coef0 = bn_coef(u, stats, coef_ready)
                 dz_sum = torch.empty(B, n_out, dtype=torch.float32, device=dev)
                 _ops.segment_weighted_colsum(dy, bs.node_off, dz_sum, z=u.z if use_batch else None, coef=coef0,
                                              rowptr=bs.rowptr, mode=1 if average else 0, eps=eps_l)
@@ -970,11 +980,7 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
             if fused:
                 # one pass: BatchNorm-backward apply (folded into the load as dz = A*dy + B*z + C), dW, db, dX and -
                 # for an inner unit - the ReLU mask + BatchNorm-backward reduction of the unit below
-                if coef_ready is not None:
-                    coef = coef_ready
-                else:
-                    coef = torch.empty(3, n_out, dtype=torch.float32, device=dev)
-                    _ops.bn_bwd_coeffs(stats if use_batch else None, u.count, u.gamma, u.mean, u.rstd, coef, p2p=p2p)
+                coef = bn_coef(u, stats, coef_ready, p2p)
                 if j > 0:
                     p = units[j - 1]
                     dy_prev = torch.empty(M, n_in, dtype=torch.float32, device=dev)
@@ -982,43 +988,25 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
                     coef_p, tail_p = _bn_backward_tail(p, stats_prev[0], comm)
                     took = _ops.linear_bwd(dy, u.z, coef, p.z, p.scale, p.shift, p.mean, p.rstd, u.w, dw, db, dy_prev,
                                            stats_prev[0], tail=tail_p)
-                    pending = (dy_prev, stats_prev, coef_p if took is True else None)
+                    ready = (dy_prev, stats_prev, coef_p if took is True else None)
                 else:
-                    need_dp = layer > 0 or need_x_grad or learn_eps or roi is not None
                     dp = torch.empty(M, n_in, dtype=torch.float32, device=dev) if need_dp else None
                     _ops.linear_bwd(dy, u.z, coef, u.x_in, None, None, None, None, u.w, dw, db, dp, None)
                     if need_dp:
-                        src = sv.x_dense if layer == 0 else h_prev
-                        if learn_eps and not (layer == 0 and roi is not None):
-                            _ops.dot_rows(dp, src, None, d_eps[layer:layer + 1])
-                        if layer > 0:
-                            d_h, carry = aggregate_into_layer_below(layer, dp, eps_l)
-                        elif roi is not None:
-                            roi_from_dp(dp, eps_l)
-                        elif need_x_grad:
-                            d_x = torch.empty(M, n_in, dtype=torch.float32, device=dev)
-                            if layer in sv.max_state:
-                                amax, cmin = sv.max_state[layer]
-                                _ops.aggregate_max_bwd(bs.rowptr, bs.colidx, dp, amax, cmin, eps_l, d_x)
-                            else:
-                                bs.aggregate(dp, None, d_x, bwd_mode, eps_l, None)
+                        through_aggregation(layer, dp, eps_l)
                 grads[gi], grads[gi + 1] = dw, db
                 continue
-            g_agg = coef0 = None
-            if gather0 and not learn_eps and not (need_x_grad and model.neighbor_pooling_type == "max"):
-                # layer-0 gather unit: dz is only ever aggregated, so the BatchNorm-backward apply rides on the
-                # aggregation kernel's row loads (dz = A*dy + B*z + C is never written); d bias follows in closed form
-                if coef_ready is not None:
-                    coef0 = coef_ready
-                else:
-                    coef0 = torch.empty(3, n_out, dtype=torch.float32, device=dev)
-                    _ops.bn_bwd_coeffs(stats if use_batch else None, u.count, u.gamma, u.mean, u.rstd, coef0)
-                g_try = torch.empty(M, n_out, dtype=torch.float32, device=dev)
-                if bs.aggregate_affine(dy, u.z, coef0, g_try, bwd_mode):
-                    g_agg = g_try
-            if g_agg is None:
+            folded = False
+            if gather0:
+                g_agg = torch.empty(M, n_out, dtype=torch.float32, device=dev)
+                if not learn_eps and not (need_x_grad and model.neighbor_pooling_type == "max"):
+                    # layer-0 gather unit: dz is only ever aggregated, so the BatchNorm-backward apply rides on the
+                    # aggregation kernel's row loads (dz = A*dy + B*z + C is never written); d bias follows in closed form
+                    coef0 = bn_coef(u, stats, coef_ready)
+                    folded = bool(bs.aggregate_affine(dy, u.z, coef0, g_agg, bwd_mode))
+            if not folded:
                 _ops.bn_bwd_apply(u.z, u.mean, u.rstd, u.gamma, stats if use_batch else None, u.count, dy)
-            dz_u = dy                                                # now d loss / d z_j (unless g_agg is set)
+            dz_u = dy                                                # now d loss / d z_j (unless folded)
             if j > 0:
                 p = units[j - 1]
                 _ops.linear_wgrad(dz_u, p.z, p.scale, p.shift, dw, db)
@@ -1029,9 +1017,7 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
             # ---- first unit of the layer: input is the neighbour aggregation --------------------
             if gather0:
                 # z0 = Agg(W1^T[tags]) + b:  dW1^T[t] = sum_{tags[r]=t} (Agg^T dz)[r]
-                folded = g_agg is not None
                 if not folded:
-                    g_agg = torch.empty(M, n_out, dtype=torch.float32, device=dev)
                     bs.aggregate(dz_u, None, g_agg, bwd_mode, eps_l, None)
                 dw1t = zp.f32(n_in, n_out)
                 if bs.same_tags and n_out % 4 == 0:
@@ -1051,40 +1037,19 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
                     db = None
                 if learn_eps:
                     _ops.dot_rows(dz_u, sv.w1t, bs.tags, d_eps[layer:layer + 1])
-                if need_x_grad:
-                    if model.neighbor_pooling_type == "max":
-                        if max_first is None:
-                            raise RuntimeError("input gradients under max pooling need the neighbour-list order "
-                                               "(use compute_saliency / compute_saliency_batched)")
-                        dp0 = torch.empty(M, n_in, dtype=torch.float32, device=dev)
-                        _ops.linear(dz_u, u.w, True, None, None, None, dp0, None)    # d loss / d pooled_0 = dz @ W1
-                        d_x = max_pool_onehot_input_grad(bs, dp0, max_first, eps_l)
-                        grads[gi], grads[gi + 1] = dw, db
-                        continue
+                if need_x_grad and model.neighbor_pooling_type == "max":
+                    d_x = max_pool_x_grad(dz_u, u.w, eps_l)
+                elif need_x_grad:
                     d_x = torch.empty(M, n_in, dtype=torch.float32, device=dev)
                     _ops.linear(g_agg, u.w, True, None, None, None, d_x, None)   # (Agg^T dz) @ W1
             else:
                 roi0 = layer == 0 and roi is not None
                 if not roi0:
                     _ops.linear_wgrad(dz_u, u.x_in, None, None, dw, db)
-                need_dp = layer > 0 or need_x_grad or learn_eps or roi0
                 if need_dp:
-                    src = sv.x_dense if layer == 0 else h_prev
                     dp = torch.empty(M, n_in, dtype=torch.float32, device=dev)
                     _ops.linear(dz_u, u.w, True, None, None, None, dp, None)
-                    if learn_eps and not roi0:
-                        _ops.dot_rows(dp, src, None, d_eps[layer:layer + 1])
-                    if layer > 0:
-                        d_h, carry = aggregate_into_layer_below(layer, dp, eps_l)
-                    elif roi0:
-                        roi_from_dp(dp, eps_l)
-                    elif need_x_grad:
-                        d_x = torch.empty(M, n_in, dtype=torch.float32, device=dev)
-                        if layer in sv.max_state:
-                            amax, cmin = sv.max_state[layer]
-                            _ops.aggregate_max_bwd(bs.rowptr, bs.colidx, dp, amax, cmin, eps_l, d_x)
-                        else:
-                            bs.aggregate(dp, None, d_x, bwd_mode, eps_l, None)
+                    through_aggregation(layer, dp, eps_l)
             grads[gi], grads[gi + 1] = dw, db
     # float64 accumulators -> float32 gradients, one conversion per pool buffer (and one more for the shares of the
     # synchronised BatchNorm reductions: after the all-reduce those are sums over ALL ranks of gradients of each

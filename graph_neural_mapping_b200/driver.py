@@ -415,6 +415,28 @@ def roi_saliency(model, graphs, classes=(0, 1), batch=1024):
     return out
 
 
+def integrated_gradients(model, graphs, classes=(0, 1), steps=50, batch=1024, return_delta=False):
+    """Integrated gradients (zero baseline, midpoint rule with `steps` points): float32 [G, len(classes), D], entry
+    [i, k] = the node average of graph i's attribution map for classes[k] (`compute_integrated_gradients_batched`, the
+    same node average as `roi_saliency`), and with return_delta the [G, len(classes)] completeness gap. Computed in
+    calls of `batch` graphs, one D2H copy per call. Graphs may differ in size; node features must be one-hot and the
+    neighbour pooling sum or average."""
+    d = int(_engine.layer_units(model, 0)[0][0].weight.shape[1])          # input_dim
+    out = np.empty((len(graphs), len(classes), d), dtype=np.float32)
+    delta = np.empty((len(graphs), len(classes)), dtype=np.float32)
+    per = len(classes) * d
+    for i in range(0, len(graphs), batch):
+        chunk = graphs[i:i + batch]
+        n = len(chunk)
+        res = model.compute_integrated_gradients_batched(chunk, classes, steps=steps, return_delta=return_delta)
+        flat = torch.cat([res[0].reshape(n, per), res[1]], 1) if return_delta else res.reshape(n, per)
+        host = flat.cpu().numpy()                                          # one copy for both results
+        out[i:i + n] = host[:, :per].reshape(n, len(classes), d)
+        if return_delta:
+            delta[i:i + n] = host[:, per:]
+    return (out, delta) if return_delta else out
+
+
 def saliency_maps_to_npy(model, graphs, cls, path, batch=64):
     """`np.save(path, get_saliency_map(model, graphs, cls))` (main.py:168-172) without holding the array: the `.npy`
     file is created as a memory map of its final shape [G, N, D] and filled batch by batch from the pinned double

@@ -22,6 +22,7 @@ import os
 from .. import dist as _dist
 from .. import engine as _engine
 from .. import graphed as _graphed
+from .. import ops as _ops
 
 
 class _HeadsFunction(torch.autograd.Function):
@@ -318,6 +319,94 @@ class GIN_InfoMaxReg(nn.Module):
                 dg_f = torch.cat([w[c] for w in heads]).expand(b, -1).contiguous()
                 _engine.run_backward(self, sv, params, dg_f, None, False, _dist.SINGLE, max_first=max_first, roi=out[:, k])
         return out
+
+    def compute_integrated_gradients_batched(self, batch_graph, classes, steps=50, points_per_pass=1024,
+                                             return_delta=False):
+        """Integrated gradients with a zero baseline: float32 [B, len(classes), D] device tensor (and, with
+        return_delta, the [B, len(classes)] completeness gap). Entry [i, k, d] is the node average over graph i of
+        IG[n, d] = X[n, d] * (1/S) sum_s dF_c/dX(alpha_s X)[n, d], c = classes[k], alpha_s = (s + 1/2)/S (the midpoint
+        rule, S = steps), F_c the eval-mode class score compute_saliency differentiates - the same node average as
+        compute_roi_saliency_batched, so either can be painted onto ROIs; multiply by n_i for the per-graph sum.
+        delta[i, k] = n_i * sum_d out[i, k, d] - (F_c(X_i) - F_c(0)) tends to 0 as steps grows (completeness).
+
+        The path points run as one virtual batch per pass (exact in eval: a graph's outputs do not depend on its batch
+        companions): one forward serves every class, one hand-derived backward per class follows, layer 0 runs once per
+        real graph and no [N, D] tensor is formed (engine.run_forward's ig_z0, run_backward's ig). A pass holds at most
+        `points_per_pass` (graph, alpha) pairs: max(1, points_per_pass // steps) graphs, a graph's points spread over
+        several passes when steps > points_per_pass. Graphs may differ in size. Puts the model in eval() and leaves
+        every parameter's .grad untouched.
+
+        Needs one-hot node features (util.py:114-116) and sum or average neighbour pooling: max pooling is not linear in
+        the input, and its input gradient takes the [N, D] tie-rule route (compute_saliency_batched). ValueError
+        otherwise, and for classes out of range or steps < 1."""
+        self.eval()
+        classes = [int(c) for c in classes]
+        n_cls = self.linears_prediction[0].weight.shape[0]
+        if any(c < 0 or c >= n_cls for c in classes):
+            raise ValueError("classes must lie in [0, %d), got %s" % (n_cls, classes))
+        steps, points_per_pass = int(steps), int(points_per_pass)
+        if steps < 1 or points_per_pass < 1:
+            raise ValueError("steps and points_per_pass must be >= 1, got %d and %d" % (steps, points_per_pass))
+        if self.neighbor_pooling_type == "max":
+            raise ValueError("integrated gradients need sum or average neighbour pooling: max pooling is not linear in "
+                             "the input (use compute_saliency_batched for its input gradient)")
+        if not all(bn.track_running_stats for layer in range(self.num_layers)
+                   for _, bn in _engine.layer_units(self, layer)):
+            raise ValueError("integrated gradients need BatchNorm running statistics (eval mode per graph)")
+        dev = self.eps.device
+        lin0 = _engine.layer_units(self, 0)[0][0]
+        d_in, f0 = lin0.weight.shape[1], lin0.weight.shape[0]
+        b, n_c = len(batch_graph), len(classes)
+        out = torch.empty(b, n_c, d_in, dtype=torch.float32, device=dev)
+        delta = torch.empty(b, n_c, dtype=torch.float32, device=dev) if return_delta else None
+        if b > 0 and n_c > 0:
+            h = self._host_batch(batch_graph)
+            if not h.onehot:
+                raise ValueError("integrated gradients need one-hot node features (util.py:114-116)")
+        res = (out, delta) if return_delta else out
+        if b == 0 or n_c == 0:
+            return res
+        params = [p.detach() for p in _engine.flat_params(self)]
+        average = self.neighbor_pooling_type == "average"
+        eps_l = params[0][0:1] if self.learn_eps else None
+        w1t = lin0.weight.detach().t().contiguous()
+        heads = [lin.weight.detach() for lin in self.linears_prediction]
+        dg_rows = [torch.cat([w[c] for w in heads]) for c in classes]     # d score_c / d g_f (graphcnn.py:228-231)
+        alphas = ((torch.arange(steps, dtype=torch.float64) + 0.5) / steps).to(dev, torch.float32)
+        per_chunk = max(1, points_per_pass // steps)
+        points = min(steps, points_per_pass)
+        with torch.no_grad():
+            for i in range(0, b, per_chunk):
+                chunk = batch_graph[i:i + per_chunk]
+                rbs = self._structure(chunk)
+                # layer 0 without its bias on the real graphs: z0(alpha) = alpha * p0 + b
+                p0 = torch.empty(rbs.n_rows, f0, dtype=torch.float32, device=dev)
+                rbs.aggregate(w1t, rbs.tags, p0, 1 if average else 0, eps_l, None)
+                acc = torch.empty(n_c, rbs.n_rows, f0, dtype=torch.float32, device=dev)
+                for s0 in range(0, steps, points):
+                    k = min(points, steps - s0)
+                    vbs = self._structure([g for g in chunk for _ in range(k)])
+                    _, _, sv = _engine.run_forward(self, vbs, None, False, False, None, params, _dist.SINGLE,
+                                                   ig_z0=(p0, alphas[s0:s0 + k], rbs.node_off, k))
+                    for j in range(n_c):
+                        dg_f = dg_rows[j].expand(vbs.n_graphs, -1).contiguous()
+                        _engine.run_backward(self, sv, params, dg_f, None, False, _dist.SINGLE,
+                                             ig=(acc[j], rbs.node_off, k, 1.0 / steps, s0 > 0))
+                for j in range(n_c):
+                    # IG = X o ((Agg^T acc) W1): per node the row dot with its tag's W1 column, averaged per ROI
+                    t = torch.empty(rbs.n_rows, f0, dtype=torch.float32, device=dev)
+                    rbs.aggregate(acc[j], None, t, 2 if average else 0, eps_l, None)
+                    _ops.ig_attribute(t, w1t, rbs.tags, rbs.node_off, out[i:i + len(chunk), j])
+                if return_delta:
+                    # F_c(X) - F_c(0): a forward-only virtual batch of the two endpoints
+                    ends = torch.tensor([1.0, 0.0], dtype=torch.float32, device=dev)
+                    vbs = self._structure([g for g in chunk for _ in range(2)])
+                    g_f, _, _ = _engine.run_forward(self, vbs, None, False, False, None, params, _dist.SINGLE,
+                                                    ig_z0=(p0, ends, rbs.node_off, 2))
+                    score = self._heads(g_f).view(len(chunk), 2, n_cls)[:, :, classes]
+                    n_g = torch.from_numpy(rbs.node_counts.astype(np.float32)).to(dev).unsqueeze(1)
+                    delta[i:i + len(chunk)] = n_g * out[i:i + len(chunk)].sum(2) - (score[:, 0] - score[:, 1])
+        return res
 
 
 GraphCNN = GIN_InfoMaxReg      # the name BASELINE.json's north_star uses for this class

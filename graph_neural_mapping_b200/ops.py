@@ -58,7 +58,7 @@ def device_info():
 
 KERNEL_FAMILIES = ("aggregate_csr", "aggregate_mma_sync", "aggregate_tc", "linear_ffma", "linear_tc", "linear_bwd_ffma",
                    "linear_bwd_dx_tc", "linear_wgrad_tc", "linear_wgrad_ffma", "other", "linear_bwd_onepass_tc",
-                   "segment_colsum")
+                   "segment_colsum", "ig_expand", "ig_accumulate", "ig_attribute")
 
 
 def launch_counts():
@@ -341,6 +341,45 @@ def segment_weighted_colsum(x, node_off, out, z=None, coef=None, rowptr=None, mo
                                                      int(out.shape[0]), int(out.shape[1]), _ptr(rowptr, torch.int32),
                                                      int(mode), _ptr(eps, torch.float32), op, ldo, _stream(out)),
                   "gnm_segment_weighted_colsum")
+    return out
+
+
+# ---- integrated gradients: the virtual batch of path points (each real graph repeated `points` times, graph-major) ----
+
+def ig_expand(p, bias, alpha, node_off, points, z):
+    """z[(g, s, i)] = alpha[s] * p[node_off[g] + i] + bias (include/gnm.h: gnm_ig_expand): layer 0's output at every path
+    point from one real-batch aggregation p. z is [points * p.shape[0], W]. Returns z."""
+    pp, ldp = _mat(p)
+    zp, ldz = _mat(z)
+    _libmod.check(_lib().gnm_ig_expand(pp, ldp, _ptr(bias, torch.float32), _ptr(alpha, torch.float32),
+                                       _ptr(node_off, torch.int32), int(node_off.shape[0]) - 1, int(p.shape[0]),
+                                       int(points), int(p.shape[1]), zp, ldz, _stream(z)), "gnm_ig_expand")
+    return z
+
+
+def ig_accumulate(dy, coef, node_off, points, weight, out, accumulate):
+    """out[r] (+)= weight * coef[0] o sum_s dy[(g, s, r - node_off[g])] (include/gnm.h: gnm_ig_accumulate): the
+    quadrature sum of the path points' layer-0 gradients on the real rows, BatchNorm-backward (eval) on load. Returns out."""
+    dp, ldd = _mat(dy)
+    op, ldo = _mat(out)
+    _libmod.check(_lib().gnm_ig_accumulate(dp, ldd, _ptr(coef, torch.float32), _ptr(node_off, torch.int32),
+                                           int(node_off.shape[0]) - 1, int(out.shape[0]), int(points), int(out.shape[1]),
+                                           float(weight), int(bool(accumulate)), op, ldo, _stream(out)),
+                  "gnm_ig_accumulate")
+    return out
+
+
+def ig_attribute(t, table, tags, node_off, out):
+    """out[g, d] = (1/n_g) sum over graph g's nodes n with tags[n] = d of <t[n], table[d]> (include/gnm.h:
+    gnm_ig_attribute; NaN rows where t is not finite). out [B, D] may be a strided view. Returns out."""
+    if table.shape[0] != out.shape[1]:
+        raise RuntimeError("ig_attribute: table has %d rows, out %d columns" % (table.shape[0], out.shape[1]))
+    tp, ldt = _mat(t)
+    wp, ldw = _mat(table)
+    op, ldo = _mat(out)
+    _libmod.check(_lib().gnm_ig_attribute(tp, ldt, wp, ldw, int(out.shape[1]), _ptr(tags, torch.int32),
+                                          _ptr(node_off, torch.int32), int(out.shape[0]), int(t.shape[1]), op, ldo,
+                                          _stream(out)), "gnm_ig_attribute")
     return out
 
 

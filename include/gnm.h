@@ -33,7 +33,7 @@ extern "C" {
 #define GNM_ERR_TOO_LARGE (-2)
 #define GNM_ERR_ALIGN (-3)
 
-#define GNM_ABI_VERSION 25
+#define GNM_ABI_VERSION 26
 
 typedef void* gnm_stream_t;
 
@@ -92,7 +92,8 @@ int gnm_device_info(int* sm_count, int* cc_major, int* cc_minor, int64_t* smem_o
  * (a kernel recorded during CUDA-graph capture counts once, its replays are the caller's to count). Families:
  * 0 aggregate (CSR warp-per-row), 1 aggregate (mma.sync dense blocks), 2 aggregate (tcgen05), 3 linear (FFMA),
  * 4 linear (tcgen05), 5 linear_bwd (fused FFMA), 6 linear_bwd dX (tcgen05), 7 linear_bwd dW (tcgen05),
- * 8 linear_wgrad (FFMA), 9 every other kernel, 10 linear_bwd one-pass dX + dW (tcgen05), 11 segment_weighted_colsum.
+ * 8 linear_wgrad (FFMA), 9 every other kernel, 10 linear_bwd one-pass dX + dW (tcgen05), 11 segment_weighted_colsum,
+ * 12 ig_expand, 13 ig_accumulate, 14 ig_attribute.
  * Returns the number of families (>= 0) or GNM_ERR_BAD_ARG.
  * Tests use it to prove WHICH kernel family a code path ran; bench.py to count launches. */
 int gnm_launch_counts(int64_t* out, int n);
@@ -475,6 +476,39 @@ int gnm_adam_step(float* const* params, const float* const* grads, const int32_t
 int gnm_segment_weighted_colsum(const float* x, int64_t ldx, const float* z, int64_t ldz, const float* coef,
                                 const int32_t* node_off, int n_graphs, int width, const int32_t* rowptr, int mode,
                                 const float* eps, float* out, int64_t ld_out, gnm_stream_t stream);
+
+/* ---- integrated gradients (zero baseline, one-hot layer-0 input) -------------------------------------------------
+ * IG of the class score F_c at the one-hot input X: IG[n, d] = X[n, d] * sum_s w_s dF_c/dX (alpha_s X)[n, d]. Layer 0 is
+ * linear in X (z0(alpha) = alpha * Agg(X) W1^T + b), so the path points run as a VIRTUAL BATCH that repeats every real
+ * graph g (rows node_off[g] .. node_off[g+1], n_g rows; node_off[0] = 0, node_off[n_graphs] = n_rows) `points` times,
+ * graph-major: virtual row of (graph g, point s, node i) = points * node_off[g] + s * n_g + i. All three calls sum in a
+ * fixed order without atomics (bit-reproducible). Vectorised when width and the leading dimensions are multiples of 4
+ * and the row operands 16-byte aligned; any width >= 1 and stride otherwise. Negative sizes return GNM_ERR_BAD_ARG;
+ * an empty problem returns GNM_OK with no launch.
+ *
+ * gnm_ig_expand: layer 0's pre-BatchNorm output at every point from ONE real-batch aggregation p = Agg(X) W1^T (no bias):
+ *   z[(g, s, i)] = alpha[s] * p[node_off[g] + i] + bias        c < width; bias ([width]) nullable, alpha [points]
+ *   z is [points * n_rows, width]. */
+int gnm_ig_expand(const float* p, int64_t ldp, const float* bias, const float* alpha, const int32_t* node_off,
+                  int n_graphs, int n_rows, int points, int width, float* z, int64_t ldz, gnm_stream_t stream);
+/* gnm_ig_accumulate: the quadrature sum of the points' layer-0 gradients back on the real rows, the eval-mode
+ * BatchNorm-backward affine applied on load (cB = cC = 0 with running statistics, so z is not read):
+ *   out[r] = (accumulate ? out[r] : 0) + weight * cA o sum_{s < points} dy[(g, s, r - node_off[g])]   r in graph g
+ * coef = [cA | ...] (gnm_bn_bwd_coeffs' output; only the first `width` floats are read) nullable: cA = 1. The points
+ * are summed in ascending order. accumulate = 1 lets a graph's points be split over several calls. */
+int gnm_ig_accumulate(const float* dy, int64_t ldy, const float* coef, const int32_t* node_off, int n_graphs,
+                      int n_rows, int points, int width, float weight, int accumulate, float* out, int64_t ld_out,
+                      gnm_stream_t stream);
+/* gnm_ig_attribute: the node-averaged attribution per ROI from t = Agg^T(accumulated dz) ([n_rows, width], real batch)
+ * and the layer-0 table W1^T ([n_table_rows, width]):
+ *   a[n] = <t[n], table[tags[n]]>          (the per-row form of gnm_dot_rows with b_map = tags)
+ *   out[g, d] = (1/n_g) sum_{n in g, tags[n] = d} a[n]          d < n_table_rows (zeros where no node carries tag d)
+ * Duplicate tags within a graph add up, in node order. A tag outside [0, n_table_rows) contributes nothing. An empty
+ * graph yields zeros. A non-finite entry in any row t[n] of graph g makes out[g, :] NaN: the full attribution
+ * X[n, d] * (t W1)[n, d] is 0 * non-finite = NaN in the columns where X is 0, and the node average carries it. */
+int gnm_ig_attribute(const float* t, int64_t ldt, const float* table, int64_t ld_table, int n_table_rows,
+                     const int32_t* tags, const int32_t* node_off, int n_graphs, int width, float* out, int64_t ld_out,
+                     gnm_stream_t stream);
 
 /* ---- data parallel: synchronised BatchNorm sums over NVLink peer memory ------------------------------
  * The reference is single-process; a global-batch BatchNorm needs the per-channel sums of all ranks before the next

@@ -17,7 +17,7 @@
 enum GnmKernelFamily {
     GNM_K_AGG_CSR = 0, GNM_K_AGG_MMA_SYNC, GNM_K_AGG_TC, GNM_K_LINEAR_FFMA, GNM_K_LINEAR_TC, GNM_K_LINEAR_BWD_FFMA,
     GNM_K_LINEAR_BWD_DX_TC, GNM_K_LINEAR_WGRAD_TC, GNM_K_LINEAR_WGRAD_FFMA, GNM_K_OTHER, GNM_K_LINEAR_BWD_ONEPASS_TC,
-    GNM_K_SEGMENT_COLSUM, GNM_K_IG_EXPAND, GNM_K_IG_ACCUMULATE, GNM_K_IG_ATTRIBUTE,
+    GNM_K_SEGMENT_COLSUM, GNM_K_IG_EXPAND, GNM_K_IG_ACCUMULATE, GNM_K_IG_ATTRIBUTE, GNM_K_OCCLUSION_EXPAND,
     GNM_K_FAMILIES
 };
 void gnm_count_launch(int family);     // gnm_dgi.cu

@@ -437,6 +437,19 @@ def integrated_gradients(model, graphs, classes=(0, 1), steps=50, batch=1024, re
     return (out, delta) if return_delta else out
 
 
+def roi_occlusion(model, graphs, classes=(0, 1), batch=1024):
+    """ROI occlusion (zero baseline): float32 [G, len(classes), D], entry [i, k, d] = (F_c(X_i) - F_c(X_i with column d
+    set to 0)) / n_i for c = classes[k] (`compute_roi_occlusion_batched`, the node-average convention of `roi_saliency`
+    and `integrated_gradients`). Computed in calls of `batch` graphs, one D2H copy per call. Graphs may differ in size;
+    node features must be one-hot, and under max neighbour pooling tags injective and edge lists duplicate-free."""
+    d = int(_engine.layer_units(model, 0)[0][0].weight.shape[1])          # input_dim
+    out = np.empty((len(graphs), len(classes), d), dtype=np.float32)
+    for i in range(0, len(graphs), batch):
+        chunk = graphs[i:i + batch]
+        out[i:i + len(chunk)] = model.compute_roi_occlusion_batched(chunk, classes).cpu().numpy()
+    return out
+
+
 def saliency_maps_to_npy(model, graphs, cls, path, batch=64):
     """`np.save(path, get_saliency_map(model, graphs, cls))` (main.py:168-172) without holding the array: the `.npy`
     file is created as a memory map of its final shape [G, N, D] and filled batch by batch from the pinned double

@@ -590,11 +590,12 @@ def _materialise_plan(model, bs, with_dgi):
     return need, on_load and with_dgi and dgi_ok
 
 
-def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, max_padded=None, bce=None, ig_z0=None):
+def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, max_padded=None, bce=None, z0=None):
     """graphcnn.py:194-251 (and :254-294 when with_dgi is False). Returns (g_f, d_logit, saved).
-    ig_z0 = (p, alpha, node_off, points), eval only: `bs` is the virtual batch of integrated gradients (each graph of a
-    real batch with offsets node_off repeated `points` times, graph-major) and layer 0's first Linear output at path
-    point s is alpha[s] * p + bias, p = Agg(X) W1^T of the real batch (ops.ig_expand) - no aggregation runs on it.
+    z0 = fill(bias, z), eval only: `bs` is a virtual batch whose graphs repeat those of a real batch, and fill writes
+    layer 0's first Linear output z [M, F] (bias included) from the real batch's aggregation p = Agg(X) W1^T - no
+    aggregation runs on the virtual batch at layer 0. Integrated gradients: alpha[s] * p + bias at every path point
+    (ops.ig_expand); occlusion: p + bias minus the rank-1 term of the occluded column (ops.occlusion_expand).
     bce = (grad_scale, loss_scale, loss_acc): the caller's loss on d_logit is BCEWithLogits against main.py:32's targets
     with these scales (driver.Trainer). The scoring pass then also adds the loss to loss_acc and forms the scorer's
     backward (saved.scored = (d_score, du, s2, d_bias)) when its kernel takes the shape; saved.scored is None otherwise
@@ -652,11 +653,9 @@ def run_forward(model, bs, neg_idx, training, with_dgi, x_dense, params, comm, m
             tail = _bn_forward_tail(u, stats, M, training, comm, buf=bn_all[layer] if last_unit else None)
             done = False
             if j == 0:
-                if layer == 0 and use_gather0 and ig_z0 is not None:
-                    # z0 is linear in the input: every path point's from one real-batch aggregation (eval: the BatchNorm
-                    # reads no statistics of z0)
-                    p0, alpha, real_off, points = ig_z0
-                    _ops.ig_expand(p0, u.b, alpha, real_off, points, u.z)
+                if layer == 0 and use_gather0 and z0 is not None:
+                    # z0 from one real-batch aggregation (eval: the BatchNorm reads no statistics of z0)
+                    z0(u.b, u.z)
                     u.x_in = None
                 elif layer == 0 and use_gather0:
                     # first layer as a row gather of W1^T (X_concat is one-hot): no dense X, no GEMM
@@ -796,9 +795,9 @@ def run_backward(model, sv, params, dg_f, dd_logit, need_x_grad, comm, max_first
     (1/n_g) sum_{n in g} dX[n], formed without dX where the layer-0 aggregation is linear (ops.segment_weighted_colsum:
     mean_n (Agg^T dz)[n] = (1/n_g) sum_m w_m dz[m], w_m the operator's row sums). Layer 0's parameter gradients are not
     formed then. Nothing here writes the saved forward state, so one forward serves a backward per class.
-    ig = (acc, node_off, points, weight, accumulate), for a forward run with ig_z0: integrated-gradients mode - the
-    layer-0 dz of every path point, weighted, is summed onto the real rows acc [M_real, F] (ops.ig_accumulate; written,
-    or added to when accumulate). Agg^T and W1 are applied once per real batch by the caller. Layer 0's parameter
+    ig = (acc, node_off, points, weight, accumulate), for a forward whose z0 ran ops.ig_expand: integrated-gradients
+    mode - the layer-0 dz of every path point, weighted, is summed onto the real rows acc [M_real, F] (ops.ig_accumulate;
+    written, or added to when accumulate). Agg^T and W1 are applied once per real batch by the caller. Layer 0's parameter
     gradients are not formed."""
     bs = sv.bs
     dev = params[0].device

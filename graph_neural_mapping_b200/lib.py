@@ -11,7 +11,7 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.path.join(CSRC, "libgnm.so")
-ABI_VERSION = 26
+ABI_VERSION = 27
 
 _c_i32 = ctypes.c_int
 _c_i64 = ctypes.c_int64
@@ -90,6 +90,8 @@ SIGNATURES = {
     "gnm_ig_expand": [_p, _c_i64, _p, _p, _p, _c_i32, _c_i32, _c_i32, _c_i32, _p, _c_i64, _p],
     "gnm_ig_accumulate": [_p, _c_i64, _p, _p, _c_i32, _c_i32, _c_i32, _c_i32, _c_f32, _c_i32, _p, _c_i64, _p],
     "gnm_ig_attribute": [_p, _c_i64, _p, _c_i64, _c_i32, _p, _p, _c_i32, _c_i32, _p, _c_i64, _p],
+    "gnm_occlusion_expand": [_p, _c_i64, _p, _p, _c_i64, _c_i32, _p, _p, _p, _p, _c_i32, _c_i32, _p, _p, _p, _c_i32,
+                             _c_i32, _c_i32, _p, _p, _c_i64, _p],
 }
 
 _lib = None

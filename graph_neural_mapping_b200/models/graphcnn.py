@@ -331,7 +331,7 @@ class GIN_InfoMaxReg(nn.Module):
 
         The path points run as one virtual batch per pass (exact in eval: a graph's outputs do not depend on its batch
         companions): one forward serves every class, one hand-derived backward per class follows, layer 0 runs once per
-        real graph and no [N, D] tensor is formed (engine.run_forward's ig_z0, run_backward's ig). A pass holds at most
+        real graph and no [N, D] tensor is formed (engine.run_forward's z0, run_backward's ig). A pass holds at most
         `points_per_pass` (graph, alpha) pairs: max(1, points_per_pass // steps) graphs, a graph's points spread over
         several passes when steps > points_per_pass. Graphs may differ in size. Puts the model in eval() and leaves
         every parameter's .grad untouched.
@@ -386,8 +386,8 @@ class GIN_InfoMaxReg(nn.Module):
                 for s0 in range(0, steps, points):
                     k = min(points, steps - s0)
                     vbs = self._structure([g for g in chunk for _ in range(k)])
-                    _, _, sv = _engine.run_forward(self, vbs, None, False, False, None, params, _dist.SINGLE,
-                                                   ig_z0=(p0, alphas[s0:s0 + k], rbs.node_off, k))
+                    fill = lambda bias, z: _ops.ig_expand(p0, bias, alphas[s0:s0 + k], rbs.node_off, k, z)
+                    _, _, sv = _engine.run_forward(self, vbs, None, False, False, None, params, _dist.SINGLE, z0=fill)
                     for j in range(n_c):
                         dg_f = dg_rows[j].expand(vbs.n_graphs, -1).contiguous()
                         _engine.run_backward(self, sv, params, dg_f, None, False, _dist.SINGLE,
@@ -401,12 +401,122 @@ class GIN_InfoMaxReg(nn.Module):
                     # F_c(X) - F_c(0): a forward-only virtual batch of the two endpoints
                     ends = torch.tensor([1.0, 0.0], dtype=torch.float32, device=dev)
                     vbs = self._structure([g for g in chunk for _ in range(2)])
-                    g_f, _, _ = _engine.run_forward(self, vbs, None, False, False, None, params, _dist.SINGLE,
-                                                    ig_z0=(p0, ends, rbs.node_off, 2))
+                    fill = lambda bias, z: _ops.ig_expand(p0, bias, ends, rbs.node_off, 2, z)
+                    g_f, _, _ = _engine.run_forward(self, vbs, None, False, False, None, params, _dist.SINGLE, z0=fill)
                     score = self._heads(g_f).view(len(chunk), 2, n_cls)[:, :, classes]
                     n_g = torch.from_numpy(rbs.node_counts.astype(np.float32)).to(dev).unsqueeze(1)
                     delta[i:i + len(chunk)] = n_g * out[i:i + len(chunk)].sum(2) - (score[:, 0] - score[:, 1])
         return res
+
+    def compute_roi_occlusion_batched(self, batch_graph, classes, occlusions_per_pass=1024):
+        """ROI occlusion with a zero baseline: float32 [B, len(classes), D] device tensor whose entry [i, k, d] is
+        (F_c(X_i) - F_c(X_i with column d set to 0)) / n_i, c = classes[k], F_c the eval-mode class score
+        compute_saliency differentiates. The 1/n_i is the node-average convention of compute_roi_saliency_batched and
+        compute_integrated_gradients_batched, so any of them can be painted onto ROIs; multiply by n_i for the score
+        drop itself. Zeroing column d zeroes every node tagged d. A tag absent from graph i gives exactly 0.0 and costs
+        no forward; a graph whose class score is not finite (average pooling's 0/0 at an isolated node under learn_eps)
+        gives NaN for every ROI.
+
+        The copies run as virtual batches of eval forwards (exact in eval: a graph's outputs do not depend on its batch
+        companions). A pass holds, for each real graph in it, one baseline copy followed by occluded copies of that
+        graph, so every difference is taken between two rows of the same forward; at most `occlusions_per_pass`
+        virtual graphs in all, and at least one occluded copy. Layer 0 is aggregated once per call on the real batch
+        and each copy's layer-0 output is that minus a rank-1 term (ops.occlusion_expand through engine.run_forward's
+        z0); no [N, D] tensor is formed and no backward runs, so one forward serves every class. Graphs may differ in
+        size. Puts the model in eval() and leaves every parameter's .grad untouched.
+
+        Needs one-hot node features (util.py:114-116), BatchNorm running statistics, and under max neighbour pooling a
+        batch whose layer-0 max equals its sum (injective tags and duplicate-free edge lists) and no node without
+        neighbours (learn_eps: no self loop; max pooling gives such a node the column minimum of the whole forward batch,
+        graphcnn.py:137-143, so a graph's score would depend on its companions). ValueError otherwise, and for classes
+        out of range or occlusions_per_pass < 1."""
+        self.eval()
+        classes = [int(c) for c in classes]
+        n_cls = self.linears_prediction[0].weight.shape[0]
+        if any(c < 0 or c >= n_cls for c in classes):
+            raise ValueError("classes must lie in [0, %d), got %s" % (n_cls, classes))
+        occlusions_per_pass = int(occlusions_per_pass)
+        if occlusions_per_pass < 1:
+            raise ValueError("occlusions_per_pass must be >= 1, got %d" % occlusions_per_pass)
+        if not all(bn.track_running_stats for layer in range(self.num_layers)
+                   for _, bn in _engine.layer_units(self, layer)):
+            raise ValueError("ROI occlusion needs BatchNorm running statistics (eval mode per graph)")
+        dev = self.eps.device
+        lin0 = _engine.layer_units(self, 0)[0][0]
+        d_in, f0 = lin0.weight.shape[1], lin0.weight.shape[0]
+        b, n_c = len(batch_graph), len(classes)
+        out = torch.zeros(b, n_c, d_in, dtype=torch.float32, device=dev)
+        if b == 0 or n_c == 0:
+            return out
+        h = self._host_batch(batch_graph)
+        if not h.onehot:
+            raise ValueError("ROI occlusion needs one-hot node features (util.py:114-116)")
+        if self.neighbor_pooling_type == "max" and not h.max0_as_sum:
+            raise ValueError("ROI occlusion under max neighbour pooling needs injective node tags and duplicate-free edge "
+                             "lists in every graph (layer 0's max then equals its sum)")
+        if self.neighbor_pooling_type == "max" and h.has_isolated:
+            raise ValueError("ROI occlusion under max neighbour pooling needs graphs without nodes without neighbours: "
+                             "such a node pools the column minimum of the whole forward batch (graphcnn.py:137-143), so "
+                             "its graph's occluded score would depend on the other copies in the pass")
+        params = [p.detach() for p in _engine.flat_params(self)]
+        mode = 1 if self.neighbor_pooling_type == "average" else 0
+        eps_l = params[0][0:1] if self.learn_eps else None
+        w1t = lin0.weight.detach().t().contiguous()
+        cls_d = torch.tensor(classes, dtype=torch.int64, device=dev)
+        inv_n = torch.from_numpy(1.0 / np.maximum(h.counts, 1)).to(dev, torch.float32)
+        bad = torch.zeros(b, n_c, dtype=torch.bool, device=dev)
+        with torch.no_grad():
+            rbs = self._structure(batch_graph, h)
+            # layer 0 without its bias on the real graphs: an occluded copy's z0 is p0 + b minus a rank-1 term
+            p0 = torch.empty(rbs.n_rows, f0, dtype=torch.float32, device=dev)
+            rbs.aggregate(w1t, rbs.tags, p0, mode, eps_l, None)
+            for v_graph, v_tag in occlusion_passes(h.node_off, rbs.tags.cpu().numpy(), occlusions_per_pass):
+                v = len(v_graph)
+                pos = np.arange(v, dtype=np.int32)
+                base = np.maximum.accumulate(np.where(v_tag < 0, pos, 0)).astype(np.int32)
+                copies = pos[v_tag >= 0]
+                idx = torch.from_numpy(np.concatenate([v_graph, v_tag, copies, base[copies], pos[v_tag < 0]]))
+                idx = idx.to(dev, non_blocking=True)
+                vg_d, vt_d = idx[:v], idx[v:2 * v]
+                n_k = len(copies)
+                copy_d, base_d, bl_d = (t.long() for t in (idx[2 * v:2 * v + n_k], idx[2 * v + n_k:2 * v + 2 * n_k],
+                                                           idx[2 * v + 2 * n_k:]))
+                vbs = self._structure([batch_graph[g] for g in v_graph.tolist()])
+                fill = lambda bias, z: _ops.occlusion_expand(p0, bias, w1t, rbs.rowptr, rbs.colidx, rbs.tags,
+                                                             rbs.node_off, rbs.n_max, vg_d, vt_d, vbs.node_off, mode,
+                                                             eps_l, z)
+                g_f, _, _ = _engine.run_forward(self, vbs, None, False, False, None, params, _dist.SINGLE, z0=fill)
+                score = self._heads(g_f).index_select(1, cls_d)                       # [V, C], eval: no dropout
+                g_k, d_k = vg_d[copy_d].long(), vt_d[copy_d].long()
+                out[g_k, :, d_k] = (score[base_d] - score[copy_d]) * inv_n[g_k].unsqueeze(1)
+                g_b = vg_d[bl_d].long()
+                bad[g_b] = bad[g_b] | ~torch.isfinite(score[bl_d])
+            out.masked_fill_(bad.unsqueeze(2), float("nan"))
+        return out
+
+
+def occlusion_passes(node_off, tags, occlusions_per_pass):
+    """The virtual batches of compute_roi_occlusion_batched: a list of (v_graph, v_tag) int32 arrays, one per pass, graph
+    major. For each real graph g (rows node_off[g] .. node_off[g+1] of `tags`) a pass holds one baseline copy (tag -1)
+    followed by occluded copies of g, one per tag present in g in ascending order; a graph whose tags do not fit one pass
+    continues in the next with a baseline copy of its own. A pass holds at most max(2, occlusions_per_pass) copies."""
+    cap = max(2, int(occlusions_per_pass))
+    passes, vg, vt = [], [], []
+    for g in range(len(node_off) - 1):
+        present = np.unique(tags[node_off[g]:node_off[g + 1]])
+        i = 0
+        while i < len(present):
+            if len(vg) + 2 > cap:
+                passes.append((vg, vt))
+                vg, vt = [], []
+            k = min(len(present) - i, cap - len(vg) - 1)
+            vg.extend([g] * (k + 1))
+            vt.append(-1)
+            vt.extend(present[i:i + k].tolist())
+            i += k
+    if vg:
+        passes.append((vg, vt))
+    return [(np.asarray(a, dtype=np.int32), np.asarray(t, dtype=np.int32)) for a, t in passes]
 
 
 GraphCNN = GIN_InfoMaxReg      # the name BASELINE.json's north_star uses for this class

@@ -58,7 +58,7 @@ def device_info():
 
 KERNEL_FAMILIES = ("aggregate_csr", "aggregate_mma_sync", "aggregate_tc", "linear_ffma", "linear_tc", "linear_bwd_ffma",
                    "linear_bwd_dx_tc", "linear_wgrad_tc", "linear_wgrad_ffma", "other", "linear_bwd_onepass_tc",
-                   "segment_colsum", "ig_expand", "ig_accumulate", "ig_attribute")
+                   "segment_colsum", "ig_expand", "ig_accumulate", "ig_attribute", "occlusion_expand")
 
 
 def launch_counts():
@@ -381,6 +381,32 @@ def ig_attribute(t, table, tags, node_off, out):
                                           _ptr(node_off, torch.int32), int(out.shape[0]), int(t.shape[1]), op, ldo,
                                           _stream(out)), "gnm_ig_attribute")
     return out
+
+
+# ---- ROI occlusion: the virtual batch of occluded copies (each real graph repeated, graph-major) ----------------------
+
+def occlusion_expand(p, bias, w1t, rowptr, colidx, tags, node_off, n_max, v_graph, v_tag, v_node_off, mode, eps, z):
+    """z[v_node_off[v] + i] = p[m] + bias - c_d[m] * w1t[d], m = node_off[v_graph[v]] + i, d = v_tag[v] (include/gnm.h:
+    gnm_occlusion_expand): layer 0's output for every occluded copy (v_tag >= 0) and baseline copy (v_tag < 0) of the
+    real batch (rowptr, colidx with global ids, tags, node_off; n_max its largest graph) from one real-batch
+    aggregation p. mode 0 sum, 1 average; eps [1] nullable (learn_eps). Returns z."""
+    n_virtual = int(v_graph.shape[0])
+    if v_tag.shape[0] != n_virtual or v_node_off.shape[0] != n_virtual + 1:
+        raise RuntimeError("occlusion_expand: v_graph, v_tag and v_node_off describe %d, %d and %d virtual graphs"
+                           % (n_virtual, v_tag.shape[0], v_node_off.shape[0] - 1))
+    if w1t.shape[1] != p.shape[1] or z.shape[1] != p.shape[1]:
+        raise RuntimeError("occlusion_expand: widths of p %d, w1t %d, z %d differ" % (p.shape[1], w1t.shape[1], z.shape[1]))
+    pp, ldp = _mat(p)
+    wp, ldw = _mat(w1t)
+    zp, ldz = _mat(z)
+    i32 = torch.int32
+    _libmod.check(_lib().gnm_occlusion_expand(pp, ldp, _ptr(bias, torch.float32), wp, ldw, int(w1t.shape[0]),
+                                              _ptr(rowptr, i32), _ptr(colidx, i32), _ptr(tags, i32), _ptr(node_off, i32),
+                                              int(node_off.shape[0]) - 1, int(n_max), _ptr(v_graph, i32),
+                                              _ptr(v_tag, i32), _ptr(v_node_off, i32), n_virtual, int(p.shape[1]),
+                                              int(mode), _ptr(eps, torch.float32), zp, ldz, _stream(z)),
+                  "gnm_occlusion_expand")
+    return z
 
 
 # ---- max pooling over neighbours ----------------------------------------------------------------

@@ -33,7 +33,7 @@ extern "C" {
 #define GNM_ERR_TOO_LARGE (-2)
 #define GNM_ERR_ALIGN (-3)
 
-#define GNM_ABI_VERSION 26
+#define GNM_ABI_VERSION 27
 
 typedef void* gnm_stream_t;
 
@@ -93,7 +93,7 @@ int gnm_device_info(int* sm_count, int* cc_major, int* cc_minor, int64_t* smem_o
  * 0 aggregate (CSR warp-per-row), 1 aggregate (mma.sync dense blocks), 2 aggregate (tcgen05), 3 linear (FFMA),
  * 4 linear (tcgen05), 5 linear_bwd (fused FFMA), 6 linear_bwd dX (tcgen05), 7 linear_bwd dW (tcgen05),
  * 8 linear_wgrad (FFMA), 9 every other kernel, 10 linear_bwd one-pass dX + dW (tcgen05), 11 segment_weighted_colsum,
- * 12 ig_expand, 13 ig_accumulate, 14 ig_attribute.
+ * 12 ig_expand, 13 ig_accumulate, 14 ig_attribute, 15 occlusion_expand.
  * Returns the number of families (>= 0) or GNM_ERR_BAD_ARG.
  * Tests use it to prove WHICH kernel family a code path ran; bench.py to count launches. */
 int gnm_launch_counts(int64_t* out, int n);
@@ -509,6 +509,29 @@ int gnm_ig_accumulate(const float* dy, int64_t ldy, const float* coef, const int
 int gnm_ig_attribute(const float* t, int64_t ldt, const float* table, int64_t ld_table, int n_table_rows,
                      const int32_t* tags, const int32_t* node_off, int n_graphs, int width, float* out, int64_t ld_out,
                      gnm_stream_t stream);
+
+/* ---- ROI occlusion (zero baseline, one-hot layer-0 input) --------------------------------------------------------
+ * Occluding ROI d sets input column d to 0. Layer 0's first Linear output then changes by a rank-1 term, so every
+ * occluded copy of a graph is written from ONE real-batch aggregation p = Agg(X) W1^T (no bias):
+ *   z[v_node_off[v] + i] = p[m] + bias - c_d[m] * w1t[d]          m = node_off[g] + i, g = v_graph[v], d = v_tag[v]
+ *   c_d[m] = s_m * #{n in CSR row m : tags[n] = d} + (eps ? (1 + *eps) * [tags[m] = d] : 0)
+ *   s_m = 1 (mode 0: sum, and max pooling where it equals the sum), 1 / (rowptr[m+1] - rowptr[m]) (mode 1: average)
+ * for every virtual graph v < n_virtual and node i < n_g of its real graph g (rows node_off[g] .. node_off[g+1] of the
+ * real batch; the virtual batch's v_node_off[v+1] - v_node_off[v] must equal n_g). rowptr / colidx (GLOBAL column ids)
+ * / tags describe the real batch, whose adjacency must be symmetric (the CSR rows of the nodes tagged d then list
+ * exactly the rows with a non-zero count). v_tag[v] < 0 or >= n_table_rows makes v a baseline copy: z = p + bias.
+ * A row whose c_d[m] is 0 is written as exactly p + bias, so baseline rows and unaffected rows are bit-identical across
+ * copies; s_m is formed only for a non-zero count, so an isolated row's 0/0 never multiplies a zero count. Counts are
+ * integer adds (exact in any order) and no atomics touch z: bit-reproducible. One CTA per virtual graph; n_max (the
+ * largest n_g) above 4096 returns GNM_ERR_TOO_LARGE. bias ([width]) and eps ([1]) nullable; w1t is [n_table_rows,
+ * width]. Vectorised when width and the leading dimensions are multiples of 4 and p, z, bias, w1t 16-byte aligned; any
+ * width >= 1 and stride otherwise. Negative sizes or a mode other than 0 / 1 return GNM_ERR_BAD_ARG; an empty problem
+ * (n_virtual, width or n_max 0) returns GNM_OK with no launch. */
+int gnm_occlusion_expand(const float* p, int64_t ldp, const float* bias, const float* w1t, int64_t ld_w1t,
+                         int n_table_rows, const int32_t* rowptr, const int32_t* colidx, const int32_t* tags,
+                         const int32_t* node_off, int n_graphs, int n_max, const int32_t* v_graph, const int32_t* v_tag,
+                         const int32_t* v_node_off, int n_virtual, int width, int mode, const float* eps, float* z,
+                         int64_t ldz, gnm_stream_t stream);
 
 /* ---- data parallel: synchronised BatchNorm sums over NVLink peer memory ------------------------------
  * The reference is single-process; a global-batch BatchNorm needs the per-channel sums of all ranks before the next

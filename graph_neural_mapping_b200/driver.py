@@ -402,17 +402,28 @@ def saliency_maps(model, graphs, cls, batch=64):
     return out.get("a", np.zeros((0, 0, 0), dtype=np.float32))
 
 
+def _attribution_chunks(model, graphs, classes, batch, compute, with_delta=False):
+    """compute(chunk) on `graphs` in chunks of `batch` graphs, one D2H copy per chunk: float32 [G, len(classes), D] from
+    its [n, len(classes), D] device results, and with_delta also [G, len(classes)] from a second result."""
+    c, d = len(classes), int(_engine.layer_units(model, 0)[0][0].weight.shape[1])          # d: input_dim
+    width = c * d + (c if with_delta else 0)
+    host = np.empty((len(graphs), width), dtype=np.float32)
+    for i in range(0, len(graphs), batch):
+        chunk = graphs[i:i + batch]
+        res = compute(chunk)
+        flat = torch.cat([res[0].reshape(len(chunk), c * d), res[1]], 1) if with_delta else res.reshape(len(chunk), width)
+        host[i:i + len(chunk)] = flat.cpu().numpy()                    # one copy for both results
+    out = np.ascontiguousarray(host[:, :c * d]).reshape(len(graphs), c, d)
+    return (out, np.ascontiguousarray(host[:, c * d:])) if with_delta else out
+
+
 def roi_saliency(model, graphs, classes=(0, 1), batch=1024):
     """ROI saliency: float32 [G, len(classes), D], entry [i, k] = the node average of `compute_saliency([graphs[i]],
     classes[k])` - what evaluate/plot_saliency_nii.py reduces each map to - computed by
     `compute_roi_saliency_batched` in batches of `batch` graphs (one forward per batch for all classes, one D2H copy
     per batch; 1.6 KB per graph and class instead of a 640 KB map at N = D = 400). Graphs may differ in size."""
-    d = int(_engine.layer_units(model, 0)[0][0].weight.shape[1])          # input_dim
-    out = np.empty((len(graphs), len(classes), d), dtype=np.float32)
-    for i in range(0, len(graphs), batch):
-        chunk = graphs[i:i + batch]
-        out[i:i + len(chunk)] = model.compute_roi_saliency_batched(chunk, classes).cpu().numpy()
-    return out
+    return _attribution_chunks(model, graphs, classes, batch,
+                               lambda chunk: model.compute_roi_saliency_batched(chunk, classes))
 
 
 def integrated_gradients(model, graphs, classes=(0, 1), steps=50, batch=1024, return_delta=False):
@@ -421,20 +432,8 @@ def integrated_gradients(model, graphs, classes=(0, 1), steps=50, batch=1024, re
     same node average as `roi_saliency`), and with return_delta the [G, len(classes)] completeness gap. Computed in
     calls of `batch` graphs, one D2H copy per call. Graphs may differ in size; node features must be one-hot and the
     neighbour pooling sum or average."""
-    d = int(_engine.layer_units(model, 0)[0][0].weight.shape[1])          # input_dim
-    out = np.empty((len(graphs), len(classes), d), dtype=np.float32)
-    delta = np.empty((len(graphs), len(classes)), dtype=np.float32)
-    per = len(classes) * d
-    for i in range(0, len(graphs), batch):
-        chunk = graphs[i:i + batch]
-        n = len(chunk)
-        res = model.compute_integrated_gradients_batched(chunk, classes, steps=steps, return_delta=return_delta)
-        flat = torch.cat([res[0].reshape(n, per), res[1]], 1) if return_delta else res.reshape(n, per)
-        host = flat.cpu().numpy()                                          # one copy for both results
-        out[i:i + n] = host[:, :per].reshape(n, len(classes), d)
-        if return_delta:
-            delta[i:i + n] = host[:, per:]
-    return (out, delta) if return_delta else out
+    return _attribution_chunks(model, graphs, classes, batch, lambda chunk: model.compute_integrated_gradients_batched(
+        chunk, classes, steps=steps, return_delta=return_delta), return_delta)
 
 
 def roi_occlusion(model, graphs, classes=(0, 1), batch=1024):
@@ -442,12 +441,8 @@ def roi_occlusion(model, graphs, classes=(0, 1), batch=1024):
     set to 0)) / n_i for c = classes[k] (`compute_roi_occlusion_batched`, the node-average convention of `roi_saliency`
     and `integrated_gradients`). Computed in calls of `batch` graphs, one D2H copy per call. Graphs may differ in size;
     node features must be one-hot, and under max neighbour pooling tags injective and edge lists duplicate-free."""
-    d = int(_engine.layer_units(model, 0)[0][0].weight.shape[1])          # input_dim
-    out = np.empty((len(graphs), len(classes), d), dtype=np.float32)
-    for i in range(0, len(graphs), batch):
-        chunk = graphs[i:i + batch]
-        out[i:i + len(chunk)] = model.compute_roi_occlusion_batched(chunk, classes).cpu().numpy()
-    return out
+    return _attribution_chunks(model, graphs, classes, batch,
+                               lambda chunk: model.compute_roi_occlusion_batched(chunk, classes))
 
 
 def saliency_maps_to_npy(model, graphs, cls, path, batch=64):

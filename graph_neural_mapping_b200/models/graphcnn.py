@@ -208,6 +208,81 @@ class GIN_InfoMaxReg(nn.Module):
                 row += 1
         return torch.from_numpy(padded), torch.from_numpy(first)
 
+    def _max_neighbours(self, batch_graph):
+        """Under max neighbour pooling, _padded_neighbours on the device: input gradients follow the reference's tie rule
+        (the first entry of the padded list). (None, None) under the other poolings."""
+        if self.neighbor_pooling_type != "max":
+            return None, None
+        padded, first = self._padded_neighbours(batch_graph)
+        return padded.to(self.eps.device), first.to(self.eps.device)
+
+    def _attribution_args(self, batch_graph, classes, what=None, counts=None, linear=False, occlusion=False):
+        """The attribution methods' argument checks, in this order: eval() and `classes`; each of `counts` (name -> value)
+        >= 1; no max neighbour pooling for a `linear` method; unless `what` is None (ROI saliency), BatchNorm running
+        statistics and, for a non-empty batch and class list, one-hot features; for `occlusion` under max pooling a
+        layer-0 max equal to its sum and no node without neighbours. `what` starts the messages. Returns (classes, counts
+        as ints, out: float32 [B, len(classes), D] uninitialised, the host batch or None if there is nothing to compute)."""
+        self.eval()
+        classes = [int(c) for c in classes]
+        n_cls = self.linears_prediction[0].weight.shape[0]
+        if any(c < 0 or c >= n_cls for c in classes):
+            raise ValueError("classes must lie in [0, %d), got %s" % (n_cls, classes))
+        counts = {k: int(v) for k, v in (counts or {}).items()}
+        if any(v < 1 for v in counts.values()):
+            raise ValueError("%s must be >= 1, got %s" % (" and ".join(counts), " and ".join(map(str, counts.values()))))
+        max_pool = self.neighbor_pooling_type == "max"
+        if linear and max_pool:
+            raise ValueError("%s sum or average neighbour pooling: max pooling is not linear in the input (use "
+                             "compute_saliency_batched for its input gradient)" % what)
+        if what is not None and not all(bn.track_running_stats for layer in range(self.num_layers)
+                                        for _, bn in _engine.layer_units(self, layer)):
+            raise ValueError("%s BatchNorm running statistics (eval mode per graph)" % what)
+        d_in = _engine.layer_units(self, 0)[0][0].weight.shape[1]
+        out = torch.empty(len(batch_graph), len(classes), d_in, dtype=torch.float32, device=self.eps.device)
+        if len(batch_graph) == 0 or not classes:
+            return classes, list(counts.values()), out, None
+        h = self._host_batch(batch_graph)
+        if what is not None and not h.onehot:
+            raise ValueError("%s one-hot node features (util.py:114-116)" % what)
+        if occlusion and max_pool and not h.max0_as_sum:
+            raise ValueError("ROI occlusion under max neighbour pooling needs injective node tags and duplicate-free edge "
+                             "lists in every graph (layer 0's max then equals its sum)")
+        if occlusion and max_pool and h.has_isolated:
+            raise ValueError("ROI occlusion under max neighbour pooling needs graphs without nodes without neighbours: "
+                             "such a node pools the column minimum of the whole forward batch (graphcnn.py:137-143), so "
+                             "its graph's occluded score would depend on the other copies in the pass")
+        return classes, list(counts.values()), out, h
+
+    def _layer0_base(self, rbs, params):
+        """Layer 0 without its bias on the real batch `rbs` (one-hot): P = Agg(X) W1^T, from which a virtual batch's
+        layer-0 output is written (engine.run_forward's z0). Returns (P, W1^T contiguous, eps or None, aggregation
+        mode: 1 under average neighbour pooling, else 0)."""
+        lin0 = _engine.layer_units(self, 0)[0][0]
+        w1t = lin0.weight.detach().t().contiguous()
+        mode = 1 if self.neighbor_pooling_type == "average" else 0
+        eps_l = params[0][0:1] if self.learn_eps else None
+        p0 = torch.empty(rbs.n_rows, lin0.weight.shape[0], dtype=torch.float32, device=self.eps.device)
+        rbs.aggregate(w1t, rbs.tags, p0, mode, eps_l, None)
+        return p0, w1t, eps_l, mode
+
+    def _head_rows(self, classes):
+        """d score_c / d g_f for each c in classes: the class-c rows of the prediction heads (graphcnn.py:228-231 in eval,
+        no dropout)."""
+        heads = [lin.weight.detach() for lin in self.linears_prediction]
+        return [torch.cat([w[c] for w in heads]) for c in classes]
+
+    def _virtual_forward(self, graphs, fill, params):
+        """Eval forward of a virtual batch: `graphs` repeats graph objects of a real batch (the graph store resolves them
+        to the same slots) and fill(vbs, bias, z) writes its layer-0 output. Returns (g_f, saved state)."""
+        vbs = self._structure(graphs)
+        g_f, _, sv = _engine.run_forward(self, vbs, None, False, False, None, params, _dist.SINGLE,
+                                         z0=lambda bias, z: fill(vbs, bias, z))
+        return g_f, sv
+
+    def _class_scores(self, g_f, classes):
+        """The eval class scores [V, len(classes)] of a virtual batch's g_f (no dropout in eval)."""
+        return self._heads(g_f)[:, classes]
+
     def _heads(self, g_f):
         """graphcnn.py:228-231: sum over layers of dropout(Linear(pooled_h)). On the GPU: one libgnm launch forward, one
         backward (_HeadsFunction) instead of ~15 + ~25 small torch kernels whose launch latency sat on the critical path
@@ -270,11 +345,7 @@ class GIN_InfoMaxReg(nn.Module):
         self.zero_grad()
         bs = self._structure(batch_graph)
         runner = _engine.Runner(self, bs, None, False, False, _dist.SINGLE, want_x_grad=True)
-        if self.neighbor_pooling_type == "max":
-            # input gradients under max pooling follow the reference's tie rule (first entry of the padded list)
-            padded, first = self._padded_neighbours(batch_graph)
-            runner.max_padded = padded.to(self.eps.device)
-            runner.max_first = first.to(self.eps.device)
+        runner.max_padded, runner.max_first = self._max_neighbours(batch_graph)
         x = self._dense_features(batch_graph, bs)
         if x is not None:
             x.requires_grad_()
@@ -293,30 +364,17 @@ class GIN_InfoMaxReg(nn.Module):
         gradient per graph instead of forming the map (engine.run_backward's ROI mode). Graphs may differ in size:
         each mean is over that graph's own nodes. Puts the model in eval() like compute_saliency but, unlike it, leaves
         every parameter's .grad untouched (no autograd pass runs)."""
-        self.eval()
-        classes = [int(c) for c in classes]
-        n_cls = self.linears_prediction[0].weight.shape[0]
-        if any(c < 0 or c >= n_cls for c in classes):
-            raise ValueError("classes must lie in [0, %d), got %s" % (n_cls, classes))
-        dev = self.eps.device
-        d_in = _engine.layer_units(self, 0)[0][0].weight.shape[1]
-        b = len(batch_graph)
-        out = torch.empty(b, len(classes), d_in, dtype=torch.float32, device=dev)
-        if b == 0 or not classes:
+        classes, _, out, h = self._attribution_args(batch_graph, classes)
+        if h is None:
             return out
-        bs = self._structure(batch_graph)
-        max_padded = max_first = None
-        if self.neighbor_pooling_type == "max":
-            padded, first = self._padded_neighbours(batch_graph)
-            max_padded, max_first = padded.to(dev), first.to(dev)
+        bs = self._structure(batch_graph, h)
+        max_padded, max_first = self._max_neighbours(batch_graph)
         x = self._dense_features(batch_graph, bs)
         params = [p.detach() for p in _engine.flat_params(self)]
         with torch.no_grad():
             _, _, sv = _engine.run_forward(self, bs, None, False, False, x, params, _dist.SINGLE, max_padded=max_padded)
-            heads = [lin.weight.detach() for lin in self.linears_prediction]
-            for k, c in enumerate(classes):
-                # d score_c / d g_f: the class-c rows of the prediction heads (graphcnn.py:228-231 in eval, no dropout)
-                dg_f = torch.cat([w[c] for w in heads]).expand(b, -1).contiguous()
+            for k, row in enumerate(self._head_rows(classes)):
+                dg_f = row.expand(len(batch_graph), -1).contiguous()
                 _engine.run_backward(self, sv, params, dg_f, None, False, _dist.SINGLE, max_first=max_first, roi=out[:, k])
         return out
 
@@ -339,39 +397,17 @@ class GIN_InfoMaxReg(nn.Module):
         Needs one-hot node features (util.py:114-116) and sum or average neighbour pooling: max pooling is not linear in
         the input, and its input gradient takes the [N, D] tie-rule route (compute_saliency_batched). ValueError
         otherwise, and for classes out of range or steps < 1."""
-        self.eval()
-        classes = [int(c) for c in classes]
-        n_cls = self.linears_prediction[0].weight.shape[0]
-        if any(c < 0 or c >= n_cls for c in classes):
-            raise ValueError("classes must lie in [0, %d), got %s" % (n_cls, classes))
-        steps, points_per_pass = int(steps), int(points_per_pass)
-        if steps < 1 or points_per_pass < 1:
-            raise ValueError("steps and points_per_pass must be >= 1, got %d and %d" % (steps, points_per_pass))
-        if self.neighbor_pooling_type == "max":
-            raise ValueError("integrated gradients need sum or average neighbour pooling: max pooling is not linear in "
-                             "the input (use compute_saliency_batched for its input gradient)")
-        if not all(bn.track_running_stats for layer in range(self.num_layers)
-                   for _, bn in _engine.layer_units(self, layer)):
-            raise ValueError("integrated gradients need BatchNorm running statistics (eval mode per graph)")
+        classes, (steps, points_per_pass), out, h = self._attribution_args(
+            batch_graph, classes, "integrated gradients need", dict(steps=steps, points_per_pass=points_per_pass),
+            linear=True)
         dev = self.eps.device
-        lin0 = _engine.layer_units(self, 0)[0][0]
-        d_in, f0 = lin0.weight.shape[1], lin0.weight.shape[0]
         b, n_c = len(batch_graph), len(classes)
-        out = torch.empty(b, n_c, d_in, dtype=torch.float32, device=dev)
         delta = torch.empty(b, n_c, dtype=torch.float32, device=dev) if return_delta else None
-        if b > 0 and n_c > 0:
-            h = self._host_batch(batch_graph)
-            if not h.onehot:
-                raise ValueError("integrated gradients need one-hot node features (util.py:114-116)")
         res = (out, delta) if return_delta else out
-        if b == 0 or n_c == 0:
+        if h is None:
             return res
         params = [p.detach() for p in _engine.flat_params(self)]
-        average = self.neighbor_pooling_type == "average"
-        eps_l = params[0][0:1] if self.learn_eps else None
-        w1t = lin0.weight.detach().t().contiguous()
-        heads = [lin.weight.detach() for lin in self.linears_prediction]
-        dg_rows = [torch.cat([w[c] for w in heads]) for c in classes]     # d score_c / d g_f (graphcnn.py:228-231)
+        dg_rows = self._head_rows(classes)
         alphas = ((torch.arange(steps, dtype=torch.float64) + 0.5) / steps).to(dev, torch.float32)
         per_chunk = max(1, points_per_pass // steps)
         points = min(steps, points_per_pass)
@@ -379,31 +415,27 @@ class GIN_InfoMaxReg(nn.Module):
             for i in range(0, b, per_chunk):
                 chunk = batch_graph[i:i + per_chunk]
                 rbs = self._structure(chunk)
-                # layer 0 without its bias on the real graphs: z0(alpha) = alpha * p0 + b
-                p0 = torch.empty(rbs.n_rows, f0, dtype=torch.float32, device=dev)
-                rbs.aggregate(w1t, rbs.tags, p0, 1 if average else 0, eps_l, None)
-                acc = torch.empty(n_c, rbs.n_rows, f0, dtype=torch.float32, device=dev)
+                p0, w1t, eps_l, mode = self._layer0_base(rbs, params)          # z0(alpha) = alpha * p0 + b
+                acc = torch.empty(n_c, rbs.n_rows, p0.shape[1], dtype=torch.float32, device=dev)
                 for s0 in range(0, steps, points):
                     k = min(points, steps - s0)
-                    vbs = self._structure([g for g in chunk for _ in range(k)])
-                    fill = lambda bias, z: _ops.ig_expand(p0, bias, alphas[s0:s0 + k], rbs.node_off, k, z)
-                    _, _, sv = _engine.run_forward(self, vbs, None, False, False, None, params, _dist.SINGLE, z0=fill)
+                    fill = lambda vbs, bias, z: _ops.ig_expand(p0, bias, alphas[s0:s0 + k], rbs.node_off, k, z)
+                    _, sv = self._virtual_forward([g for g in chunk for _ in range(k)], fill, params)
                     for j in range(n_c):
-                        dg_f = dg_rows[j].expand(vbs.n_graphs, -1).contiguous()
+                        dg_f = dg_rows[j].expand(len(chunk) * k, -1).contiguous()
                         _engine.run_backward(self, sv, params, dg_f, None, False, _dist.SINGLE,
                                              ig=(acc[j], rbs.node_off, k, 1.0 / steps, s0 > 0))
                 for j in range(n_c):
                     # IG = X o ((Agg^T acc) W1): per node the row dot with its tag's W1 column, averaged per ROI
-                    t = torch.empty(rbs.n_rows, f0, dtype=torch.float32, device=dev)
-                    rbs.aggregate(acc[j], None, t, 2 if average else 0, eps_l, None)
+                    t = torch.empty_like(p0)
+                    rbs.aggregate(acc[j], None, t, 2 if mode == 1 else 0, eps_l, None)
                     _ops.ig_attribute(t, w1t, rbs.tags, rbs.node_off, out[i:i + len(chunk), j])
                 if return_delta:
                     # F_c(X) - F_c(0): a forward-only virtual batch of the two endpoints
                     ends = torch.tensor([1.0, 0.0], dtype=torch.float32, device=dev)
-                    vbs = self._structure([g for g in chunk for _ in range(2)])
-                    fill = lambda bias, z: _ops.ig_expand(p0, bias, ends, rbs.node_off, 2, z)
-                    g_f, _, _ = _engine.run_forward(self, vbs, None, False, False, None, params, _dist.SINGLE, z0=fill)
-                    score = self._heads(g_f).view(len(chunk), 2, n_cls)[:, :, classes]
+                    fill = lambda vbs, bias, z: _ops.ig_expand(p0, bias, ends, rbs.node_off, 2, z)
+                    g_f, _ = self._virtual_forward([g for g in chunk for _ in range(2)], fill, params)
+                    score = self._class_scores(g_f, classes).view(len(chunk), 2, n_c)
                     n_g = torch.from_numpy(rbs.node_counts.astype(np.float32)).to(dev).unsqueeze(1)
                     delta[i:i + len(chunk)] = n_g * out[i:i + len(chunk)].sum(2) - (score[:, 0] - score[:, 1])
         return res
@@ -430,46 +462,19 @@ class GIN_InfoMaxReg(nn.Module):
         neighbours (learn_eps: no self loop; max pooling gives such a node the column minimum of the whole forward batch,
         graphcnn.py:137-143, so a graph's score would depend on its companions). ValueError otherwise, and for classes
         out of range or occlusions_per_pass < 1."""
-        self.eval()
-        classes = [int(c) for c in classes]
-        n_cls = self.linears_prediction[0].weight.shape[0]
-        if any(c < 0 or c >= n_cls for c in classes):
-            raise ValueError("classes must lie in [0, %d), got %s" % (n_cls, classes))
-        occlusions_per_pass = int(occlusions_per_pass)
-        if occlusions_per_pass < 1:
-            raise ValueError("occlusions_per_pass must be >= 1, got %d" % occlusions_per_pass)
-        if not all(bn.track_running_stats for layer in range(self.num_layers)
-                   for _, bn in _engine.layer_units(self, layer)):
-            raise ValueError("ROI occlusion needs BatchNorm running statistics (eval mode per graph)")
-        dev = self.eps.device
-        lin0 = _engine.layer_units(self, 0)[0][0]
-        d_in, f0 = lin0.weight.shape[1], lin0.weight.shape[0]
-        b, n_c = len(batch_graph), len(classes)
-        out = torch.zeros(b, n_c, d_in, dtype=torch.float32, device=dev)
-        if b == 0 or n_c == 0:
+        classes, (occlusions_per_pass,), out, h = self._attribution_args(
+            batch_graph, classes, "ROI occlusion needs", dict(occlusions_per_pass=occlusions_per_pass), occlusion=True)
+        if h is None:
             return out
-        h = self._host_batch(batch_graph)
-        if not h.onehot:
-            raise ValueError("ROI occlusion needs one-hot node features (util.py:114-116)")
-        if self.neighbor_pooling_type == "max" and not h.max0_as_sum:
-            raise ValueError("ROI occlusion under max neighbour pooling needs injective node tags and duplicate-free edge "
-                             "lists in every graph (layer 0's max then equals its sum)")
-        if self.neighbor_pooling_type == "max" and h.has_isolated:
-            raise ValueError("ROI occlusion under max neighbour pooling needs graphs without nodes without neighbours: "
-                             "such a node pools the column minimum of the whole forward batch (graphcnn.py:137-143), so "
-                             "its graph's occluded score would depend on the other copies in the pass")
+        out.zero_()                                                        # absent tags stay exactly 0
+        dev = self.eps.device
         params = [p.detach() for p in _engine.flat_params(self)]
-        mode = 1 if self.neighbor_pooling_type == "average" else 0
-        eps_l = params[0][0:1] if self.learn_eps else None
-        w1t = lin0.weight.detach().t().contiguous()
         cls_d = torch.tensor(classes, dtype=torch.int64, device=dev)
         inv_n = torch.from_numpy(1.0 / np.maximum(h.counts, 1)).to(dev, torch.float32)
-        bad = torch.zeros(b, n_c, dtype=torch.bool, device=dev)
+        bad = torch.zeros(len(batch_graph), len(classes), dtype=torch.bool, device=dev)
         with torch.no_grad():
             rbs = self._structure(batch_graph, h)
-            # layer 0 without its bias on the real graphs: an occluded copy's z0 is p0 + b minus a rank-1 term
-            p0 = torch.empty(rbs.n_rows, f0, dtype=torch.float32, device=dev)
-            rbs.aggregate(w1t, rbs.tags, p0, mode, eps_l, None)
+            p0, w1t, eps_l, mode = self._layer0_base(rbs, params)          # a copy's z0: p0 + b minus a rank-1 term
             for v_graph, v_tag in occlusion_passes(h.node_off, rbs.tags.cpu().numpy(), occlusions_per_pass):
                 v = len(v_graph)
                 pos = np.arange(v, dtype=np.int32)
@@ -481,12 +486,11 @@ class GIN_InfoMaxReg(nn.Module):
                 n_k = len(copies)
                 copy_d, base_d, bl_d = (t.long() for t in (idx[2 * v:2 * v + n_k], idx[2 * v + n_k:2 * v + 2 * n_k],
                                                            idx[2 * v + 2 * n_k:]))
-                vbs = self._structure([batch_graph[g] for g in v_graph.tolist()])
-                fill = lambda bias, z: _ops.occlusion_expand(p0, bias, w1t, rbs.rowptr, rbs.colidx, rbs.tags,
-                                                             rbs.node_off, rbs.n_max, vg_d, vt_d, vbs.node_off, mode,
-                                                             eps_l, z)
-                g_f, _, _ = _engine.run_forward(self, vbs, None, False, False, None, params, _dist.SINGLE, z0=fill)
-                score = self._heads(g_f).index_select(1, cls_d)                       # [V, C], eval: no dropout
+                fill = lambda vbs, bias, z: _ops.occlusion_expand(p0, bias, w1t, rbs.rowptr, rbs.colidx, rbs.tags,
+                                                                  rbs.node_off, rbs.n_max, vg_d, vt_d, vbs.node_off,
+                                                                  mode, eps_l, z)
+                g_f, _ = self._virtual_forward([batch_graph[g] for g in v_graph.tolist()], fill, params)
+                score = self._class_scores(g_f, cls_d)                                # [V, C]
                 g_k, d_k = vg_d[copy_d].long(), vt_d[copy_d].long()
                 out[g_k, :, d_k] = (score[base_d] - score[copy_d]) * inv_n[g_k].unsqueeze(1)
                 g_b = vg_d[bl_d].long()

@@ -427,3 +427,95 @@ def dgi_neg_grad(neg_idx, s2, u, d_neg):
 
 def aggregate_dense_table(bitmap_addr, node_off, rowptr, n_graphs, n_max, table, tags, dst, mode, eps, bias, out_stats, tail=None):
     return False          # the stand-in has no shared-table kernel: the engine falls back to aggregate + col_stats
+
+
+# ---- attribution (contracts of gnm_segment.cu, gnm_ig.cu, gnm_occlusion.cu) --------------------
+
+def segment_weighted_colsum(x, node_off, out, z=None, coef=None, rowptr=None, mode=0, eps=None):
+    """gnm_segment_weighted_colsum: out[g] = (1/n_g) sum_{m in g} w_m v[m], v = x or cA x + cB z + cC, w_m the row sums
+    of the aggregation operator (deg, or 1 / 0 for an isolated node under average, + 1 + eps), zeros for an empty graph."""
+    v = x.double()
+    if coef is not None:
+        v = coef[0].double() * v
+        if z is not None:
+            v = v + coef[1].double() * z.double() + coef[2].double()
+    m = x.shape[0]
+    if rowptr is None:
+        w = torch.ones(m, dtype=torch.float64)
+    else:
+        deg = (rowptr[1:] - rowptr[:-1]).double()
+        w = (deg > 0).double() if mode == 1 else deg
+        if eps is not None:
+            w = w + 1.0 + eps.double()
+    no = node_off.long()
+    gid = torch.repeat_interleave(torch.arange(no.numel() - 1), no[1:] - no[:-1])
+    s = torch.zeros(out.shape[0], x.shape[1], dtype=torch.float64).index_add_(0, gid, w.unsqueeze(1) * v)
+    n = (no[1:] - no[:-1]).double().clamp(min=1).unsqueeze(1)
+    out.copy_((s / n).float())
+    return out
+
+
+def ig_expand(p, bias, alpha, node_off, points, z):
+    """gnm_ig_expand: z[(g, s, i)] = alpha[s] * p[node_off[g] + i] + bias, graph-major virtual rows."""
+    no = node_off.long().tolist()
+    rows = []
+    for g in range(len(no) - 1):
+        for s in range(points):
+            v = float(alpha[s]) * p[no[g]:no[g + 1]].double()
+            rows.append(v + bias.double() if bias is not None else v)
+    if rows:
+        z.copy_(torch.cat(rows).float())
+    return z
+
+
+def ig_accumulate(dy, coef, node_off, points, weight, out, accumulate):
+    """gnm_ig_accumulate: out[r] (+)= weight * cA o sum_s dy[(g, s, r - node_off[g])]."""
+    no = node_off.long().tolist()
+    ca = coef[0].double() if coef is not None else 1.0
+    for g in range(len(no) - 1):
+        n = no[g + 1] - no[g]
+        base = points * no[g]
+        v = weight * ca * dy[base:base + points * n].double().view(points, n, -1).sum(0)
+        if accumulate:
+            v = v + out[no[g]:no[g + 1]].double()
+        out[no[g]:no[g + 1]] = v.float()
+    return out
+
+
+def ig_attribute(t, table, tags, node_off, out):
+    """gnm_ig_attribute: out[g, d] = (1/n_g) sum_{n in g, tags[n] = d} <t[n], table[d]>; NaN row for non-finite t."""
+    a = (t.double() * table.double()[tags.long()]).sum(1)
+    no = node_off.long().tolist()
+    for g in range(len(no) - 1):
+        r0, r1 = no[g], no[g + 1]
+        row = torch.zeros(out.shape[1], dtype=torch.float64).index_add_(0, tags[r0:r1].long(), a[r0:r1])
+        row = row / max(r1 - r0, 1)
+        if not bool(torch.isfinite(t[r0:r1]).all()):
+            row[:] = float("nan")
+        out[g] = row.float()
+    return out
+
+
+def occlusion_expand(p, bias, w1t, rowptr, colidx, tags, node_off, n_max, v_graph, v_tag, v_node_off, mode, eps, z):
+    """gnm_occlusion_expand: z[v_node_off[v] + i] = p[m] + bias - c_d[m] w1t[d], c_d[m] = s_m #{n in CSR row m:
+    tags[n] = d} + (eps ? (1 + eps) [tags[m] = d] : 0), s_m = 1 (mode 0) or 1 / (row length) (mode 1)."""
+    m_all = p.shape[0]
+    rp, ci, tg = rowptr.long(), colidx.long(), tags.long()
+    rows = torch.repeat_interleave(torch.arange(m_all), rp[1:] - rp[:-1])
+    counts = torch.zeros(m_all, w1t.shape[0], dtype=torch.float64)
+    counts.index_put_((rows, tg[ci]), torch.ones(ci.numel(), dtype=torch.float64), accumulate=True)
+    deg = (rp[1:] - rp[:-1]).double()
+    no, vno = node_off.long().tolist(), v_node_off.long().tolist()
+    base = p.double() + (bias.double() if bias is not None else 0.0)
+    for v in range(v_graph.shape[0]):
+        g, d = int(v_graph[v]), int(v_tag[v])
+        r0, r1 = no[g], no[g + 1]
+        val = base[r0:r1].clone()
+        if 0 <= d < w1t.shape[0]:
+            c = counts[r0:r1, d]
+            coef = torch.where(c != 0, c / deg[r0:r1] if mode == 1 else c, torch.zeros_like(c))
+            if eps is not None:
+                coef = coef + (1.0 + float(eps[0])) * (tg[r0:r1] == d).double()
+            val = val - coef.unsqueeze(1) * w1t[d].double()
+        z[vno[v]:vno[v] + r1 - r0] = val.float()
+    return z

@@ -1,4 +1,4 @@
-"""Shared test helpers: golden-fixture loading and tolerance checks."""
+"""Shared test helpers: golden-fixture loading, tolerance checks and the CPU stand-in's installation."""
 import glob
 import json
 import os
@@ -7,6 +7,11 @@ import re
 import numpy as np
 import torch
 
+import emul_ops
+from graph_neural_mapping_b200 import engine
+from graph_neural_mapping_b200.models import discriminator as dmod
+from graph_neural_mapping_b200.models import graphcnn as gmod
+from graph_neural_mapping_b200.models import mlp as mlpmod
 from graph_neural_mapping_b200.synth import SynthGraph
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -60,6 +65,23 @@ class Golden(object):
         for k, v in self.group("buf_after/").items():
             sd[k] = torch.from_numpy(v.copy())
         return sd
+
+
+def use_cpu_stand_in(monkeypatch):
+    """Route every kernel call of the model code to the CPU stand-in (tests/emul_ops.py) for the current test."""
+    for mod in (engine, gmod, mlpmod, dmod):
+        monkeypatch.setattr(mod, "_ops", emul_ops)
+    monkeypatch.setattr(engine, "require_cuda", lambda dev: None)
+
+
+def build_model(g, sd=None):
+    """The golden fixture's model on the CPU, with its initial state or `sd`."""
+    c = g.cfg
+    m = gmod.GIN_InfoMaxReg(c["num_layers"], c["num_mlp_layers"], c["input_dim"], c["hidden_dim"], c["output_dim"],
+                            c["final_dropout"], c["learn_eps"], c["graph_pooling_type"], c["neighbor_pooling_type"],
+                            torch.device("cpu"))
+    m.load_state_dict(sd if sd is not None else g.state_dict())
+    return m
 
 
 def rel_err(a, b):

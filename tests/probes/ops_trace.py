@@ -1,6 +1,6 @@
 """Call trace of the kernel entry points the engine reaches; a refactor of the host orchestration must leave it as it is.
 
-The ops module seen by engine, mlp, discriminator and driver is replaced by a shim that passes every attribute through
+The ops module seen by engine, graphcnn, mlp, discriminator and driver is replaced by a shim that passes every attribute through
 and records each call of a public function: its name, every argument bound to the callee's signature (defaults filled
 in, so a positional and a keyword spelling of one call record alike) and any boolean return. A tensor is recorded as
 shape, dtype, strides and storage offset (which places the views of engine._ZeroPool's buffers), None as None, a
@@ -8,15 +8,18 @@ scalar as its value, an ops.BnTail as its kind and count; no pointer value is re
 digest of the trace and one of the case's outputs (parameter gradients, saliency maps, ROI averages) as raw bytes;
 `--dump DIR` also writes each full trace, one call per line, to diff.
 
-  cpu: the CPU stand-in kernels (tests/emul_ops.py and the segment_weighted_colsum stand-in of
-       tests/test_roi_saliency_cpu.py). Every golden fixture with N < 400 through a training step, compute_saliency,
-       compute_saliency_batched and compute_roi_saliency_batched((0, 1)); the same under FORCE_CSR_AGGREGATE and under
-       FORCE_UNFUSED_BACKWARD; a batch whose node features are not exactly one-hot. Deterministic: both digests are
-       compared bit for bit.
+  cpu: the CPU stand-in kernels (tests/emul_ops.py). Every golden fixture with N < 400 through a training step,
+       compute_saliency, compute_saliency_batched and compute_roi_saliency_batched((0, 1)); the same under
+       FORCE_CSR_AGGREGATE and under FORCE_UNFUSED_BACKWARD; a batch whose node features are not exactly one-hot; and
+       every such fixture through compute_integrated_gradients_batched with return_delta (a points_per_pass that splits
+       a graph's points over two passes, and one that packs several graphs per pass) and compute_roi_occlusion_batched at
+       two occlusions_per_pass that split differently. A call that raises ValueError records its message. Deterministic:
+       both digests are compared bit for bit.
   gpu: the libgnm kernels. Trainer steps (fused and not, the eager warm-up steps), model(graphs) + backward at
-       1024 x 400, learn_eps, average pooling with an isolated node, max pooling, hidden width 128 and ROI saliency
-       (one-hot, dense, max pooling). CUDA graphs are off, so every call is eager and recorded. Only the trace digests
-       are meant to match across builds: the kernels' float atomics make outputs differ in the last bits.
+       1024 x 400, learn_eps, average pooling with an isolated node, max pooling, hidden width 128, ROI saliency
+       (one-hot, dense, max pooling) and the integrated-gradients and occlusion calls of the cpu mode on the same models.
+       CUDA graphs are off, so every call is eager and recorded. Only the trace digests are meant to match across
+       builds: the kernels' float atomics make outputs differ in the last bits.
 
     python tests/probes/ops_trace.py cpu|gpu [--dump DIR]"""
 import argparse
@@ -34,9 +37,10 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 from graph_neural_mapping_b200 import driver, engine, synth  # noqa: E402
 from graph_neural_mapping_b200.models import GIN_InfoMaxReg  # noqa: E402
 from graph_neural_mapping_b200.models import discriminator as dmod  # noqa: E402
+from graph_neural_mapping_b200.models import graphcnn as gmod  # noqa: E402
 from graph_neural_mapping_b200.models import mlp as mlpmod  # noqa: E402
 
-USERS = (engine, mlpmod, dmod, driver)
+USERS = (engine, gmod, mlpmod, dmod, driver)
 
 
 def _sig(v):
@@ -147,11 +151,33 @@ def run_model_cases(case, model, graphs, beta, seed, roi_per_graph=False):
         case.add(model.compute_roi_saliency_batched(graphs[:2], (0, 1)))
 
 
+def _attempt(case, fn):
+    try:
+        res = fn()
+    except ValueError as e:
+        case.outputs.update(str(e).encode())
+        return
+    for t in (res if isinstance(res, tuple) else (res,)):
+        case.add(t)
+
+
+def run_attribution_cases(shim, name, model, graphs, steps, points_per_pass, occlusions_per_pass, dump):
+    """Integrated gradients with the completeness gap at each points_per_pass, then ROI occlusion at each
+    occlusions_per_pass, both for classes (0, 1): one case each, outputs hashed."""
+    with Case(shim) as case:
+        for p in points_per_pass:
+            _attempt(case, lambda: model.compute_integrated_gradients_batched(graphs, (0, 1), steps=steps,
+                                                                              points_per_pass=p, return_delta=True))
+    report(name + ".ig", case, dump)
+    with Case(shim) as case:
+        for o in occlusions_per_pass:
+            _attempt(case, lambda: model.compute_roi_occlusion_batched(graphs, (0, 1), occlusions_per_pass=o))
+    report(name + ".occlusion", case, dump)
+
+
 def cpu_cases(dump):
     import emul_ops
-    from helpers import Golden, SEED0, golden_names
-    from test_roi_saliency_cpu import build_model, segment_weighted_colsum
-    emul_ops.segment_weighted_colsum = segment_weighted_colsum
+    from helpers import Golden, SEED0, build_model, golden_names
     shim = TracingOps(emul_ops)
     for m in USERS:
         m._ops = shim
@@ -179,6 +205,11 @@ def cpu_cases(dump):
     with Case(shim) as case:
         run_model_cases(case, build_model(g), graphs, g.cfg["beta"], 7)
     report("tiny_eps_sum.dense_input", case, dump)
+    # 6 points: 4 per pass splits each graph's points 4 + 2, 13 per pass packs two graphs; 7 copies per pass split every
+    # graph's tags over several passes, 40 pack two small graphs or split one of 48 tags in two
+    for name in names:
+        g = Golden(name)
+        run_attribution_cases(shim, name, build_model(g, g.state_after_train()), g.graphs(), 6, (4, 13), (7, 40), dump)
 
 
 def gpu_cases(dump):
@@ -224,6 +255,10 @@ def gpu_cases(dump):
     model = model_of(5, 400, 64, seed=2)
     train_case("model.1024x400", model, big)
     saliency_case("saliency.onehot.1024x400", model, big)
+    # 8 points: 5 per pass splits each graph's points 5 + 3, 20 per pass packs two graphs; at 400 tags 300 copies per
+    # pass split a graph's tags in two, 1024 pack two graphs
+    attribution = dict(steps=8, points_per_pass=(5, 20), occlusions_per_pass=(300, 1024), dump=dump)
+    run_attribution_cases(shim, "attribution.1024x400", model, big[:16], **attribution)
     dense = [synth.SynthGraph(400, g.label, g.edge_mat, g.node_features.clone()) for g in big[:64]]
     for gr in dense:
         gr.node_features[0, 0] = 0.5                          # not exactly one-hot: the dense layer-0 path
@@ -239,16 +274,19 @@ def gpu_cases(dump):
     model = model_of(3, 64, 64, learn_eps=True, nb_pool="average", graph_pool="average", seed=4)
     train_case("average.isolated", model, iso)
     saliency_case("average.isolated.saliency", model, iso)
+    run_attribution_cases(shim, "average.isolated.attribution", model, iso, **attribution)
 
     mx = synth.make_graphs(8, n_rois=64, n_time=128, seed0=50, with_neighbors=True)
     model = model_of(3, 64, 64, nb_pool="max", seed=5)
     train_case("max", model, mx)
     saliency_case("max.saliency", model, mx[:1], roi_graphs=mx[:1])
+    run_attribution_cases(shim, "max.attribution", model, mx, **attribution)
 
     wide = synth.make_graphs(16, n_rois=64, n_time=128, seed0=60)
     model = model_of(3, 64, 128, seed=6)
     train_case("hidden128", model, wide)
     saliency_case("hidden128.saliency", model, wide)
+    run_attribution_cases(shim, "hidden128.attribution", model, wide, **attribution)
 
 
 def main():

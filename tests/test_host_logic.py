@@ -6,10 +6,8 @@ import numpy as np
 import pytest
 import torch
 
-import emul_ops
-from helpers import Golden, SEED0, assert_close, golden_names, grad_floor
+from helpers import Golden, SEED0, assert_close, build_model, golden_names, grad_floor, use_cpu_stand_in
 from graph_neural_mapping_b200 import engine
-from graph_neural_mapping_b200.models import graphcnn as gmod
 from graph_neural_mapping_b200.models import mlp as mlpmod
 from graph_neural_mapping_b200.models import discriminator as dmod
 
@@ -20,19 +18,7 @@ TOL_GRAD = 2e-3
 
 @pytest.fixture(autouse=True)
 def cpu_backend(monkeypatch):
-    monkeypatch.setattr(engine, "_ops", emul_ops)
-    monkeypatch.setattr(mlpmod, "_ops", emul_ops)
-    monkeypatch.setattr(dmod, "_ops", emul_ops)
-    monkeypatch.setattr(engine, "require_cuda", lambda dev: None)
-
-
-def build_model(g, sd=None):
-    c = g.cfg
-    m = gmod.GIN_InfoMaxReg(c["num_layers"], c["num_mlp_layers"], c["input_dim"], c["hidden_dim"], c["output_dim"],
-                            c["final_dropout"], c["learn_eps"], c["graph_pooling_type"], c["neighbor_pooling_type"],
-                            torch.device("cpu"))
-    m.load_state_dict(sd if sd is not None else g.state_dict())
-    return m
+    use_cpu_stand_in(monkeypatch)
 
 
 def train_step(model, graphs, g, seed):

@@ -1,85 +1,24 @@
 """Host logic of integrated gradients on CPU: GIN_InfoMaxReg.compute_integrated_gradients_batched /
-driver.integrated_gradients over the CPU stand-in kernels (tests/emul_ops.py) plus stand-ins of gnm_ig_expand,
-gnm_ig_accumulate and gnm_ig_attribute written from their include/gnm.h contracts. Checks the attributions and the
-completeness gap against plain autograd on the fp64 oracle (tests/ig_reference.py), the virtual-batch plumbing (one
-forward per pass, one backward per class and pass, chunking), the argument errors, and that the new entry points check
-their arguments without a GPU."""
+driver.integrated_gradients over the CPU stand-in kernels (tests/emul_ops.py). Checks the attributions and the
+completeness gap against plain autograd on the fp64 oracle (tests/attribution_reference.py), the virtual-batch plumbing
+(one forward per pass, one backward per class and pass, chunking), the argument errors, and that the new entry points
+check their arguments without a GPU."""
 import numpy as np
 import pytest
 import torch
 
-import emul_ops
-from helpers import Golden, assert_close
-from ig_reference import integrated_gradients as ig_oracle, oracle_config
+from attribution_reference import integrated_gradients as ig_oracle, oracle_config
+from helpers import Golden, assert_close, build_model, use_cpu_stand_in
 from graph_neural_mapping_b200 import driver, engine, lib
-from graph_neural_mapping_b200.models import graphcnn as gmod
-from graph_neural_mapping_b200.models import mlp as mlpmod
-from graph_neural_mapping_b200.models import discriminator as dmod
 from graph_neural_mapping_b200.synth import SynthGraph
 
 NAMES = ["tiny_eps_sum", "tiny_noeps_sum", "tiny_eps_avg", "tiny_noeps_avg", "tiny_mlp1", "tiny_mlp3", "mid_eps_sum_h64"]
 TOL_GRAD = 2e-3
 
 
-def ig_expand(p, bias, alpha, node_off, points, z):
-    """gnm_ig_expand: z[(g, s, i)] = alpha[s] * p[node_off[g] + i] + bias, graph-major virtual rows."""
-    no = node_off.long().tolist()
-    rows = []
-    for g in range(len(no) - 1):
-        for s in range(points):
-            v = float(alpha[s]) * p[no[g]:no[g + 1]].double()
-            rows.append(v + bias.double() if bias is not None else v)
-    if rows:
-        z.copy_(torch.cat(rows).float())
-    return z
-
-
-def ig_accumulate(dy, coef, node_off, points, weight, out, accumulate):
-    """gnm_ig_accumulate: out[r] (+)= weight * cA o sum_s dy[(g, s, r - node_off[g])]."""
-    no = node_off.long().tolist()
-    ca = coef[0].double() if coef is not None else 1.0
-    for g in range(len(no) - 1):
-        n = no[g + 1] - no[g]
-        base = points * no[g]
-        v = weight * ca * dy[base:base + points * n].double().view(points, n, -1).sum(0)
-        if accumulate:
-            v = v + out[no[g]:no[g + 1]].double()
-        out[no[g]:no[g + 1]] = v.float()
-    return out
-
-
-def ig_attribute(t, table, tags, node_off, out):
-    """gnm_ig_attribute: out[g, d] = (1/n_g) sum_{n in g, tags[n] = d} <t[n], table[d]>; NaN row for non-finite t."""
-    a = (t.double() * table.double()[tags.long()]).sum(1)
-    no = node_off.long().tolist()
-    for g in range(len(no) - 1):
-        r0, r1 = no[g], no[g + 1]
-        row = torch.zeros(out.shape[1], dtype=torch.float64).index_add_(0, tags[r0:r1].long(), a[r0:r1])
-        row = row / max(r1 - r0, 1)
-        if not bool(torch.isfinite(t[r0:r1]).all()):
-            row[:] = float("nan")
-        out[g] = row.float()
-    return out
-
-
 @pytest.fixture(autouse=True)
 def cpu_backend(monkeypatch):
-    for name, fn in (("ig_expand", ig_expand), ("ig_accumulate", ig_accumulate), ("ig_attribute", ig_attribute)):
-        monkeypatch.setattr(emul_ops, name, fn, raising=False)
-    monkeypatch.setattr(engine, "_ops", emul_ops)
-    monkeypatch.setattr(gmod, "_ops", emul_ops)
-    monkeypatch.setattr(mlpmod, "_ops", emul_ops)
-    monkeypatch.setattr(dmod, "_ops", emul_ops)
-    monkeypatch.setattr(engine, "require_cuda", lambda dev: None)
-
-
-def build_model(g, sd=None):
-    c = g.cfg
-    m = gmod.GIN_InfoMaxReg(c["num_layers"], c["num_mlp_layers"], c["input_dim"], c["hidden_dim"], c["output_dim"],
-                            c["final_dropout"], c["learn_eps"], c["graph_pooling_type"], c["neighbor_pooling_type"],
-                            torch.device("cpu"))
-    m.load_state_dict(sd if sd is not None else g.state_dict())
-    return m
+    use_cpu_stand_in(monkeypatch)
 
 
 @pytest.mark.parametrize("name", NAMES)

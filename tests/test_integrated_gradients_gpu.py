@@ -9,15 +9,14 @@ import numpy as np
 import pytest
 import torch
 
+from attribution_cases import CONFIGS, DEV, graphs_of, launches, make_model, strided
+from attribution_reference import integrated_gradients as ig_oracle, oracle_config
 from helpers import Golden, assert_close, golden_names
-from ig_reference import integrated_gradients as ig_oracle, oracle_config
-from test_roi_saliency_gpu import CONFIGS, graphs_of, make_model
 from graph_neural_mapping_b200 import driver, lib, ops
 from graph_neural_mapping_b200.models import GIN_InfoMaxReg
 from graph_neural_mapping_b200.synth import SynthGraph
 
 pytestmark = pytest.mark.gpu
-DEV = torch.device("cuda")
 TOL_GRAD = 3e-3
 STEPS = 8
 
@@ -113,19 +112,12 @@ def test_isolated_nodes_average_learn_eps():
         assert_close_composed(out[:, k], ref[:, k], "class %d" % k)
 
 
-def _ran(fn):
-    before = ops.launch_counts()
-    out = fn()
-    torch.cuda.synchronize()
-    return out, {k: v - before[k] for k, v in ops.launch_counts().items()}
-
-
 def test_launch_counts_and_reproducibility():
     """At the benchmark shape: 50 points x 20 graphs x 400 nodes = one 1000-graph virtual batch per pass."""
     model = make_model(400, seed=1)
     graphs = graphs_of(40, 400, seed=3)
     model.compute_integrated_gradients_batched(graphs[:1], (0,), steps=2)
-    a, ran = _ran(lambda: model.compute_integrated_gradients_batched(graphs, (0, 1), steps=50))
+    a, ran = launches(lambda: model.compute_integrated_gradients_batched(graphs, (0, 1), steps=50))
     passes = chunks = 2
     assert ran["aggregate_tc"] > 0 and ran["linear_tc"] > 0, ran
     assert ran["linear_ffma"] == 0, ran                                       # no [M, 64] -> [M, 400] Linear
@@ -153,13 +145,6 @@ def test_parameter_gradients_untouched():
 COUNTS = [5, 0, 400, 1, 0, 37, 129, 2]
 
 
-def _strided(m, w, pad, gen):
-    """[m, w] view with leading dimension w + pad, starting one float into its buffer when pad > 0 (misaligned rows)."""
-    off = 1 if pad else 0
-    buf = torch.randn(m * (w + pad) + off, generator=gen).to(DEV)
-    return buf[off:off + m * (w + pad)].view(m, w + pad)[:, :w]
-
-
 def _offsets():
     counts = torch.tensor(COUNTS)
     return counts, torch.cat([torch.zeros(1, dtype=torch.int64), counts.cumsum(0)]).to(torch.int32).to(DEV)
@@ -171,18 +156,18 @@ def test_expand_and_accumulate_against_torch(width, pad):
     gen = torch.Generator().manual_seed(width * 10 + pad)
     counts, node_off = _offsets()
     m, points = int(counts.sum()), 5
-    p = _strided(m, width, pad, gen)
+    p = strided(m, width, pad, gen)
     bias = torch.randn(width, generator=gen).to(DEV)
     alpha = torch.rand(points, generator=gen).to(DEV)
     no = node_off.long().tolist()
-    z = _strided(points * m, width, pad, gen)
+    z = strided(points * m, width, pad, gen)
     ops.ig_expand(p, bias, alpha, node_off, points, z)
     ref = torch.cat([alpha[s].double() * p[no[g]:no[g + 1]].double() + bias.double()
                      for g in range(len(COUNTS)) for s in range(points)])
     assert_close(z, ref.cpu(), 1e-6, "expand")
-    dy = _strided(points * m, width, pad, gen)
+    dy = strided(points * m, width, pad, gen)
     coef = torch.randn(3, width, generator=gen).to(DEV)
-    out = _strided(m, width, pad, gen)
+    out = strided(m, width, pad, gen)
     ops.ig_accumulate(dy, coef, node_off, points, 0.25, out, False)
     ref = torch.cat([0.25 * coef[0].double() * dy[points * no[g]:points * no[g + 1]].double().view(points, COUNTS[g], width).sum(0)
                      for g in range(len(COUNTS))])
@@ -199,8 +184,8 @@ def test_attribute_against_torch(width, pad):
     gen = torch.Generator().manual_seed(width * 10 + pad + 1)
     counts, node_off = _offsets()
     m, d = int(counts.sum()), 450
-    t = _strided(m, width, pad, gen)
-    table = _strided(d, width, pad, gen)
+    t = strided(m, width, pad, gen)
+    table = strided(d, width, pad, gen)
     tags = torch.randint(0, d, (m,), generator=gen)
     tags[400:410] = 3                                          # duplicate tags inside the 400-node graph
     tags = tags.to(torch.int32).to(DEV)

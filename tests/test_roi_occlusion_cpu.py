@@ -1,20 +1,15 @@
 """Host logic of ROI occlusion on CPU: GIN_InfoMaxReg.compute_roi_occlusion_batched / driver.roi_occlusion over the CPU
-stand-in kernels (tests/emul_ops.py) plus a stand-in of gnm_occlusion_expand written from its include/gnm.h contract.
-Checks the output against the fp64 oracle (tests/occlusion_reference.py), the pass planning (graphs split over passes,
-several graphs per pass, one forward per pass), the argument errors, and that the new entry point checks its arguments
-without a GPU."""
+stand-in kernels (tests/emul_ops.py). Checks the output against the fp64 oracle (tests/attribution_reference.py), the
+pass planning (graphs split over passes, several graphs per pass, one forward per pass), the argument errors, and that
+the new entry point checks its arguments without a GPU."""
 import numpy as np
 import pytest
 import torch
 
-import emul_ops
-from helpers import Golden, assert_close
-from ig_reference import oracle_config
-from occlusion_reference import roi_occlusion as occ_oracle, with_neighbours
+from attribution_reference import oracle_config, roi_occlusion as occ_oracle, with_neighbours
+from helpers import Golden, assert_close, build_model, use_cpu_stand_in
 from graph_neural_mapping_b200 import driver, engine, lib
 from graph_neural_mapping_b200.models import graphcnn as gmod
-from graph_neural_mapping_b200.models import mlp as mlpmod
-from graph_neural_mapping_b200.models import discriminator as dmod
 from graph_neural_mapping_b200.synth import SynthGraph
 
 NAMES = ["tiny_eps_sum", "tiny_noeps_sum", "tiny_eps_avg", "tiny_noeps_avg", "tiny_eps_max", "tiny_noeps_max",
@@ -22,48 +17,9 @@ NAMES = ["tiny_eps_sum", "tiny_noeps_sum", "tiny_eps_avg", "tiny_noeps_avg", "ti
 TOL = 1e-4
 
 
-def occlusion_expand(p, bias, w1t, rowptr, colidx, tags, node_off, n_max, v_graph, v_tag, v_node_off, mode, eps, z):
-    """gnm_occlusion_expand: z[v_node_off[v] + i] = p[m] + bias - c_d[m] w1t[d], c_d[m] = s_m #{n in CSR row m:
-    tags[n] = d} + (eps ? (1 + eps) [tags[m] = d] : 0), s_m = 1 (mode 0) or 1 / (row length) (mode 1)."""
-    m_all = p.shape[0]
-    rp, ci, tg = rowptr.long(), colidx.long(), tags.long()
-    rows = torch.repeat_interleave(torch.arange(m_all), rp[1:] - rp[:-1])
-    counts = torch.zeros(m_all, w1t.shape[0], dtype=torch.float64)
-    counts.index_put_((rows, tg[ci]), torch.ones(ci.numel(), dtype=torch.float64), accumulate=True)
-    deg = (rp[1:] - rp[:-1]).double()
-    no, vno = node_off.long().tolist(), v_node_off.long().tolist()
-    base = p.double() + (bias.double() if bias is not None else 0.0)
-    for v in range(v_graph.shape[0]):
-        g, d = int(v_graph[v]), int(v_tag[v])
-        r0, r1 = no[g], no[g + 1]
-        val = base[r0:r1].clone()
-        if 0 <= d < w1t.shape[0]:
-            c = counts[r0:r1, d]
-            coef = torch.where(c != 0, c / deg[r0:r1] if mode == 1 else c, torch.zeros_like(c))
-            if eps is not None:
-                coef = coef + (1.0 + float(eps[0])) * (tg[r0:r1] == d).double()
-            val = val - coef.unsqueeze(1) * w1t[d].double()
-        z[vno[v]:vno[v] + r1 - r0] = val.float()
-    return z
-
-
 @pytest.fixture(autouse=True)
 def cpu_backend(monkeypatch):
-    monkeypatch.setattr(emul_ops, "occlusion_expand", occlusion_expand, raising=False)
-    monkeypatch.setattr(engine, "_ops", emul_ops)
-    monkeypatch.setattr(gmod, "_ops", emul_ops)
-    monkeypatch.setattr(mlpmod, "_ops", emul_ops)
-    monkeypatch.setattr(dmod, "_ops", emul_ops)
-    monkeypatch.setattr(engine, "require_cuda", lambda dev: None)
-
-
-def build_model(g, sd=None):
-    c = g.cfg
-    m = gmod.GIN_InfoMaxReg(c["num_layers"], c["num_mlp_layers"], c["input_dim"], c["hidden_dim"], c["output_dim"],
-                            c["final_dropout"], c["learn_eps"], c["graph_pooling_type"], c["neighbor_pooling_type"],
-                            torch.device("cpu"))
-    m.load_state_dict(sd if sd is not None else g.state_dict())
-    return m
+    use_cpu_stand_in(monkeypatch)
 
 
 def assert_matches(out, ref, f_x, n, what):

@@ -8,17 +8,15 @@ import numpy as np
 import pytest
 import torch
 
+from attribution_cases import CONFIGS, DEV, graphs_of, launches, make_model, strided
+from attribution_reference import oracle_config, roi_occlusion as occ_oracle, with_neighbours
 from helpers import Golden, assert_close, golden_names
-from ig_reference import oracle_config
-from occlusion_reference import roi_occlusion as occ_oracle, with_neighbours
-from test_roi_saliency_gpu import CONFIGS, graphs_of, make_model
 from graph_neural_mapping_b200 import driver, lib, ops
 from graph_neural_mapping_b200.models import GIN_InfoMaxReg
 from graph_neural_mapping_b200.models import graphcnn as gmod
 from graph_neural_mapping_b200.synth import SynthGraph
 
 pytestmark = pytest.mark.gpu
-DEV = torch.device("cuda")
 # The score is continuous in the input, so unlike a gradient it cannot jump at a ReLU kink: each class is compared on
 # its own max-abs, with the scores' |F_c(X)| / n as floor (the output is a difference of two scores, divided by n).
 TOL = 1e-4
@@ -135,18 +133,11 @@ def test_isolated_nodes_average_learn_eps():
     assert torch.equal(torch.isnan(out).any(2), torch.isnan(out).all(2))
 
 
-def _ran(fn):
-    before = ops.launch_counts()
-    out = fn()
-    torch.cuda.synchronize()
-    return out, {k: v - before[k] for k, v in ops.launch_counts().items()}
-
-
 def test_launch_counts_and_reproducibility():
     model = make_model(400, seed=1)
     graphs = graphs_of(40, 400, seed=3)
     model.compute_roi_occlusion_batched(graphs[:1], (0,))
-    a, ran = _ran(lambda: model.compute_roi_occlusion_batched(graphs, (0, 1)))
+    a, ran = launches(lambda: model.compute_roi_occlusion_batched(graphs, (0, 1)))
     h = model._host_batch(graphs)
     passes = len(gmod.occlusion_passes(h.node_off, model._structure(graphs).tags.cpu().numpy(), 1024))
     assert passes == 16, passes                               # 40 x (400 + 1) virtual graphs, 1024 per pass
@@ -181,13 +172,6 @@ def test_parameter_gradients_untouched():
 
 COUNTS = [5, 0, 400, 1, 37, 129, 2]
 D_TAGS = 450
-
-
-def _strided(m, w, pad, gen):
-    """[m, w] view with leading dimension w + pad, starting one float into its buffer when pad > 0 (misaligned rows)."""
-    off = 1 if pad else 0
-    buf = torch.randn(m * (w + pad) + off, generator=gen).to(DEV)
-    return buf[off:off + m * (w + pad)].view(m, w + pad)[:, :w]
 
 
 def _real_batch(gen, self_loops):
@@ -230,11 +214,11 @@ def test_kernel_against_torch(width, pad, mode, learn_eps):
             v_graph.append(g)
             v_tag.append(t)
     v_node_off = np.cumsum([0] + [COUNTS[g] for g in v_graph])
-    p = _strided(m, width, pad, gen)
-    w1t = _strided(D_TAGS, width, pad, gen)
+    p = strided(m, width, pad, gen)
+    w1t = strided(D_TAGS, width, pad, gen)
     bias = torch.randn(width, generator=gen).to(DEV)
     eps = torch.tensor([0.3]).to(DEV) if learn_eps else None
-    z = _strided(int(v_node_off[-1]), width, pad, gen)
+    z = strided(int(v_node_off[-1]), width, pad, gen)
     to_d = lambda t: t.to(DEV)
     ops.occlusion_expand(p, bias, w1t, to_d(rowptr), to_d(colidx), to_d(tags), to_d(node_off), max(COUNTS),
                          to_d(torch.tensor(v_graph, dtype=torch.int32)), to_d(torch.tensor(v_tag, dtype=torch.int32)),

@@ -1,63 +1,21 @@
 """Host logic of ROI saliency on CPU: GIN_InfoMaxReg.compute_roi_saliency_batched / driver.roi_saliency over the CPU
-stand-in kernels (tests/emul_ops.py) plus a stand-in of gnm_segment_weighted_colsum written from its include/gnm.h
-contract. Checks the node averages against the reference's saliency maps in the golden fixtures, the one-forward /
-many-backward reuse, and that no parameter gradient is written."""
+stand-in kernels (tests/emul_ops.py). Checks the node averages against the reference's saliency maps in the golden
+fixtures, the one-forward / many-backward reuse, and that no parameter gradient is written."""
 import numpy as np
 import pytest
 import torch
 
-import emul_ops
-from helpers import Golden, assert_close, golden_names
+from helpers import Golden, assert_close, build_model, golden_names, use_cpu_stand_in
 from graph_neural_mapping_b200 import driver, engine
-from graph_neural_mapping_b200.models import graphcnn as gmod
-from graph_neural_mapping_b200.models import mlp as mlpmod
-from graph_neural_mapping_b200.models import discriminator as dmod
 from graph_neural_mapping_b200.synth import SynthGraph
 
 NAMES = [n for n in golden_names() if Golden(n).cfg["N"] < 400]     # the dense CPU stand-in is too slow at N = 400
 TOL_GRAD = 2e-3
 
 
-def segment_weighted_colsum(x, node_off, out, z=None, coef=None, rowptr=None, mode=0, eps=None):
-    """gnm_segment_weighted_colsum: out[g] = (1/n_g) sum_{m in g} w_m v[m], v = x or cA x + cB z + cC, w_m the row sums
-    of the aggregation operator (deg, or 1 / 0 for an isolated node under average, + 1 + eps), zeros for an empty graph."""
-    v = x.double()
-    if coef is not None:
-        v = coef[0].double() * v
-        if z is not None:
-            v = v + coef[1].double() * z.double() + coef[2].double()
-    m = x.shape[0]
-    if rowptr is None:
-        w = torch.ones(m, dtype=torch.float64)
-    else:
-        deg = (rowptr[1:] - rowptr[:-1]).double()
-        w = (deg > 0).double() if mode == 1 else deg
-        if eps is not None:
-            w = w + 1.0 + eps.double()
-    no = node_off.long()
-    gid = torch.repeat_interleave(torch.arange(no.numel() - 1), no[1:] - no[:-1])
-    s = torch.zeros(out.shape[0], x.shape[1], dtype=torch.float64).index_add_(0, gid, w.unsqueeze(1) * v)
-    n = (no[1:] - no[:-1]).double().clamp(min=1).unsqueeze(1)
-    out.copy_((s / n).float())
-    return out
-
-
 @pytest.fixture(autouse=True)
 def cpu_backend(monkeypatch):
-    monkeypatch.setattr(emul_ops, "segment_weighted_colsum", segment_weighted_colsum, raising=False)
-    monkeypatch.setattr(engine, "_ops", emul_ops)
-    monkeypatch.setattr(mlpmod, "_ops", emul_ops)
-    monkeypatch.setattr(dmod, "_ops", emul_ops)
-    monkeypatch.setattr(engine, "require_cuda", lambda dev: None)
-
-
-def build_model(g, sd=None):
-    c = g.cfg
-    m = gmod.GIN_InfoMaxReg(c["num_layers"], c["num_mlp_layers"], c["input_dim"], c["hidden_dim"], c["output_dim"],
-                            c["final_dropout"], c["learn_eps"], c["graph_pooling_type"], c["neighbor_pooling_type"],
-                            torch.device("cpu"))
-    m.load_state_dict(sd if sd is not None else g.state_dict())
-    return m
+    use_cpu_stand_in(monkeypatch)
 
 
 @pytest.mark.parametrize("name", NAMES)

@@ -7,60 +7,22 @@ import numpy as np
 import pytest
 import torch
 
+from attribution_cases import CONFIGS, DEV, graphs_of, launches, make_model, strided
+from attribution_reference import oracle_config
 from helpers import Golden, assert_close, golden_names, rel_err
 from oracle import gin_oracle
-from graph_neural_mapping_b200 import engine, lib, ops, synth
+from graph_neural_mapping_b200 import engine, lib, ops
 from graph_neural_mapping_b200.models import GIN_InfoMaxReg
 from graph_neural_mapping_b200.synth import SynthGraph
 
 pytestmark = pytest.mark.gpu
-DEV = torch.device("cuda")
 TOL_GRAD = 3e-3
-
-
-def make_model(d, f=64, layers=5, mlp=2, eps=False, graph_pool="sum", neigh_pool="sum", seed=0):
-    torch.manual_seed(seed)
-    m = GIN_InfoMaxReg(layers, mlp, d, f, 2, 0.0, eps, graph_pool, neigh_pool, DEV).to(DEV)
-    with torch.no_grad():
-        # eval BatchNorm with non-trivial running statistics and affine, so that the ReLU masks are mixed
-        for mod in m.modules():
-            if isinstance(mod, torch.nn.BatchNorm1d):
-                mod.running_mean.uniform_(-0.2, 0.2)
-                mod.running_var.uniform_(0.5, 2.0)
-                mod.weight.uniform_(0.5, 1.5)
-                mod.bias.uniform_(-0.1, 0.2)
-        m.eps.uniform_(-0.3, 0.3)
-    return m
-
-
-def graphs_of(b, n, seed=0, dense_dim=None, sparsity=30):
-    gs = synth.make_graphs_bulk(b, n, sparsity, 128, seed0=seed, device=DEV)
-    if dense_dim is not None:
-        gen = torch.Generator().manual_seed(seed)
-        gs = [SynthGraph(n, g.label, g.edge_mat, torch.rand(n, dense_dim, generator=gen)) for g in gs]
-    return gs
 
 
 def full_map_mean(model, graphs, cls):
     s = model.compute_saliency_batched(graphs, cls).detach()
     off = np.cumsum([0] + [len(g.g) for g in graphs])
     return torch.stack([s[off[i]:off[i + 1]].mean(0) for i in range(len(graphs))])
-
-
-CONFIGS = {
-    # name: (model kwargs, B, N, dense input width or None)
-    "b1024_sum_tcgen05": (dict(), 1024, 400, None),
-    "learn_eps": (dict(eps=True), 64, 400, None),
-    "average_neighbour": (dict(neigh_pool="average"), 64, 400, None),
-    "average_graph": (dict(graph_pool="average"), 64, 400, None),
-    "max_neighbour": (dict(neigh_pool="max"), 8, 400, None),
-    "mlp1": (dict(mlp=1), 64, 400, None),
-    "mlp3_eps": (dict(mlp=3, eps=True), 64, 400, None),
-    "dense_input_d400": (dict(), 32, 400, 400),
-    "dense_input_d48_fused": (dict(eps=True), 32, 400, 48),
-    "dense_input_max": (dict(neigh_pool="max"), 8, 200, 48),
-    "n1000_f128": (dict(f=128), 8, 1000, None),
-}
 
 
 @pytest.mark.parametrize("name", sorted(CONFIGS))
@@ -116,8 +78,7 @@ def test_roi_vs_reference_and_oracle(name):
     model.load_state_dict(g.state_after_train())
     model = model.to(DEV)
     graphs = g.graphs()
-    ocfg = gin_oracle.OracleConfig(c["num_layers"], c["num_mlp_layers"], c["input_dim"], c["hidden_dim"], c["output_dim"],
-                                   c["final_dropout"], c["learn_eps"], c["graph_pooling_type"], c["neighbor_pooling_type"])
+    ocfg = oracle_config(c)
     sd = {k: v.detach().cpu() for k, v in model.state_dict().items()}
     for k, v in g.group("saliency/").items():
         gi, cls = int(k[1:k.index("_")]), int(k[-1])
@@ -127,13 +88,6 @@ def test_roi_vs_reference_and_oracle(name):
         assert_close(got, oracle_mean, TOL_GRAD, "roi vs fp64 oracle " + k)
         own = rel_err(ref_mean, oracle_mean)
         assert_close(got, ref_mean, TOL_GRAD + own, "roi vs reference " + k)
-
-
-def _ran(fn):
-    before = ops.launch_counts()
-    out = fn()
-    torch.cuda.synchronize()
-    return out, {k: v - before[k] for k, v in ops.launch_counts().items()}
 
 
 @pytest.fixture(scope="module")
@@ -146,9 +100,9 @@ def bench_shape():
 
 def test_one_forward_serves_both_classes(bench_shape):
     model, graphs = bench_shape
-    both, ran2 = _ran(lambda: model.compute_roi_saliency_batched(graphs, (0, 1)))
-    one0, ran1 = _ran(lambda: model.compute_roi_saliency_batched(graphs, (0,)))
-    one1, _ = _ran(lambda: model.compute_roi_saliency_batched(graphs, (1,)))
+    both, ran2 = launches(lambda: model.compute_roi_saliency_batched(graphs, (0, 1)))
+    one0, ran1 = launches(lambda: model.compute_roi_saliency_batched(graphs, (0,)))
+    one1, _ = launches(lambda: model.compute_roi_saliency_batched(graphs, (1,)))
     # every kernel here sums in a fixed order (no fp32 atomics on these outputs): bit-identical
     assert torch.equal(both[:, 0], one0[:, 0]) and torch.equal(both[:, 1], one1[:, 0])
 
@@ -157,7 +111,7 @@ def test_one_forward_serves_both_classes(bench_shape):
         params = [p.detach() for p in engine.flat_params(model)]
         with torch.no_grad():
             engine.run_forward(model, bs, None, False, False, None, params, engine._dist.SINGLE)
-    _, fwd = _ran(forward_only)
+    _, fwd = launches(forward_only)
     assert fwd["linear_tc"] > 0 and fwd["aggregate_tc"] > 0, fwd
     # the second class adds exactly one backward: every family's count grows by (one class) - (the forward)
     for k in ran1:
@@ -168,8 +122,8 @@ def test_one_forward_serves_both_classes(bench_shape):
 
 def test_launch_counts_against_full_map(bench_shape):
     model, graphs = bench_shape
-    _, roi = _ran(lambda: model.compute_roi_saliency_batched(graphs, (1,)))
-    _, full = _ran(lambda: model.compute_saliency_batched(graphs, 1))
+    _, roi = launches(lambda: model.compute_roi_saliency_batched(graphs, (1,)))
+    _, full = launches(lambda: model.compute_saliency_batched(graphs, 1))
     assert roi["aggregate_tc"] == full["aggregate_tc"] - 1, (roi, full)      # no affine aggregation of dz
     assert roi["linear_ffma"] == 0 and full["linear_ffma"] >= 1, (roi, full)  # no [M, 64] -> [M, 400] Linear
     assert roi["segment_colsum"] == 1 and full["segment_colsum"] == 0, (roi, full)
@@ -215,13 +169,6 @@ def _reference(x, node_off, z, coef, rowptr, mode, eps):
     return s / (no[1:] - no[:-1]).double().clamp(min=1)[:, None]
 
 
-def _strided(m, w, pad, gen):
-    """[m, w] view with leading dimension w + pad, starting one float into its buffer when pad > 0 (misaligned rows)."""
-    off = 1 if pad else 0
-    buf = torch.randn(m * (w + pad) + off, generator=gen).to(DEV)
-    return buf[off:off + m * (w + pad)].view(m, w + pad)[:, :w]
-
-
 @pytest.mark.parametrize("width", [1, 3, 64, 400])
 @pytest.mark.parametrize("pad", [0, 3])
 def test_kernel_against_torch(width, pad):
@@ -232,7 +179,7 @@ def test_kernel_against_torch(width, pad):
     deg = torch.randint(0, 9, (m,), generator=gen)
     deg[::17] = 0                                              # isolated rows
     rowptr = torch.cat([torch.zeros(1, dtype=torch.int64), deg.cumsum(0)]).to(torch.int32).to(DEV)
-    x, z = _strided(m, width, pad, gen), _strided(m, width, pad, gen)
+    x, z = strided(m, width, pad, gen), strided(m, width, pad, gen)
     coef = torch.randn(3, width, generator=gen).to(DEV)
     eps = torch.tensor([0.25]).to(DEV)
     b = counts.numel()

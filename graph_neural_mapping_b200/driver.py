@@ -27,22 +27,14 @@ from . import ops as _ops
 
 
 class _WholeStepPlan(object):
-    def __init__(self, trainer, h, n_global):
+    def __init__(self, trainer, h, key, n_global):
         model = trainer.model
         dev = model.eps.device
         self.trainer, self.dev = trainer, dev
-        self.sig = trainer._signature(h, n_global)
-        self.nnz_cap = int(h.nnz * 1.02) + 4096
-        self.packed = torch.zeros(5 * h.b + 1, dtype=torch.int64, device=dev)
-        self.node_off = torch.zeros(h.b + 1, dtype=torch.int32, device=dev)
-        self.neg_idx = torch.zeros(n_global, dtype=torch.int32, device=dev)
-        self.labels = torch.zeros(h.b, dtype=torch.int64, device=dev)
+        self.inputs = _graphed.StepInputs(model, h, key, n_global, labels=True)
         self.d_labels = torch.cat([torch.ones(h.m, 1), torch.zeros(h.m, 1)], 0).to(dev)      # main.py:32-33
-        self.stage = [None, None, None]
-        self.stage_i = 0
         self.graph = None
         self.loss = None
-        self.h = h
         self.launches = 0
         if trainer.fused:
             heads = list(model.linears_prediction)
@@ -52,31 +44,6 @@ class _WholeStepPlan(object):
             self.heads_ws = torch.empty(_ops.heads_ce_workspace(h.b, len(heads), n_feat, n_cls), dtype=torch.float32, device=dev)
             self.heads_counter = torch.zeros(1, dtype=torch.int32, device=dev)
             self.c_logit = None
-
-    def load(self, h, perm, labels):
-        """Host -> device traffic of one step, staged through a ring of pinned buffers (never waits for the GPU)."""
-        self.h = h
-        i = self.stage_i
-        self.stage_i = (i + 1) % len(self.stage)
-        if self.stage[i] is None:
-            self.stage[i] = (torch.empty(self.packed.shape[0], dtype=torch.int64, pin_memory=True),
-                             torch.empty(self.node_off.shape[0], dtype=torch.int32, pin_memory=True),
-                             torch.empty(self.neg_idx.shape[0], dtype=torch.int32, pin_memory=True),
-                             torch.empty(self.labels.shape[0], dtype=torch.int64, pin_memory=True),
-                             torch.cuda.Event())
-        else:
-            self.stage[i][4].synchronize()
-        s_packed, s_off, s_neg, s_lab, ev = self.stage[i]
-        s_packed.numpy()[:] = h.packed
-        s_off.numpy()[:] = h.node_off
-        s_neg.numpy()[:] = perm
-        s_lab.numpy()[:] = labels
-        self.packed.copy_(s_packed, non_blocking=True)
-        self.node_off.copy_(s_off, non_blocking=True)
-        self.neg_idx.copy_(s_neg, non_blocking=True)
-        self.labels.copy_(s_lab, non_blocking=True)
-        ev.record()
-        return h.packed.nbytes + h.node_off.nbytes + 4 * perm.size + 8 * len(labels)
 
     def body(self):
         return self.body_fused() if self.trainer.fused else self.body_autograd()
@@ -90,15 +57,13 @@ class _WholeStepPlan(object):
         tr = self.trainer
         model = tr.model
         dev = self.dev
-        store = model._graph_store()
-        bs = store.assemble_device(self.h, self.packed, self.node_off, nnz_capacity=self.nnz_cap)
-        bs.set_pooling(model.graph_pooling_type, dev)
+        bs = self.inputs.structure()
         enc_params = _engine.flat_params(model)
         params = [p.detach() for p in enc_params]
         b, m = bs.n_graphs, bs.n_rows
         self.loss_terms.zero_()                     # [CE mean, beta * BCE mean], float64
         w_bce = tr.beta / (2.0 * m)                 # main.py:32-37: BCEWithLogits mean over 2m scores, times beta
-        g_f, d_logit, sv = _engine.run_forward(model, bs, self.neg_idx, True, True, None, params, tr.comm,
+        g_f, d_logit, sv = _engine.run_forward(model, bs, self.inputs.neg_idx, True, True, None, params, tr.comm,
                                                bce=(w_bce, w_bce, self.loss_terms[1:2]))
         heads = list(model.linears_prediction)
         n_layers, n_cls, n_feat = len(heads), heads[0].weight.shape[0], heads[0].weight.shape[1]
@@ -113,7 +78,7 @@ class _WholeStepPlan(object):
             mask = torch.empty(n_layers, b, n_cls, dtype=torch.float32, device=dev).bernoulli_(keep).mul_(1.0 / keep)
         c_logit = torch.empty(b, n_cls, dtype=torch.float32, device=dev)
         d_gf = torch.empty_like(g_f)
-        _ops.heads_ce(g_f, hw, hb, mask, self.labels, 1.0 / b, c_logit, self.loss_terms[0:1], d_gf, d_hw, d_hb,
+        _ops.heads_ce(g_f, hw, hb, mask, self.inputs.labels, 1.0 / b, c_logit, self.loss_terms[0:1], d_gf, d_hw, d_hb,
                       self.heads_ws, self.heads_counter)
         dd = None
         if sv.scored is None:
@@ -155,14 +120,11 @@ class _WholeStepPlan(object):
         """One training step on the static buffers (runs eagerly while warming up, then under capture)."""
         tr = self.trainer
         model = tr.model
-        store = model._graph_store()
-        bs = store.assemble_device(self.h, self.packed, self.node_off, nnz_capacity=self.nnz_cap)
-        bs.set_pooling(model.graph_pooling_type, self.dev)
-        runner = _engine.Runner(model, bs, self.neg_idx, True, True, tr.comm)
+        runner = _engine.Runner(model, self.inputs.structure(), self.inputs.neg_idx, True, True, tr.comm)
         tr.optimizer.zero_grad(set_to_none=True)
         g_f, d_logit = _engine.GINFunction.apply(runner, None, *_engine.flat_params(model))
         c_logit = model._heads(g_f)
-        loss = tr.c_criterion(c_logit, self.labels) + tr.beta * tr.d_criterion(d_logit, self.d_labels)     # main.py:34-37
+        loss = tr.c_criterion(c_logit, self.inputs.labels) +tr.beta * tr.d_criterion(d_logit, self.d_labels)     # main.py:34-37
         loss.backward()
         _dist.average_gradients(model, tr.comm)
         tr.optimizer.step()
@@ -170,15 +132,8 @@ class _WholeStepPlan(object):
 
     def run(self):
         if self.graph is None:
-            g = torch.cuda.CUDAGraph()
-            n0 = _ops.kernels_recorded()
-            with _graphed.quiet_capture(), torch.cuda.graph(g):
-                self.loss = self.body()
-            self.launches = _ops.kernels_recorded() - n0     # libgnm kernels inside the graph (C-side counters)
-            _ops.REPLAYED[0] -= self.launches                # capture records, replay launches
-            self.graph = g
-        self.graph.replay()
-        _ops.REPLAYED[0] += self.launches
+            self.graph, self.loss, self.launches = _graphed.capture(self.body)
+        _graphed.replay(self.graph, self.launches)
         return self.loss
 
 
@@ -215,11 +170,6 @@ class Trainer(object):
         self._plans = {}
         self._seen = {}
         self.h2d_bytes = 0
-
-    @staticmethod
-    def _signature(h, n_global):
-        return (h.b, h.m, h.uniform_n, h.onehot, h.feat_dim, h.n_max, h.dense, h.has_isolated, h.same_tags,
-                h.max0_as_sum, n_global)
 
     def adam_state(self, tensors):
         """Flat Adam moments shared with `self.optimizer.state` (so `optimizer.state_dict()` checkpoints them and a
@@ -292,18 +242,18 @@ class Trainer(object):
             raise RuntimeError("Trainer runs the one-hot input path (util.py:114-116); use the model API for dense features")
         if labels is None:
             labels = [g.label for g in batch_graph]             # main.py:31
-        key = self._signature(h, n_global)
+        key = _graphed.plan_key(h, n_global, self.comm.world)
         plan = self._plans.get(key)
-        if plan is not None and h.nnz > plan.nnz_cap:
+        if plan is not None and not plan.inputs.fits(h, key):
             del self._plans[key]
             plan = None
         if plan is None:
             while len(self._plans) >= 2:
                 self._plans.pop(next(iter(self._plans)))
-            plan = _WholeStepPlan(self, h, n_global)
+            plan = _WholeStepPlan(self, h, key, n_global)
             self._plans[key] = plan
             self._seen[key] = 0
-        self.h2d_bytes += plan.load(h, perm, labels)
+        self.h2d_bytes += plan.inputs.load(h, perm, labels)
         self._seen[key] += 1
         self.steps_done += 1
         if self.check_every > 0 and self.steps_done % self.check_every == 0:

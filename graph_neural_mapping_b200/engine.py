@@ -267,17 +267,22 @@ class GraphStore(object):
         h.max0_as_sum = bool(b > 0 and h.onehot and (t[:, 9] != 0).all() and has_bm)
         return h
 
-    def assemble_device(self, h, packed_d, node_off_d, nnz_capacity=None):
-        """Device half: gather the stored CSRs into the batch CSR (one kernel)."""
+    def assemble(self, h, graph_pooling_type, packed_d=None, node_off_d=None, nnz_capacity=None):
+        """Device half: gather the stored CSRs of host batch `h` into the batch CSR (one kernel) and set the graph
+        pooling's scale. `packed_d` / `node_off_d` are device copies of h.packed / h.node_off - a captured step passes
+        its static buffers, with the batch CSR sized for `nnz_capacity` entries; by default they are copied here."""
+        if packed_d is None:
+            packed_d = torch.from_numpy(h.packed).to(self.device, non_blocking=True)
+            node_off_d = torch.from_numpy(h.node_off).to(self.device, non_blocking=True)
+            self.h2d_bytes += h.packed.nbytes + h.node_off.nbytes
         b = h.b
+        nnz_cap = h.nnz if nnz_capacity is None else nnz_capacity
         # batches that run on the dense-block kernels never read the batch column indices: gather them lazily
         # (BatchStructure.colidx) - the copy is 2 x 195 MB of HBM traffic per step at B=1024, N=400
         lazy_cols = h.dense and not FORCE_CSR_AGGREGATE
-        gather_args = (packed_d[0:b], packed_d[b:2 * b], None, node_off_d, packed_d[3 * b:4 * b + 1], b, h.m,
-                       h.nnz if nnz_capacity is None else nnz_capacity)
+        gather_args = (packed_d[0:b], packed_d[b:2 * b], None, node_off_d, packed_d[3 * b:4 * b + 1], b, h.m, nnz_cap)
         rowptr, colidx, tags = _ops.csr_batch_gather(packed_d[0:b], packed_d[b:2 * b], packed_d[2 * b:3 * b],
-                                                     node_off_d, packed_d[3 * b:4 * b + 1], b, h.m,
-                                                     h.nnz if nnz_capacity is None else nnz_capacity,
+                                                     node_off_d, packed_d[3 * b:4 * b + 1], b, h.m, nnz_cap,
                                                      with_colidx=not lazy_cols)
         bs = BatchStructure()
         bs.n_graphs, bs.n_rows, bs.nnz = b, h.m, h.nnz
@@ -293,15 +298,11 @@ class GraphStore(object):
         bs.has_isolated = h.has_isolated
         bs.same_tags = h.same_tags
         bs.max0_as_sum = h.max0_as_sum
+        # graphcnn.py:118-120: 1 / len(graph.g) per graph under average pooling - from the device node offsets (no host
+        # copy: this also runs under CUDA-graph capture)
+        bs.pool_scale = (1.0 / (node_off_d[1:] - node_off_d[:-1]).to(torch.float32)
+                         if graph_pooling_type == "average" else None)
         return bs
-
-    def assemble(self, graphs):
-        h = self.assemble_host(graphs)
-        dev = self.device
-        packed_d = torch.from_numpy(h.packed).to(dev, non_blocking=True)
-        node_off_d = torch.from_numpy(h.node_off).to(dev, non_blocking=True)
-        self.h2d_bytes += h.packed.nbytes + h.node_off.nbytes
-        return self.assemble_device(h, packed_d, node_off_d)
 
 
 class _HostBatch(object):
@@ -374,15 +375,6 @@ class BatchStructure(object):
         return _ops.aggregate_dense_affine(self.bitmap_addr, self.node_off, self.rowptr, self.n_graphs, self.n_max, dy, z,
                                            coef, dst, mode)
 
-    def set_pooling(self, graph_pooling_type, device):
-        if graph_pooling_type == "average":
-            # graphcnn.py:118-120: 1 / len(graph.g) per graph - from the device node offsets (no host copy: this also
-            # runs under CUDA-graph capture)
-            no = self.node_off
-            self.pool_scale = 1.0 / (no[1:] - no[:-1]).to(torch.float32)
-        else:
-            self.pool_scale = None
-
 
 # ------------------------------------------------------------------------------------------
 # parameter plumbing
@@ -421,12 +413,9 @@ def flat_buffers(model):
     if bns is None:
         bns = [bn for layer in range(model.num_layers) for _, bn in layer_units(model, layer)]
         model.__dict__["_gnm_flat_bns"] = bns
-    bs = []
-    for bn in bns:               # buffers are re-read every time: load_state_dict / .to() may replace the tensors
-        for t in (bn.running_mean, bn.running_var, bn.num_batches_tracked):
-            if t is not None:
-                bs.append(t)
-    return bs
+    # buffers are re-read every time: load_state_dict / .to() may replace the tensors. Read from the module's buffer
+    # dict, as model.buffers() does: attribute access through nn.Module.__getattr__ costs 0.5 us per buffer
+    return [t for bn in bns for t in bn._buffers.values() if t is not None]
 
 
 class _Unit(object):

@@ -14,6 +14,10 @@ Inputs and outputs live in static buffers owned by the plan; outputs and gradien
 cloned before they are handed to autograd so the caller never aliases graph memory.
 BatchNorm running statistics, NCCL all-reduces (data parallel) and the batch assembly kernel
 are part of the captured work.
+
+driver.Trainer captures its whole step as one graph on the same pieces: the plan key, the
+check that a plan still fits a batch and the static inputs with their pinned ring
+(StepInputs), and capture / replay with the launch accounting.
 """
 import torch
 
@@ -41,112 +45,125 @@ def quiet_capture():
             gc.enable()
 
 
-class StepPlan(object):
-    """Static buffers + captured graphs for one (B, N, flags) training-step shape."""
+def plan_key(h, n_global, world):
+    """What a captured step bakes in from host batch `h` through its kernel choices and buffer shapes, with `n_global`
+    DGI negatives over `world` data-parallel ranks: batches with equal keys can replay one plan (StepInputs.fits)."""
+    return (h.b, h.m, h.uniform_n, h.onehot, h.feat_dim, h.n_max, h.dense, h.has_isolated, h.same_tags, h.max0_as_sum,
+            n_global, world)
 
-    def __init__(self, model, host_batch, n_neg, comm):
+
+def _pointers(model):
+    return list(map(torch.Tensor.data_ptr, _engine.flat_params(model) + _engine.flat_buffers(model)))
+
+
+class StepInputs(object):
+    """The static inputs of a captured training step - the batch's slot addresses / offsets (`packed`, `node_off`), the
+    DGI permutation (`neg_idx`) and, with `labels`, the class labels - refilled by load() before every step. Also keeps
+    what else the graph bakes in: the plan key, the capacity of the batch CSR and the addresses of the model's
+    parameters and BatchNorm buffers when the plan was made."""
+
+    def __init__(self, model, h, key, n_neg, labels=False):
         dev = model.eps.device
-        h = host_batch
-        self.model, self.comm, self.dev = model, comm, dev
-        self.b, self.m = h.b, h.m
+        self.model, self.key, self.h = model, key, h
         self.nnz_cap = int(h.nnz * 1.02) + 4096
+        self.ptrs = _pointers(model)
         self.packed = torch.zeros(5 * h.b + 1, dtype=torch.int64, device=dev)
         self.node_off = torch.zeros(h.b + 1, dtype=torch.int32, device=dev)
         self.neg_idx = torch.zeros(n_neg, dtype=torch.int32, device=dev)
-        self.pool = torch.cuda.graph_pool_handle()
-        self.fwd_graph = None
-        self.bwd_graph = None
-        self.generation = 0
-        self.h = None
+        self.labels = torch.zeros(h.b, dtype=torch.int64, device=dev) if labels else None
+        self._dst = [t for t in (self.packed, self.node_off, self.neg_idx, self.labels) if t is not None]
         self._stage = [None, None, None]
         self._stage_i = 0
-        self.sig = self._signature(h)
-        self.ptrs = self._pointers()
 
-    # a captured graph bakes in kernel choices and pointers: anything that changes them is part of the key
-    @staticmethod
-    def _signature(h):
-        return (h.b, h.m, h.uniform_n, h.onehot, h.feat_dim, h.n_max, h.dense, h.has_isolated, h.same_tags)
+    def fits(self, h, key):
+        """Whether a step on host batch `h` with plan key `key` may replay the plan: same key, nnz within the capacity,
+        and the model's parameters and BatchNorm buffers still where they were. Replacing a buffer tensor
+        (`bn.running_mean = bn.running_mean.clone()`, load_state_dict(assign=True) + release_graphs()) moves it: a
+        replay would update the tensor the model no longer holds."""
+        return key == self.key and h.nnz <= self.nnz_cap and _pointers(self.model) == self.ptrs
 
-    def _pointers(self):
-        ps = [p.data_ptr() for p in _engine.flat_params(self.model)]
-        ps += [b.data_ptr() for b in _engine.flat_buffers(self.model)]
-        return ps
-
-    def compatible(self, h, n_neg):
-        return (self._signature(h) == self.sig and h.nnz <= self.nnz_cap and n_neg == self.neg_idx.shape[0]
-                and self._pointers() == self.ptrs)
-
-    def load(self, h, perm):
-        """Per-step host -> device traffic: slot addresses / offsets and the DGI permutation, staged through a small
-        ring of pinned buffers and copied asynchronously, so the host never waits for the previous step's kernels and
-        can prepare (and enqueue) the next step while the GPU is still busy with this one."""
+    def load(self, h, perm, labels=None):
+        """Per-step host -> device traffic: slot addresses / offsets, the DGI permutation and the labels, staged through
+        a small ring of pinned buffers and copied asynchronously, so the host never waits for the previous step's
+        kernels and can prepare (and enqueue) the next step while the GPU is still busy with this one. Returns the
+        bytes shipped."""
         self.h = h
         i = self._stage_i
         self._stage_i = (i + 1) % len(self._stage)
         if self._stage[i] is None:
-            self._stage[i] = (torch.empty(self.packed.shape[0], dtype=torch.int64, pin_memory=True),
-                              torch.empty(self.node_off.shape[0], dtype=torch.int32, pin_memory=True),
-                              torch.empty(self.neg_idx.shape[0], dtype=torch.int32, pin_memory=True),
+            self._stage[i] = ([torch.empty(t.shape[0], dtype=t.dtype, pin_memory=True) for t in self._dst],
                               torch.cuda.Event())
         else:
-            self._stage[i][3].synchronize()           # the copies that last read this slot (three steps ago) are done
-        s_packed, s_off, s_neg, ev = self._stage[i]
-        s_packed.numpy()[:] = h.packed
-        s_off.numpy()[:] = h.node_off
-        s_neg.numpy()[:] = perm
-        self.packed.copy_(s_packed, non_blocking=True)
-        self.node_off.copy_(s_off, non_blocking=True)
-        self.neg_idx.copy_(s_neg, non_blocking=True)
+            self._stage[i][1].synchronize()           # the copies that last read this slot (three steps ago) are done
+        pinned, ev = self._stage[i]
+        for s, x in zip(pinned, (h.packed, h.node_off, perm, labels)):
+            s.numpy()[:] = x
+        for t, s in zip(self._dst, pinned):
+            t.copy_(s, non_blocking=True)
         ev.record()
-        return h.packed.nbytes + h.node_off.nbytes + 4 * perm.size
+        return sum(s.nbytes for s in pinned)
 
-    def _structure(self):
-        store = self.model._graph_store()
-        bs = store.assemble_device(self.h, self.packed, self.node_off, nnz_capacity=self.nnz_cap)
-        bs.set_pooling(self.model.graph_pooling_type, self.dev)
-        return bs
+    def structure(self):
+        """The BatchStructure of the loaded batch, gathered from the static buffers (also under capture)."""
+        model = self.model
+        return model._graph_store().assemble(self.h, model.graph_pooling_type, self.packed, self.node_off, self.nnz_cap)
+
+
+def capture(body, pool=None):
+    """body() captured into a CUDA graph in memory pool `pool` (None: a private one). Returns (graph, body's result,
+    libgnm kernels recorded). Capture records the kernels without running them, so they come off ops.REPLAYED here and
+    replay() adds them back whenever they run."""
+    g = torch.cuda.CUDAGraph()
+    n0 = _ops.kernels_recorded()
+    with quiet_capture(), torch.cuda.graph(g, pool=pool):
+        out = body()
+    launches = _ops.kernels_recorded() - n0           # libgnm kernels inside the graph (C-side counters)
+    _ops.REPLAYED[0] -= launches
+    return g, out, launches
+
+
+def replay(graph, launches):
+    graph.replay()
+    _ops.REPLAYED[0] += launches
+
+
+class StepPlan(object):
+    """Captured encoder forward and backward graphs, in one memory pool, for one training-step shape."""
+
+    def __init__(self, model, host_batch, key, n_neg, comm):
+        self.model, self.comm = model, comm
+        self.inputs = StepInputs(model, host_batch, key, n_neg)
+        self.pool = torch.cuda.graph_pool_handle()
+        self.fwd_graph = None
+        self.bwd_graph = None
+        self.generation = 0
 
     def forward(self):
-        model = self.model
         if self.fwd_graph is None:
-            g = torch.cuda.CUDAGraph()
-            params = [p.detach() for p in _engine.flat_params(model)]
-            n0 = _ops.kernels_recorded()
-            with quiet_capture(), torch.cuda.graph(g, pool=self.pool):
-                bs = self._structure()
-                g_f, d_logit, sv = _engine.run_forward(model, bs, self.neg_idx, True, True, None, params, self.comm)
-            self.fwd_launches = _ops.kernels_recorded() - n0   # libgnm kernels inside the graph (C-side counters)
-            _ops.REPLAYED[0] -= self.fwd_launches              # capture records, replay launches
-            self.fwd_graph, self.g_f, self.d_logit, self.sv, self.params = g, g_f, d_logit, sv, params
-            self.bwd_graph = None
-        self.fwd_graph.replay()
-        _ops.REPLAYED[0] += self.fwd_launches
+            model, inputs = self.model, self.inputs
+            self.params = [p.detach() for p in _engine.flat_params(model)]
+            self.fwd_graph, (self.g_f, self.d_logit, self.sv), self.fwd_launches = capture(
+                lambda: _engine.run_forward(model, inputs.structure(), inputs.neg_idx, True, True, None, self.params,
+                                            self.comm), self.pool)
+        replay(self.fwd_graph, self.fwd_launches)
         self.generation += 1
         return self.g_f.clone(), self.d_logit.clone()
+
+    def _backward_body(self):
+        _, grads = _engine.run_backward(self.model, self.sv, self.params, self.dg_in, self.dd_in, False, self.comm)
+        self.grad_shapes = [None if x is None else tuple(x.shape) for x in grads]
+        self.grad_sizes = [int(x.numel()) for x in grads if x is not None]
+        return torch.cat([x.reshape(-1) for x in grads if x is not None])
 
     def backward(self, dg_f, dd_logit):
         if self.bwd_graph is None:
             self.dg_in = torch.zeros_like(self.g_f)
             self.dd_in = torch.zeros_like(self.d_logit)
-            self.dg_in.copy_(dg_f)
-            self.dd_in.copy_(dd_logit)
-            g = torch.cuda.CUDAGraph()
-            n0 = _ops.kernels_recorded()
-            with quiet_capture(), torch.cuda.graph(g, pool=self.pool):
-                _, grads = _engine.run_backward(self.model, self.sv, self.params, self.dg_in, self.dd_in, False,
-                                                self.comm)
-                self.grad_shapes = [None if x is None else tuple(x.shape) for x in grads]
-                self.grad_sizes = [int(x.numel()) for x in grads if x is not None]
-                self.flat = torch.cat([x.reshape(-1) for x in grads if x is not None])
-            self.bwd_launches = _ops.kernels_recorded() - n0
-            _ops.REPLAYED[0] -= self.bwd_launches
-            self.bwd_graph = g
-        else:
-            self.dg_in.copy_(dg_f)
-            self.dd_in.copy_(dd_logit)
-        self.bwd_graph.replay()
-        _ops.REPLAYED[0] += self.bwd_launches
+        self.dg_in.copy_(dg_f)
+        self.dd_in.copy_(dd_logit)
+        if self.bwd_graph is None:
+            self.bwd_graph, self.flat, self.bwd_launches = capture(self._backward_body, self.pool)
+        replay(self.bwd_graph, self.bwd_launches)
         pieces = iter(self.flat.clone().split(self.grad_sizes))        # one call: the per-tensor slicing was host time
         return [None if shp is None else next(pieces).view(shp) for shp in self.grad_shapes]
 

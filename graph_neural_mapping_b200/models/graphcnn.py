@@ -134,14 +134,7 @@ class GIN_InfoMaxReg(nn.Module):
 
     def _structure(self, batch_graph, host_batch=None):
         h = host_batch if host_batch is not None else self._host_batch(batch_graph)
-        store = self._graph_store()
-        dev = self.eps.device
-        packed_d = torch.from_numpy(h.packed).to(dev, non_blocking=True)
-        node_off_d = torch.from_numpy(h.node_off).to(dev, non_blocking=True)
-        store.h2d_bytes += h.packed.nbytes + h.node_off.nbytes
-        bs = store.assemble_device(h, packed_d, node_off_d)
-        bs.set_pooling(self.graph_pooling_type, dev)
-        return bs
+        return self._graph_store().assemble(h, self.graph_pooling_type)
 
     def _step_plan(self, h, n_global):
         """The CUDA-graph plan for this training-step shape, or None (first sighting runs eagerly: it warms up
@@ -149,9 +142,9 @@ class GIN_InfoMaxReg(nn.Module):
         if not (self.use_cuda_graphs and self.training and torch.is_grad_enabled() and h.onehot
                 and (self.neighbor_pooling_type != "max" or h.max0_as_sum) and self.eps.device.type == "cuda"):
             return None
-        key = _graphed.StepPlan._signature(h) + (n_global, self._comm.world)      # training only: comm is self._comm
+        key = _graphed.plan_key(h, n_global, self._comm.world)          # training only: comm is self._comm
         plan = self._plans.get(key)
-        if plan is not None and not plan.compatible(h, n_global):
+        if plan is not None and not plan.inputs.fits(h, key):
             del self._plans[key]
             plan = None
         if plan is None:
@@ -160,7 +153,7 @@ class GIN_InfoMaxReg(nn.Module):
                 return None
             while len(self._plans) >= 2:
                 self._plans.pop(next(iter(self._plans)))
-            plan = _graphed.StepPlan(self, h, n_global, self._comm)
+            plan = _graphed.StepPlan(self, h, key, n_global, self._comm)
             self._plans[key] = plan
         return plan
 
@@ -320,7 +313,7 @@ class GIN_InfoMaxReg(nn.Module):
             raise RuntimeError("GIN_InfoMaxReg.forward needs graphs with the same number of nodes")
         plan = self._step_plan(h, n_global)
         if plan is not None:
-            self._graph_store().h2d_bytes += plan.load(h, rand_seq)
+            self._graph_store().h2d_bytes += plan.inputs.load(h, rand_seq)
             g_f, d_logit = _graphed.GraphedGINFunction.apply(plan, *_engine.flat_params(self))
         else:
             bs = self._structure(batch_graph, h)

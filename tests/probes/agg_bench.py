@@ -18,7 +18,7 @@ def main():
     dev = torch.device("cuda")
     graphs = synth.make_graphs_bulk(b, n_nodes, 30, 128, seed0=0, device=dev)
     store = engine.GraphStore(dev, add_self_loops=True)
-    bs = store.assemble(graphs)
+    bs = store.assemble(store.assemble_host(graphs), "sum")
     m, f = bs.n_rows, (int(sys.argv[5]) if len(sys.argv) > 5 else 64)
     torch.manual_seed(0)
     src = torch.randn(m, f, device=dev)

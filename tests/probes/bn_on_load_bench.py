@@ -38,7 +38,7 @@ def main():
     dev = torch.device("cuda")
     graphs = synth.make_graphs_bulk(b, n, 30, 128, seed0=0, device=dev)
     store = engine.GraphStore(dev, add_self_loops=True)
-    bs = store.assemble(graphs)
+    bs = store.assemble(store.assemble_host(graphs), "sum")
     m = bs.n_rows
     torch.manual_seed(0)
     z = torch.randn(m, f, device=dev)

@@ -15,11 +15,15 @@ digest of the trace and one of the case's outputs (parameter gradients, saliency
        a graph's points over two passes, and one that packs several graphs per pass) and compute_roi_occlusion_batched at
        two occlusions_per_pass that split differently. A call that raises ValueError records its message. Deterministic:
        both digests are compared bit for bit.
-  gpu: the libgnm kernels. Trainer steps (fused and not, the eager warm-up steps), model(graphs) + backward at
-       1024 x 400, learn_eps, average pooling with an isolated node, max pooling, hidden width 128, ROI saliency
-       (one-hot, dense, max pooling) and the integrated-gradients and occlusion calls of the cpu mode on the same models.
-       CUDA graphs are off, so every call is eager and recorded. Only the trace digests are meant to match across
-       builds: the kernels' float atomics make outputs differ in the last bits.
+  gpu: the libgnm kernels. Trainer steps (fused and not: the two eager warm-up steps, the capture and a replay),
+       model(graphs) + backward with CUDA graphs on (the eager first sighting, the capture and a replay), then with CUDA
+       graphs off model(graphs) + backward at 1024 x 400, learn_eps, average pooling with an isolated node, max pooling,
+       hidden width 128, ROI saliency (one-hot, dense, max pooling) and the integrated-gradients and occlusion calls of
+       the cpu mode on the same models. A capture records its calls, a replay none. Only the trace digests are meant to
+       match across builds: the kernels' float atomics make outputs differ in the last bits.
+
+The launch counter readers (ops.launch_counts, kernels_recorded, kernels_launched) are not recorded: they launch
+nothing, and which module reads them around a capture is plumbing.
 
     python tests/probes/ops_trace.py cpu|gpu [--dump DIR]"""
 import argparse
@@ -34,13 +38,14 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
-from graph_neural_mapping_b200 import driver, engine, synth  # noqa: E402
+from graph_neural_mapping_b200 import driver, engine, graphed, synth  # noqa: E402
 from graph_neural_mapping_b200.models import GIN_InfoMaxReg  # noqa: E402
 from graph_neural_mapping_b200.models import discriminator as dmod  # noqa: E402
 from graph_neural_mapping_b200.models import graphcnn as gmod  # noqa: E402
 from graph_neural_mapping_b200.models import mlp as mlpmod  # noqa: E402
 
-USERS = (engine, gmod, mlpmod, dmod, driver)
+USERS = (engine, gmod, mlpmod, dmod, driver, graphed)
+COUNTERS = ("launch_counts", "kernels_recorded", "kernels_launched")
 
 
 def _sig(v):
@@ -66,7 +71,7 @@ class TracingOps(object):
 
     def __getattr__(self, name):
         attr = getattr(self._base, name)
-        if name.startswith("_") or not inspect.isfunction(attr):
+        if name.startswith("_") or name in COUNTERS or not inspect.isfunction(attr):
             return attr
         params = inspect.signature(attr)
         trace = self.trace
@@ -244,12 +249,17 @@ def gpu_cases(dump):
         model = model_of(5, 400, 64, seed=1)
         tr = driver.Trainer(model, fused=fused)
         graphs = synth.make_graphs_bulk(256, 400, 30, 128, seed0=10, device=dev)
-        for step in range(2):                              # the eager warm-up steps
+        for step in range(4):                              # two eager warm-up steps, capture, replay
             np.random.seed(step)
             with Case(shim) as case:
                 case.add(tr.step(graphs).reshape(1))
                 torch.cuda.synchronize()
             report("trainer.fused=%s.step%d" % (fused, step), case, dump)
+
+    model = model_of(5, 400, 64, seed=7)
+    model.use_cuda_graphs = True
+    for step in range(3):                                  # eager first sighting, capture, replay
+        train_case("model.graphed.step%d" % step, model, graphs, seed=step)
 
     big = synth.make_graphs_bulk(1024, 400, 30, 128, seed0=20, device=dev)
     model = model_of(5, 400, 64, seed=2)

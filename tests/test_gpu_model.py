@@ -488,6 +488,44 @@ def test_trainer_learning_rate_schedule_reaches_the_captured_step():
     assert again > 3.0 * small, (small, again)
 
 
+@pytest.mark.parametrize("path", ["trainer", "model"])
+def test_captured_step_follows_a_replaced_batchnorm_buffer(path):
+    """A captured step bakes in the addresses of the BatchNorm buffers it updates. After four steps (Trainer: eager,
+    eager, capture, replay; model(graphs) with CUDA graphs: eager, capture, replay, replay) one running_mean is replaced
+    by a clone, as load_state_dict(assign=True) would: the next step must update the new tensor and count itself in
+    num_batches_tracked, and leave the tensor the model no longer holds alone."""
+    from graph_neural_mapping_b200.driver import Trainer
+    g = Golden("mid_eps_sum_h64")
+    graphs = g.graphs()
+    model = build_model(g)
+    model.train()
+    model.use_cuda_graphs = True
+    tr = Trainer(model, lr=0.01, beta=g.cfg["beta"]) if path == "trainer" else None
+
+    def step(seed):
+        if tr is not None:
+            np.random.seed(seed)
+            tr.step(graphs)
+        else:
+            train_step(model, graphs, g.cfg["beta"], seed)
+
+    for sd in range(4):
+        step(20 + sd)
+    plans = tr._plans if tr is not None else model._plans
+    plan = next(iter(plans.values()))
+    assert len(plans) == 1 and (plan.graph if tr is not None else plan.bwd_graph) is not None
+    bn = model.batch_norms[0]
+    old = bn.running_mean
+    bn.running_mean = old.clone()
+    new, old_before, new_before = bn.running_mean, old.clone(), bn.running_mean.clone()
+    count = int(bn.num_batches_tracked)
+    step(30)
+    torch.cuda.synchronize()
+    assert not torch.equal(new, new_before), "the step did not update the model's running_mean"
+    assert torch.equal(old, old_before), "the step wrote the replaced running_mean"
+    assert int(bn.num_batches_tracked) == count + 1
+
+
 def test_graph_store_stays_within_its_byte_budget():
     """Callers that build fresh graph objects every step must not leak device memory: the store drops its contents
     when the budget is exceeded and the results do not change."""
